@@ -2,6 +2,7 @@
 """Benchmark of the torchext op path on B200 (BASELINE.json metric, configs[1]).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this framework (libctd_b200.so)
+    python bench.py --dump-outputs DIR [...]                        # + the last timed step's outputs as DIR/<name>.npy
     python bench.py --impl reference [...]                          # the reference's CPU path, host cores
     torchrun --nproc-per-node N ... bench.py --gpus N ...           # one rank per GPU, weak scaling
 
@@ -479,6 +480,8 @@ def run_b200_arm(args, rank, world, local_rank):
     n_evented = min(NSETS, max(1, args.steps // 10), args.steps)
     ms_per_step = timed_run(args.steps, plain_graphs, args.pipeline, evented_tail=n_evented)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # before the legs below overwrite the buffers
+        dump_outputs(args.dump_outputs, sets[(args.steps - 1) % NSETS])
     used = sorted({k % NSETS for k in range(args.steps - n_evented, args.steps)})
     op_ms = {n: float(np.mean([set_events[si][i].elapsed_time(set_events[si][i + 1]) for si in used])) for i, n in enumerate(OPS)}
     launches = (_lib.launch_count() - launches0) if not use_graph else kernels_per_graph * args.steps
@@ -646,6 +649,23 @@ def run_b200_arm(args, rank, world, local_rank):
         dist.destroy_process_group()
 
 
+DUMP_IMAGES = 8  # six [8,1,480,640] float32 maps = 59 MB: the dump stays under 64 MB at any batch
+
+
+def dump_outputs(out_dir, d):
+    """What the last timed step hands its caller, as float32 .npy files in out_dir: LCN's two outputs, the loss map
+    and d loss / d es of both losses (images 0..7 of the batch; a larger batch repeats those frames), and each
+    loss's masked-mean terms over the whole batch (sum(std * loss), sum(std)).  Inputs are seeded, so two builds run
+    with the same arguments can be compared file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = DUMP_IMAGES
+    arrays = {"lcn": d["lcn"][:n], "lcn_std": d["std"][:n], "sad_loss": d["out_sad"][:n], "sad_grad": d["gi_sad"][:n],
+              "census_sad_loss": d["out_cs"][:n], "census_sad_grad": d["gi_cs"][:n],
+              "sad_masked_sums": d["sums"][0], "census_sad_masked_sums": d["sums"][1]}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float32))
+
+
 def run_strong_block(args, rank, world, dev, sync_all):
     """BASELINE configs[4] as stated: a FIXED global batch of 64 frames (16 tracks of 4 frames) split over the ranks by
     shard_range, the ops of configs 2 and 4 -- LCN, sad and census_sad forward+backward with their masked sums, ProjNN
@@ -774,7 +794,12 @@ def main():
     ap.add_argument("--census-sym", type=int, default=-1, help="A/B runs: ctd_set_option('census_sym', v) before the benchmark (0 gather kernels, 1 pair-symmetric kernel everywhere, 2 automatic = library default)")
     ap.add_argument("--no-strong", action="store_true", help="skip the `strong` block (BASELINE configs[4]: global batch 64 over the ranks)")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra op timings (XCorrVol, ProjNN, ...) and the reference CUDA extension leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the B200 path's outputs; the reference arm times a CPU sample and keeps none")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -4,9 +4,12 @@ Argument meaning and return shapes mirror the reference's CPU entry points
 (torchext/ext/ext_cpu.cpp:14-184) so tests read like calls into the reference.  Only
 tests/, __graft_entry__.smoke() and bench.py's CPU-baseline legs may import this module.
 """
+import atexit
 import ctypes
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -19,19 +22,26 @@ _lib = None
 
 
 def build():
-    """(Re)build libctd_oracle.so with the committed Makefile if it is missing or stale."""
-    srcs = [os.path.join(HERE, f) for f in ("ctd_oracle.c", "ctd_oracle_impl.h", "Makefile")]
-    if os.path.exists(LIB_PATH) and all(os.path.getmtime(LIB_PATH) >= os.path.getmtime(s) for s in srcs):
+    """Path of a libctd_oracle.so built from the current sources: the in-tree one, (re)built with the committed
+    Makefile if it is missing or stale.  In a read-only tree a missing or stale library is built in a temporary
+    directory instead (removed at exit)."""
+    names = ("ctd_oracle.c", "ctd_oracle_impl.h", "Makefile")
+    if os.path.exists(LIB_PATH) and all(os.path.getmtime(LIB_PATH) >= os.path.getmtime(os.path.join(HERE, f)) for f in names):
         return LIB_PATH
-    subprocess.run(["make", "-C", HERE, "libctd_oracle.so"], check=True, capture_output=True)
-    return LIB_PATH
+    where = HERE
+    if not os.access(HERE, os.W_OK):
+        where = tempfile.mkdtemp(prefix="ctd_oracle_")
+        atexit.register(shutil.rmtree, where, True)
+        for f in names:
+            shutil.copy(os.path.join(HERE, f), where)
+    subprocess.run(["make", "-C", where, "libctd_oracle.so"], check=True, capture_output=True)
+    return os.path.join(where, "libctd_oracle.so")
 
 
 def lib():
     global _lib
     if _lib is None:
-        build()
-        _lib = ctypes.CDLL(LIB_PATH)
+        _lib = ctypes.CDLL(build())
     return _lib
 
 

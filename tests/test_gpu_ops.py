@@ -668,7 +668,7 @@ def test_xcorrvol_full_size_properties(tx):
 @pytest.mark.parametrize("bs", (9, 5))
 def test_xcorrvol_full_size_golden(tx, golden, bs):
     """BASELINE configs[2] at its own size against the UNMODIFIED reference: 480x640, D = 128, the batched B = 8 call;
-    image 0 is compared with the rows of the reference's volume kept in tests/golden/xcorrvol_full.npz
+    image 0 is compared with the rows and columns of the reference's volume kept in tests/golden/xcorrvol_full.npz
     (tests/golden/make_golden_full.py: oracle/_ref xcorrvol_cpu on the same synthetic LCN'd pair)."""
     from connecting_the_dots_b200 import synth
     g = golden("xcorrvol_full")
@@ -679,8 +679,8 @@ def test_xcorrvol_full_size_golden(tx, golden, bs):
     assert float(in0[0].astype(np.float64).sum()) == float(g["in0_sum"])
     vol = tx.xcorrvol(cu(in0), cu(in1), 128, bs)
     assert vol.shape == (8, 128, 480, 640)
-    rows = torch.from_numpy(g["rows"]).to(DEV)
-    got = vol[0].index_select(1, rows).cpu().numpy()
+    rows, cols = torch.from_numpy(g["rows"]).to(DEV), torch.from_numpy(g["cols"]).to(DEV)
+    got = vol[0].index_select(1, rows).index_select(2, cols).cpu().numpy()
     assert_close(got, g["bs%d" % bs], what="xcorrvol 480x640 D128 bs%d vs reference" % bs)
     one = tx.xcorrvol(cu(in0[0]), cu(in1[0]), 128, bs)   # the reference's unbatched 3-D signature, same result
     assert torch.equal(one, vol[0])

@@ -1,5 +1,5 @@
-import sys
-sys.path.insert(0, "/root/repo")
+import os, sys
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 from connecting_the_dots_b200 import _lib, synth
 H, W, B = 480, 640, 8
