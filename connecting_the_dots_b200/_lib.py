@@ -17,6 +17,11 @@ SIGNATURES = {
     "ctd_photometric_bwd_f64": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _int, _int, _f32, _ptr],
     "ctd_photometric_fwd_bwd_f32": [_ptr, _ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _int, _int, _f32, _ptr],
     "ctd_photometric_fwd_bwd_masked_f32": [_ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _int, _int, _f32, _ptr],
+    "ctd_ssim_fwd_f32": [_ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _int, _f64, _f64, _ptr],
+    "ctd_ssim_fwd_f64": [_ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _int, _f64, _f64, _ptr],
+    "ctd_ssim_bwd_f32": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _int, _f64, _f64, _ptr],
+    "ctd_ssim_bwd_f64": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _int, _f64, _f64, _ptr],
+    "ctd_ssim_fwd_bwd_masked_f32": [_ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _int, _f64, _f64, _ptr],
     "ctd_warp_pattern_fwd_f32": [_ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _i64, _ptr],
     "ctd_warp_pattern_bwd_f32": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _i64, _ptr],
     "ctd_depth_similarity_f32": [_ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _f32, _f32, _int, _ptr],

@@ -184,6 +184,67 @@ def photometric_loss_forward_backward_masked(es, ta, grad_out, mask, block_size,
     return out, grad_in, sums
 
 
+def _ssim_args(es, ta):
+    _check_input_cuda(es, "es")
+    _check_input_cuda(ta, "ta")
+    _check(es.dim() == 4, "es has to be B x C x H x W")
+    _check(tuple(es.shape) == tuple(ta.shape), "es and ta have to be the same shape")
+    _same(es, ta, "es", "ta")
+    return _real_suffix(es, "ssim_loss")
+
+
+def _ssim_grad_out(es, grad_out):
+    _check_input_cuda(grad_out, "grad_out")
+    B, C, H, W = es.shape
+    _check(grad_out.numel() == B * H * W, "grad_out has to be B x 1 x H x W")
+    _same(es, grad_out, "es", "grad_out")
+
+
+def ssim_forward(es, ta, block_size, c1, c2):
+    """SSIM loss map (ctd_ssim_fwd_*): es, ta [B,C,H,W] -> [B,1,H,W] = sum over channels of (1 - SSIM) / 2 over the
+    replicate-clamped block_size^2 window of photometric_loss."""
+    sfx = _ssim_args(es, ta)
+    B, C, H, W = es.shape
+    out = torch.empty((B, 1, H, W), dtype=es.dtype, device=es.device)
+    with torch.cuda.device(es.device):
+        _lib.call("ctd_ssim_fwd" + sfx, es.data_ptr(), ta.data_ptr(), out.data_ptr(), B, C, H, W, int(block_size),
+                  float(c1), float(c2), _stream(es))
+    return out
+
+
+def ssim_backward(es, ta, grad_out, block_size, c1, c2):
+    """Gradient of ssim_forward w.r.t. es for grad_out [B,1,H,W] -> [B,C,H,W] (ctd_ssim_bwd_*)."""
+    sfx = _ssim_args(es, ta)
+    _ssim_grad_out(es, grad_out)
+    B, C, H, W = es.shape
+    grad_in = torch.empty((B, C, H, W), dtype=es.dtype, device=es.device)
+    with torch.cuda.device(es.device):
+        _lib.call("ctd_ssim_bwd" + sfx, es.data_ptr(), ta.data_ptr(), grad_out.data_ptr(), grad_in.data_ptr(), B, C, H, W,
+                  int(block_size), float(c1), float(c2), _stream(es))
+    return grad_in
+
+
+def ssim_forward_backward_masked(es, ta, grad_out, mask, block_size, c1, c2):
+    """Loss map, gradient w.r.t. es and sums = (sum(mask * loss), sum(mask)) from one pass
+    (ctd_ssim_fwd_bwd_masked_f32).  Returns (loss map [B,1,H,W], gradient [B,C,H,W], sums float32 [2]); fp32 only."""
+    _ssim_args(es, ta)
+    _check(es.dtype == torch.float32, "ssim_forward_backward_masked is float32 only")
+    _ssim_grad_out(es, grad_out)
+    _check_input_cuda(mask, "mask")
+    B, C, H, W = es.shape
+    _check(mask.numel() == B * H * W, "mask has to be B x 1 x H x W")
+    _check(mask.dtype == torch.float32, "mask has to be float32")
+    _same(es, mask, "es", "mask")
+    out = torch.empty((B, 1, H, W), dtype=es.dtype, device=es.device)
+    grad_in = torch.empty((B, C, H, W), dtype=es.dtype, device=es.device)
+    sums = torch.empty(2, dtype=torch.float32, device=es.device)
+    with torch.cuda.device(es.device):
+        _lib.call("ctd_ssim_fwd_bwd_masked_f32", es.data_ptr(), ta.data_ptr(), grad_out.data_ptr(), mask.data_ptr(),
+                  out.data_ptr(), grad_in.data_ptr(), sums.data_ptr(), B, C, H, W, int(block_size), float(c1), float(c2),
+                  _stream(es))
+    return out, grad_in, sums
+
+
 def _warp_args(pattern, disp):
     _check_input_cuda(pattern, "pattern")
     _check_input_cuda(disp, "disp")

@@ -161,6 +161,81 @@ def weighted_photometric_loss(es, ta, mask, block_size, type="mse", eps=0.1):
     return WeightedPhotometricLossFunction.apply(es, ta, mask, block_size, _loss_type_id(type), eps)
 
 
+SSIM_C1, SSIM_C2 = 0.01 ** 2, 0.03 ** 2
+
+
+class SSIMLossFunction(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, es, ta, block_size, c1, c2):
+        if not es.is_cuda:
+            raise RuntimeError("torchext.ssim_loss: connecting_the_dots_b200 has no CPU implementation")
+        es, ta = es.detach(), ta.detach()
+        ctx.save_for_backward(es, ta)
+        ctx.block_size, ctx.c1, ctx.c2 = block_size, c1, c2
+        return ext_cuda.ssim_forward(es, ta, block_size, c1, c2)
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        es, ta = ctx.saved_tensors
+        return ext_cuda.ssim_backward(es, ta, grad_out.contiguous(), ctx.block_size, ctx.c1, ctx.c2), None, None, None, None
+
+
+def ssim_loss(es, ta, block_size, c1=SSIM_C1, c2=SSIM_C2):
+    """SSIM photometric loss map [B,1,H,W]: for every pixel and channel the structural similarity S of es and ta over the
+    block_size^2 window of photometric_loss (taps clamp(h + i - block_size//2), clamp(w + j - block_size//2), i, j in
+    [0, block_size): replicate-clamped at the border), with population statistics
+        S = (2 mx my + c1)(2 vxy + c2) / ((mx^2 + my^2 + c1)(vxx + vyy + c2)),
+    and out = sum over channels of (1 - S) / 2 (not clamped).  c1, c2 > 0.  Differentiable w.r.t. es (ta gets no
+    gradient).  CUDA tensors only, float32 or float64."""
+    return SSIMLossFunction.apply(es, ta, block_size, c1, c2)
+
+
+def ssim_loss_pytorch(es, ta, block_size, c1=SSIM_C1, c2=SSIM_C2):
+    """Plain-torch evaluation of ssim_loss (differentiable by autograd, any device): the same loop over window offsets on
+    a replicate-padded copy as photometric_loss_pytorch, with centred second moments."""
+    lo = block_size // 2
+    hi = block_size - 1 - lo
+    H, W = es.shape[2], es.shape[3]
+    es_p = torch.nn.functional.pad(es, (lo, hi, lo, hi), mode="replicate")
+    ta_p = torch.nn.functional.pad(ta, (lo, hi, lo, hi), mode="replicate")
+    taps = [(es_p[:, :, dy:dy + H, dx:dx + W], ta_p[:, :, dy:dy + H, dx:dx + W]) for dy in range(block_size) for dx in range(block_size)]
+    n = block_size ** 2
+    mx = sum(e for e, _ in taps) / n
+    my = sum(t for _, t in taps) / n
+    vxx = sum((e - mx) ** 2 for e, _ in taps) / n
+    vyy = sum((t - my) ** 2 for _, t in taps) / n
+    vxy = sum((e - mx) * (t - my) for e, t in taps) / n
+    s = (2 * mx * my + c1) * (2 * vxy + c2) / ((mx * mx + my * my + c1) * (vxx + vyy + c2))
+    return ((1 - s) / 2).sum(dim=1, keepdim=True)
+
+
+class WeightedSSIMLossFunction(torch.autograd.Function):
+    """`(mask * ssim_loss(es, ta)).sum() / mask.sum()` as ONE op, like WeightedPhotometricLossFunction: loss map,
+    gradient and both sums from one fused pass (ctd_ssim_fwd_bwd_masked_f32); autograd's backward is a scalar multiply.
+    Returns (value, loss_map); mask is not differentiated."""
+
+    @staticmethod
+    def forward(ctx, es, ta, mask, block_size, c1, c2):
+        if not es.is_cuda:
+            raise RuntimeError("torchext.weighted_ssim_loss: connecting_the_dots_b200 has no CPU implementation")
+        mask = mask.detach().contiguous()
+        # grad_out = mask: the gradient comes back unnormalised and is divided by sum(mask) in backward
+        out, grad_es, sums = ext_cuda.ssim_forward_backward_masked(es.detach(), ta.detach(), mask, mask, block_size, c1, c2)
+        ctx.save_for_backward(grad_es, sums)
+        ctx.mark_non_differentiable(out)
+        return sums[0] / sums[1], out
+
+    @staticmethod
+    def backward(ctx, g_val, g_map):
+        grad_es, sums = ctx.saved_tensors
+        return grad_es * (g_val / sums[1]), None, None, None, None, None
+
+
+def weighted_ssim_loss(es, ta, mask, block_size, c1=SSIM_C1, c2=SSIM_C2):
+    """Masked mean of the SSIM loss map and the map itself: (value, loss_map [B,1,H,W]); float32 CUDA tensors."""
+    return WeightedSSIMLossFunction.apply(es, ta, mask, block_size, c1, c2)
+
+
 class WarpPatternFunction(torch.autograd.Function):
     """The disparity warp of the reference pattern (model/networks.py:362-371): one gather kernel instead of
     building uv grids and calling grid_sample; differentiable w.r.t. disp."""

@@ -39,6 +39,17 @@ class PhotometricLoss(torch.nn.Module):
         return F.photometric_loss(es, ta, self.block_size, self.type, self.eps)
 
 
+class SSIMLoss(torch.nn.Module):
+    """forward(es, ta) -> ssim_loss map [B,1,H,W]."""
+
+    def __init__(self, block_size=3, c1=F.SSIM_C1, c2=F.SSIM_C2):
+        super().__init__()
+        self.block_size, self.c1, self.c2 = block_size, c1, c2
+
+    def forward(self, es, ta):
+        return F.ssim_loss(es, ta, self.block_size, self.c1, self.c2)
+
+
 class XCorrVol(torch.nn.Module):
     def __init__(self, n_disps=128, block_size=9):
         super().__init__()

@@ -83,6 +83,25 @@ int ctd_photometric_fwd_bwd_masked_f32(const float* es, const float* ta, const f
                                        float* out, float* grad_in, float* sums2, int64_t B, int64_t C, int64_t H,
                                        int64_t W, int block_size, int type, float eps, ctd_stream_t stream);
 
+/* ---- SSIM photometric loss (an addition: the reference has no SSIM op).  Same window as the photometric loss:
+ * taps (clamp(h + i - bs/2), clamp(w + j - bs/2)), i, j in [0, bs), N = bs^2; with x = es, y = ta and population
+ * statistics over the window, S = (2 mx my + c1)(2 vxy + c2) / ((mx^2 + my^2 + c1)(vxx + vyy + c2)) and
+ * out[n,0,h,w] = sum_c (1 - S_c) / 2.  c1 > 0 and c2 > 0 (usual values 0.01^2, 0.03^2).  The backward is the gradient
+ * w.r.t. es for grad_out [B,1,H,W]; grad_in [B,C,H,W] is fully overwritten, no atomics. */
+int ctd_ssim_fwd_f32(const float* es, const float* ta, float* out, int64_t B, int64_t C, int64_t H, int64_t W,
+                     int block_size, double c1, double c2, ctd_stream_t stream);
+int ctd_ssim_fwd_f64(const double* es, const double* ta, double* out, int64_t B, int64_t C, int64_t H, int64_t W,
+                     int block_size, double c1, double c2, ctd_stream_t stream);
+int ctd_ssim_bwd_f32(const float* es, const float* ta, const float* grad_out, float* grad_in, int64_t B, int64_t C,
+                     int64_t H, int64_t W, int block_size, double c1, double c2, ctd_stream_t stream);
+int ctd_ssim_bwd_f64(const double* es, const double* ta, const double* grad_out, double* grad_in, int64_t B, int64_t C,
+                     int64_t H, int64_t W, int block_size, double c1, double c2, ctd_stream_t stream);
+/* forward + backward + sums2 = (sum(mask * out), sum(mask)) in one pass (one kernel for odd block sizes 3..11),
+ * deterministic; mask [B,1,H,W] */
+int ctd_ssim_fwd_bwd_masked_f32(const float* es, const float* ta, const float* grad_out, const float* mask, float* out,
+                                float* grad_in, float* sums2, int64_t B, int64_t C, int64_t H, int64_t W,
+                                int block_size, double c1, double c2, ctd_stream_t stream);
+
 /* ---- the disparity warp in front of the loss: model/networks.py:362-371 (RectifiedPatternSimilarityLoss.tforward),
  * grid_sample(pattern, grid(disp), bilinear, padding_mode='border', align_corners=False) with the reference's (W-1)
  * grid normalisation.  pattern [Bp,1,Hp,Wp] (Bp = 1 or B), disp [B,1,H,W] -> out [B,1,H,W]; backward: gradient

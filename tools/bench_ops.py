@@ -3,7 +3,7 @@
 launching stream, rotating buffer sets larger than L2 where the op is HBM-bound).  Prints one JSON
 object; bench.py stays the contract benchmark, this is the per-op table that goes into profiles/.
 
-    python tools/bench_ops.py [--iters 30] [--only photometric,lcn,xcorrvol,proj_nn,nn,crosscheck]
+    python tools/bench_ops.py [--iters 30] [--only photometric,ssim,lcn,xcorrvol,proj_nn,nn,crosscheck]
 """
 import argparse
 import json
@@ -55,7 +55,7 @@ def timeit(fn, iters, warmup=5, nrep=NREP):
     return float(np.median(ts)), float(np.min(ts))
 
 
-ALL = "calib,photometric,warp,pyramid,geometric,disparity,lcn,xcorrvol,proj_nn,config4,nn,crosscheck,reduce,gpu_reference"
+ALL = "calib,photometric,ssim,warp,pyramid,geometric,disparity,lcn,xcorrvol,proj_nn,config4,nn,crosscheck,reduce,gpu_reference"
 
 
 def main():
@@ -117,6 +117,49 @@ def run(only=ALL, iters=30, batch=8, device_index=0, verbose=True):
                 _lib.call("ctd_photometric_bwd_f32", d["es"].data_ptr(), d["ta"].data_ptr(), d["go"].data_ptr(), d["o2"].data_ptr(), B, 1, H, W, 9, ty, 0.5, st)
             add(name + "_fwd", *timeit(f, args.iters), 12 * npx)
             add(name + "_bwd", *timeit(g, args.iters), 16 * npx)
+    if "ssim" in only:
+        # the SSIM loss (ssim.cu) at block 3 and 9: forward, backward, and the fused forward + backward + masked sums, against
+        # the usual torch formulation on the same GPU (avg_pool2d window moments over a replicate-padded copy, autograd backward)
+        gis = [torch.empty(B, 1, H, W, device=dev) for _ in range(NS)]
+        sums = torch.zeros(2, device=dev)
+        c1, c2 = tx.SSIM_C1, tx.SSIM_C2
+        for bs in (3, 9):
+            def f(i, st, bs=bs):
+                d = sets[i % NS]
+                _lib.call("ctd_ssim_fwd_f32", d["es"].data_ptr(), d["ta"].data_ptr(), d["o1"].data_ptr(), B, 1, H, W, bs, c1, c2, st)
+            def g(i, st, bs=bs):
+                d = sets[i % NS]
+                _lib.call("ctd_ssim_bwd_f32", d["es"].data_ptr(), d["ta"].data_ptr(), d["go"].data_ptr(), d["o2"].data_ptr(), B, 1, H, W, bs,
+                          c1, c2, st)
+            def h(i, st, bs=bs):
+                d = sets[i % NS]
+                _lib.call("ctd_ssim_fwd_bwd_masked_f32", d["es"].data_ptr(), d["ta"].data_ptr(), d["std"].data_ptr(), d["std"].data_ptr(),
+                          d["o1"].data_ptr(), gis[i % NS].data_ptr(), sums.data_ptr(), B, 1, H, W, bs, c1, c2, st)
+            add("ssim_bs%d_fwd" % bs, *timeit(f, args.iters), 12 * npx)
+            add("ssim_bs%d_bwd" % bs, *timeit(g, args.iters), 16 * npx)
+            add("ssim_bs%d_fwd_bwd_masked" % bs, *timeit(h, args.iters), 24 * npx)
+
+            def torch_ref(bs=bs):
+                pool = lambda t: torch.nn.functional.avg_pool2d(
+                    torch.nn.functional.pad(t, (bs // 2, bs - 1 - bs // 2, bs // 2, bs - 1 - bs // 2), mode="replicate"), bs, stride=1)
+                x = sets[0]["es"].detach().requires_grad_(True)
+                y, m = sets[0]["ta"], sets[0]["std"]
+                mx, my = pool(x), pool(y)
+                vxx, vyy, vxy = pool(x * x) - mx * mx, pool(y * y) - my * my, pool(x * y) - mx * my
+                s_ = (2 * mx * my + c1) * (2 * vxy + c2) / ((mx * mx + my * my + c1) * (vxx + vyy + c2))
+                ((m * (1 - s_) / 2).sum() / m.sum()).backward()
+            for _ in range(3):
+                torch_ref()
+            torch.cuda.synchronize()
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            for _ in range(10):
+                torch_ref()
+            e1.record()
+            torch.cuda.synchronize()
+            r = res["ops"]["ssim_bs%d_fwd_bwd_masked" % bs]
+            r["torch_eager_ms"] = e0.elapsed_time(e1) / 10
+            r["speedup_vs_torch_eager"] = r["torch_eager_ms"] / r["ms_median"]
     if "warp" in only:
         # SURVEY 8(f) rank 1: the disparity warp in front of the loss, and the whole RectifiedPatternSimilarityLoss step
         # (warp -> fused census_sad loss forward+backward+masked mean -> warp backward)
