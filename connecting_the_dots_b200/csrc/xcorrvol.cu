@@ -17,48 +17,112 @@ extern int g_xcorr_direct;
 extern int g_xcorr_nofix;
 extern int g_xcorr_hitcap;
 
-// generic: any C, any block size, float or double; one thread per output, reference operation order
-// (built with -fmad=false), so it reproduces the reference's two-pass centred statistics exactly.
+// generic: any C, any block size, float or double; one output, reference operation order (built with -fmad=false), so it
+// reproduces the reference's two-pass centred statistics exactly.  Shared by the volume and the disparity kernels.
+template <typename T>
+__device__ __forceinline__ T xcorr_generic_one(const T* __restrict__ in0, const T* __restrict__ in1, int64_t b, int C, int H,
+                                               int W, int h, int w, int d, int bs) {
+  const int half = bs / 2;
+  const T bs2 = (T)(bs * bs);
+  T val = 0;
+  for (int c = 0; c < C; ++c) {
+    const T* p0 = in0 + (b * C + c) * H * W;
+    const T* p1 = in1 + (b * C + c) * H * W;
+    T mu0 = 0, mu1 = 0;
+    for (int bh = 0; bh < bs; ++bh) {
+      const int64_t row = (int64_t)clampi(h + bh - half, 0, H - 1) * W;
+      for (int bw = 0; bw < bs; ++bw) {
+        const int w0 = w + bw - half;
+        mu0 += __ldg(p0 + row + clampi(w0, 0, W - 1)) / bs2;
+        mu1 += __ldg(p1 + row + clampi(w0 - d, 0, W - 1)) / bs2;
+      }
+    }
+    T s0 = 0, s1 = 0, dot = 0;
+    for (int bh = 0; bh < bs; ++bh) {
+      const int64_t row = (int64_t)clampi(h + bh - half, 0, H - 1) * W;
+      for (int bw = 0; bw < bs; ++bw) {
+        const int w0 = w + bw - half;
+        const T v0 = __ldg(p0 + row + clampi(w0, 0, W - 1)) - mu0;
+        const T v1 = __ldg(p1 + row + clampi(w0 - d, 0, W - 1)) - mu1;
+        dot += v0 * v1;
+        s0 += v0 * v0;
+        s1 += v1 * v1;
+      }
+    }
+    const T norm = (T)((double)sqrt(s0 * s1) + 1e-8);
+    val += dot / norm;
+  }
+  return val;
+}
+
+// one thread per output
 template <typename T>
 __global__ void __launch_bounds__(256)
 xcorrvol_generic(const T* __restrict__ in0, const T* __restrict__ in1, T* __restrict__ out, int64_t B, int C,
                  int H, int W, int D, int bs) {
   const int64_t total = B * D * H * W;
-  const int half = bs / 2;
-  const T bs2 = (T)(bs * bs);
   for (int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; idx < total;
        idx += (int64_t)gridDim.x * blockDim.x) {
     const int w = idx % W, h = (idx / W) % H, d = (idx / ((int64_t)W * H)) % D;
     const int64_t b = idx / ((int64_t)W * H * D);
-    T val = 0;
-    for (int c = 0; c < C; ++c) {
-      const T* p0 = in0 + (b * C + c) * H * W;
-      const T* p1 = in1 + (b * C + c) * H * W;
-      T mu0 = 0, mu1 = 0;
-      for (int bh = 0; bh < bs; ++bh) {
-        const int64_t row = (int64_t)clampi(h + bh - half, 0, H - 1) * W;
-        for (int bw = 0; bw < bs; ++bw) {
-          const int w0 = w + bw - half;
-          mu0 += __ldg(p0 + row + clampi(w0, 0, W - 1)) / bs2;
-          mu1 += __ldg(p1 + row + clampi(w0 - d, 0, W - 1)) / bs2;
-        }
+    out[idx] = xcorr_generic_one<T>(in0, in1, b, C, H, W, h, w, d, bs);
+  }
+}
+
+// ------------------------------------------------------------------------------------------
+// Winner-take-all disparity (ctd_xcorr_disparity_*): d* = the first d with V[d] = max_d V[d], score = V[d*].
+// Partial maxima merge through a 64-bit integer key: the order-preserving bits of the score above 0xFFFFFFFF - d, so
+// the unsigned maximum is the largest score and, among equal scores, the smallest d.  -0.0 is keyed as +0.0 (they
+// compare equal).  Key 0 is below every real key.
+// ------------------------------------------------------------------------------------------
+__device__ __forceinline__ unsigned long long wta_key(float v, int d) {
+  unsigned u = __float_as_uint(v);
+  if (u == 0x80000000u) u = 0u;
+  u = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+  return ((unsigned long long)u << 32) | (0xFFFFFFFFu - (unsigned)d);
+}
+__device__ __forceinline__ float wta_score(unsigned long long key) {
+  const unsigned u = (unsigned)(key >> 32);
+  return __uint_as_float((u & 0x80000000u) ? (u & 0x7FFFFFFFu) : ~u);
+}
+__device__ __forceinline__ int wta_disp(unsigned long long key, int D) {  // clamped: a key of 0 (no candidate) is never read out of range
+  return (int)min(0xFFFFFFFFu - (unsigned)key, (unsigned)(D - 1));
+}
+// three-point parabola through the scores at d* - 1, d*, d* + 1: vertex offset in [-0.5, 0.5], 0 unless the peak is strict
+// (den < 0); fp64 like disparity_from_volume
+__device__ __forceinline__ double wta_subpixel(double cm, double c0, double cp) {
+  const double den = cm - 2.0 * c0 + cp;
+  if (!(den < 0.0)) return 0.0;
+  return fmin(fmax((cm - cp) / (2.0 * den), -0.5), 0.5);
+}
+
+// generic disparity: one thread per pixel sweeps d with xcorr_generic_one, so d* and the score are the exact argmax and
+// maximum of xcorrvol_generic's volume
+template <typename T>
+__global__ void __launch_bounds__(256)
+xcorr_disparity_generic(const T* __restrict__ in0, const T* __restrict__ in1, T* __restrict__ disp, T* __restrict__ score,
+                        int64_t B, int C, int H, int W, int D, int bs, int subpixel) {
+  const int64_t total = B * H * W;
+  for (int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; idx < total;
+       idx += (int64_t)gridDim.x * blockDim.x) {
+    const int w = idx % W, h = (idx / W) % H;
+    const int64_t b = idx / ((int64_t)W * H);
+    T best = 0, prev = 0, cm = 0, cp = 0;  // cm, cp: V at best - 1 and best + 1
+    int bd = 0;
+    for (int d = 0; d < D; ++d) {
+      const T v = xcorr_generic_one<T>(in0, in1, b, C, H, W, h, w, d, bs);
+      if (d == 0 || v > best) {
+        best = v;
+        bd = d;
+        cm = prev;
+      } else if (d == bd + 1) {
+        cp = v;
       }
-      T s0 = 0, s1 = 0, dot = 0;
-      for (int bh = 0; bh < bs; ++bh) {
-        const int64_t row = (int64_t)clampi(h + bh - half, 0, H - 1) * W;
-        for (int bw = 0; bw < bs; ++bw) {
-          const int w0 = w + bw - half;
-          const T v0 = __ldg(p0 + row + clampi(w0, 0, W - 1)) - mu0;
-          const T v1 = __ldg(p1 + row + clampi(w0 - d, 0, W - 1)) - mu1;
-          dot += v0 * v1;
-          s0 += v0 * v0;
-          s1 += v1 * v1;
-        }
-      }
-      const T norm = (T)((double)sqrt(s0 * s1) + 1e-8);
-      val += dot / norm;
+      prev = v;
     }
-    out[idx] = val;
+    if (score) score[idx] = best;
+    const double delta = subpixel && bd > 0 && bd < D - 1 ? wta_subpixel((double)cm, (double)best, (double)cp) : 0.0;
+    disp[idx] = (T)((double)bd + delta);
   }
 }
 
@@ -293,6 +357,49 @@ __device__ __forceinline__ float xcorr_centred_one(const float* __restrict__ p0,
   return ((dot[0] + dot[1]) + dot[2]) / (sd0 * sd1 + 1e-8f);
 }
 
+// xcorr_centred_one at disparities d - 1, d, d + 1 in one pass (c[k] at d - 1 + k, the same arithmetic, so the same
+// values): the three in1 windows share BS - 1 of their BS + 1 columns, and the in0 window is common.
+template <int BS>
+__device__ __forceinline__ void xcorr_centred_three(const float* __restrict__ p0, const float* __restrict__ p1, int H, int W,
+                                                    int h, int w, int d, float mu0, float sd0, const float (&mu1)[3],
+                                                    const float (&sd1)[3], float (&c)[3]) {
+  constexpr int R = BS / 2;
+  unsigned ca[BS], cb[BS + 2];  // byte offsets of the clamped columns; tap bw of disparity d - 1 + k is in1 column cb[bw + 2 - k]
+#pragma unroll
+  for (int bw = 0; bw < BS; ++bw) ca[bw] = 4u * (unsigned)clampi(w + bw - R, 0, W - 1);
+#pragma unroll
+  for (int j = 0; j < BS + 2; ++j) cb[j] = 4u * (unsigned)clampi(w + j - R - d - 1, 0, W - 1);
+  const char* q0 = reinterpret_cast<const char*>(p0);
+  const char* q1 = reinterpret_cast<const char*>(p1);
+  // rows accumulate into dot[k][bh % 3] as in xcorr_centred_one; the loop stays rolled (registers), so the row's slot is
+  // always dot[k][0] and the slots rotate after each row
+  float dot[3][3] = {};
+#pragma unroll 1
+  for (int bh = 0; bh < BS; ++bh) {
+    const int64_t row = (int64_t)clampi(h + bh - R, 0, H - 1) * W * 4;
+    float bv[BS + 2];
+#pragma unroll
+    for (int j = 0; j < BS + 2; ++j) bv[j] = __ldg(reinterpret_cast<const float*>(q1 + row + cb[j]));
+#pragma unroll
+    for (int bw = 0; bw < BS; ++bw) {
+      const float av = __ldg(reinterpret_cast<const float*>(q0 + row + ca[bw])) - mu0;
+#pragma unroll
+      for (int k = 0; k < 3; ++k) dot[k][0] = fmaf(av, bv[bw + 2 - k] - mu1[k], dot[k][0]);
+    }
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      const float t = dot[k][0];
+      dot[k][0] = dot[k][1];
+      dot[k][1] = dot[k][2];
+      dot[k][2] = t;
+    }
+  }
+  // slot j (rows bh = j mod 3) now sits at position (j - BS) mod 3
+  constexpr int P0 = (0 + 3 - BS % 3) % 3, P1 = (1 + 3 - BS % 3) % 3, P2 = (2 + 3 - BS % 3) % 3;
+#pragma unroll
+  for (int k = 0; k < 3; ++k) c[k] = ((dot[k][P0] + dot[k][P1]) + dot[k][P2]) / (sd0 * sd1[k] + 1e-8f);
+}
+
 // Window statistics of one image over positions i = u + uoff, u = column of the window centre (may be
 // negative: replicate padding).  st_out = {scale * mean, sqrt(sum (v - mean)^2)} interleaved, grade_out = L.
 // Windows with L >= XS_LLIST are appended to `list` as (side | position).
@@ -421,11 +528,19 @@ __device__ __forceinline__ void xs_hsum9_fma(const float* a, const float* b, flo
 // TD = disparities per thread.  TD = 4: 128 threads, 246 registers (suffix sums of 16 outputs), 8 warps/SM.
 // TD = 2: 256 threads, half the suffix registers, 16 warps/SM -- the tile and the arithmetic per output are the
 // same, the resident warps double (the kernel is latency-bound), the in1 row is read as seven 64-bit loads.
-template <int BS, int TD, bool VEC>
+//
+// Out = float: the volume.  Out = unsigned long long: the winner-take-all variant -- the same outputs, but instead of
+// being stored each is a candidate for its pixel's maximum: a thread keeps the best of its TD disparities per column and
+// merges it into the key plane `out` [B,H,W] with a 64-bit integer atomicMax (wta_key) per column and output row.  (A
+// key tile in shared memory that merged the CTA's warps first cost 38 KB of shared memory per CTA and compiled to
+// compare-and-swap loops: measured slower, 751 against 674 us at block 9, batch 8.)  Outputs the fix-up recomputes
+// (L0 + L1 >= XS_LSUM, grades g0 / g1 of the statistics pass) take no part: their fast-path value can be far off.
+template <int BS, int TD, bool VEC, typename Out>
 __global__ void __launch_bounds__(512 / TD, 2)
-xcorr_sep_kernel(const float* __restrict__ in0, const float* __restrict__ in1, float* __restrict__ out,
-                 const float2* __restrict__ st0, const float2* __restrict__ st1, int H, int W, int D, int ws0, int ws1,
-                 int uoff, int ndchunks) {
+xcorr_sep_kernel(const float* __restrict__ in0, const float* __restrict__ in1, Out* __restrict__ out,
+                 const float2* __restrict__ st0, const float2* __restrict__ st1, const uint8_t* __restrict__ g0,
+                 const uint8_t* __restrict__ g1, int H, int W, int D, int ws0, int ws1, int uoff, int ndchunks) {
+  constexpr bool WTA = std::is_same<Out, unsigned long long>::value;
   constexpr int R = BS / 2, TH = XsCfg<BS>::TH, XH = XsCfg<BS>::XH, NBLK = XsCfg<BS>::NBLK;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float(*At)[XS_AW] = reinterpret_cast<float(*)[XS_AW]>(smem_raw);
@@ -498,10 +613,30 @@ xcorr_sep_kernel(const float* __restrict__ in0, const float* __restrict__ in1, f
   const float* brow = &Bt[0][4 * lane + 16 - BOFF - TD * g];
   // store pointer of the row being emitted (tile row r -> output row y0 + r - 2R), advanced by W per row: no
   // 64-bit index arithmetic inside the loop
-  float* orow = out + (((int64_t)b * D + dbase) * H + (y0 - 2 * R)) * W + x;
+  // (WTA: the key plane [B,H,W] -- this lane's four keys of the row)
+  Out* orow = out + ((WTA ? (int64_t)b * H : ((int64_t)b * D + dbase) * H) + (y0 - 2 * R)) * W + x;
   const int64_t dstride = (int64_t)H * W;
   const int ndl = min(TD, D - dbase);  // disparities of this warp that exist
   const bool xin = VEC ? x < W : true;
+  // WTA: grades of the lane's four w positions (gr[0], a byte each) and of its eight u positions (gr[1], gr[2]) in an
+  // output row; a lane whose columns lie outside the image keeps 0xff grades (no candidates)
+  const uint8_t* g0row = WTA ? g0 + ((int64_t)b * H + y0) * ws0 + x : nullptr;
+  const uint8_t* g1row = WTA ? g1 + ((int64_t)b * H + y0) * ws1 + (x - dbase - 4 + uoff) : nullptr;
+  unsigned grn[3] = {~0u, ~0u, ~0u};  // WTA: grades of the next output row, loaded one row ahead (the L2 round trip
+                                     // overlaps a row of arithmetic)
+  auto load_grades = [&](int e, unsigned (&gr)[3]) {
+    const uint8_t* p0 = g0row + (int64_t)e * ws0;
+    const uint8_t* p1 = g1row + (int64_t)e * ws1;
+    gr[0] = __ldg(reinterpret_cast<const unsigned*>(p0));
+    if (TD == 4) {  // 4-byte aligned: x, dbase, uoff and the row strides are multiples of 4
+      gr[1] = __ldg(reinterpret_cast<const unsigned*>(p1));
+      gr[2] = __ldg(reinterpret_cast<const unsigned*>(p1 + 4));
+    } else {
+      gr[1] = gr[2] = 0u;
+#pragma unroll
+      for (int j = 0; j < 8; ++j) gr[1 + j / 4] |= (unsigned)__ldg(p1 + j) << (8 * (j % 4));
+    }
+  };
   // Window statistics of the output rows stream through a per-warp shared-memory ring: one lane fetches a
   // row's w-side {N*mu0, sd0} (128 positions) and u-side {mu1, sd1} (136 positions u = x0-dbase-4 ..) with two
   // cp.async.bulk copies, NST rows ahead, completion on an mbarrier -- no registers are held across the
@@ -540,6 +675,7 @@ xcorr_sep_kernel(const float* __restrict__ in0, const float* __restrict__ in1, f
   for (int e = 0; e < NST; ++e)
     if (e < nrows) issue(e);
   __syncwarp();
+  if (WTA && x < W) load_grades(0, grn);
   // the pieces of a row step shared by the two vertical-sum schemes below
   auto load_ab = [&](int r, float (&a)[12], float (&bv)[16]) {
     const float4* ap = reinterpret_cast<const float4*>(arow + r * XS_AW);
@@ -589,20 +725,36 @@ xcorr_sep_kernel(const float* __restrict__ in0, const float* __restrict__ in1, f
   };
   // lane's four columns: {N*mu0, sd0} pairs; its eight u positions (x - dbase - 4 ..): {mu1, sd1} pairs, of which
   // disparity dbase + dl uses positions 4 + k - dl
-  auto emit_out = [&](int dl, const float (&S)[4], const float2 (&wst)[4], const float2 (&ust)[8]) {
+  // WTA: best[k] = the largest trusted output of column k so far in this row, byte k of bestdl = 1 + its dl (0: none yet);
+  // ascending dl and a strict comparison keep the smallest d among equal scores
+  auto emit_out = [&](int dl, const float (&S)[4], const float2 (&wst)[4], const float2 (&ust)[8], const unsigned (&gr)[3],
+                      float (&best)[4], unsigned& bestdl) {
     float v[4];
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
       const float2 ws_ = wst[k], us_ = ust[4 + k - dl];
       v[k] = fmaf(-ws_.x, us_.x, S[k]) * rcp_approx(fmaf(ws_.y, us_.y, 1e-8f));  // untrusted outputs: see fix-up
     }
-    float* dst = orow + dl * dstride;
-    if (VEC) {
-      if (xin && dl < ndl) __stcs(reinterpret_cast<float4*>(dst), make_float4(v[0], v[1], v[2], v[3]));
-    } else {
+    if constexpr (WTA) {
 #pragma unroll
-      for (int k = 0; k < 4; ++k)
-        if (x + k < W && dl < ndl) dst[k] = v[k];
+      for (int k = 0; k < 4; ++k) {
+        const int j = 4 + k - dl;  // u position of column k at this disparity
+        const unsigned L0 = (gr[0] >> (8 * k)) & 255u, L1 = (gr[1 + j / 4] >> (8 * (j % 4))) & 255u;
+        const bool ok = (VEC ? xin : x + k < W) && dl < ndl && L0 + L1 < (unsigned)XS_LSUM;
+        if (ok && v[k] > best[k]) {
+          best[k] = v[k];
+          bestdl = (bestdl & ~(255u << (8 * k))) | ((unsigned)(dl + 1) << (8 * k));
+        }
+      }
+    } else {
+      float* dst = orow + dl * dstride;
+      if (VEC) {
+        if (xin && dl < ndl) __stcs(reinterpret_cast<float4*>(dst), make_float4(v[0], v[1], v[2], v[3]));
+      } else {
+#pragma unroll
+        for (int k = 0; k < 4; ++k)
+          if (x + k < W && dl < ndl) dst[k] = v[k];
+      }
     }
   };
   // One block of BS tile rows.  FIRST: the tile's first block only fills the vertical state (its last row
@@ -616,6 +768,14 @@ xcorr_sep_kernel(const float* __restrict__ in0, const float* __restrict__ in1, f
       const bool emit = !FIRST || j == BS - 1;  // compile-time after unrolling
       const int e = r - 2 * R;                  // output row of the tile completed by tile row r
       if (emit && e >= nrows) return true;      // warp-uniform
+      unsigned gr[3] = {grn[0], grn[1], grn[2]};
+      float best[4];
+      unsigned bestdl = 0u;
+      if (WTA && emit) {
+        if (x < W && e + 1 < nrows) load_grades(e + 1, grn);
+#pragma unroll
+        for (int k = 0; k < 4; ++k) best[k] = -INFINITY;
+      }
       float a[12], bv[16];
       load_ab(r, a, bv);
       // stage of this row's statistics: static when NST divides BS
@@ -669,9 +829,16 @@ xcorr_sep_kernel(const float* __restrict__ in0, const float* __restrict__ in1, f
           }
         }
 #endif
-        if (emit) emit_out(dl, S, wst, ust);
+        if (emit) emit_out(dl, S, wst, ust, gr, best, bestdl);
       }
       if (emit) {  // every lane has read this stage: hand it to the row NST further down
+        if constexpr (WTA) {
+#pragma unroll
+          for (int k = 0; k < 4; ++k) {
+            const unsigned dl1 = (bestdl >> (8 * k)) & 255u;
+            if (dl1 != 0u) atomicMax(orow + k, wta_key(best[k], dbase + (int)dl1 - 1));
+          }
+        }
         __syncwarp();
         if (nissued < nrows) issue(st);
       }
@@ -685,10 +852,34 @@ xcorr_sep_kernel(const float* __restrict__ in0, const float* __restrict__ in1, f
     if (do_block(std::false_type{}, blk)) return;
 }
 
-// Recompute one untrusted output: centred form with the statistics pass's means, or the reference arithmetic
+// One output in the fix-up's arithmetic: centred form with the statistics pass's means, or the reference arithmetic
 // where a window is flat.
 template <int BS>
-__device__ __forceinline__ void xcorr_fix_one(const float* __restrict__ in0, const float* __restrict__ in1, float* __restrict__ out,
+__device__ __forceinline__ float xcorr_fixed_value(const float* __restrict__ in0, const float* __restrict__ in1,
+                                                   const float2* __restrict__ st0, const float2* __restrict__ st1,
+                                                   const uint8_t* __restrict__ g0, const uint8_t* __restrict__ g1, int64_t b,
+                                                   int h, int w, int d, int H, int W, int ws0, int ws1, int uoff) {
+  const int64_t plane = (int64_t)H * W;
+  const int64_t i0 = (b * H + h) * ws0 + w, i1 = (b * H + h) * ws1 + (w - d + uoff);
+  if (g0[i0] >= XS_LEXACT || g1[i1] >= XS_LEXACT) return xcorr_exact_one<BS>(in0 + b * plane, in1 + b * plane, H, W, h, w, d);
+  const float2 s0 = __ldg(st0 + i0), s1 = __ldg(st1 + i1);  // {N mu0, sd0}, {mu1, sd1}
+  return xcorr_centred_one<BS>(in0 + b * plane, in1 + b * plane, H, W, h, w, d, s0.x * (1.0f / float(BS * BS)), s1.x, s0.y,
+                               s1.y);
+}
+
+// where a recomputed output goes: the volume, or (winner-take-all) its pixel's key
+__device__ __forceinline__ void xcorr_put(float* __restrict__ out, unsigned bd, int64_t b, int d, int64_t plane, unsigned hw,
+                                          float v) {
+  out[(int64_t)bd * plane + hw] = v;
+}
+__device__ __forceinline__ void xcorr_put(unsigned long long* __restrict__ keys, unsigned bd, int64_t b, int d, int64_t plane,
+                                          unsigned hw, float v) {
+  atomicMax(keys + b * plane + hw, wta_key(v, d));
+}
+
+// Recompute one untrusted output.
+template <int BS, typename Out>
+__device__ __forceinline__ void xcorr_fix_one(const float* __restrict__ in0, const float* __restrict__ in1, Out* __restrict__ out,
                                               const float2* __restrict__ st0, const float2* __restrict__ st1,
                                               const uint8_t* __restrict__ g0, const uint8_t* __restrict__ g1,
                                               unsigned long long e, int H, int W, int D, int ws0, int ws1, int uoff) {
@@ -697,16 +888,7 @@ __device__ __forceinline__ void xcorr_fix_one(const float* __restrict__ in0, con
   const int w = (int)(hw % (unsigned)W), h = (int)(hw / (unsigned)W);
   const int d = (int)(bd % (unsigned)D);
   const int64_t b = bd / (unsigned)D;
-  const int64_t i0 = (b * H + h) * ws0 + w, i1 = (b * H + h) * ws1 + (w - d + uoff);
-  float v;
-  if (g0[i0] >= XS_LEXACT || g1[i1] >= XS_LEXACT) {
-    v = xcorr_exact_one<BS>(in0 + b * plane, in1 + b * plane, H, W, h, w, d);
-  } else {
-    const float2 s0 = __ldg(st0 + i0), s1 = __ldg(st1 + i1);  // {N mu0, sd0}, {mu1, sd1}
-    v = xcorr_centred_one<BS>(in0 + b * plane, in1 + b * plane, H, W, h, w, d, s0.x * (1.0f / float(BS * BS)), s1.x, s0.y,
-                              s1.y);
-  }
-  out[(int64_t)bd * plane + hw] = v;
+  xcorr_put(out, bd, b, d, plane, hw, xcorr_fixed_value<BS>(in0, in1, st0, st1, g0, g1, b, h, w, d, H, W, ws0, ws1, uoff));
 }
 
 // Fix-up, step 1: which outputs are untrusted.  A listed window (side 0: window of in0 at (h, w) -> outputs
@@ -786,9 +968,9 @@ xcorr_sweep_kernel(const uint8_t* __restrict__ g0, const uint8_t* __restrict__ g
 
 // Fix-up, step 2: one thread per untrusted output (neighbouring hits are neighbouring disparities of one window, so
 // the gathers of a warp stay within a few cache lines).
-template <int BS>
+template <int BS, typename Out>
 __global__ void __launch_bounds__(256)
-xcorr_eval_kernel(const float* __restrict__ in0, const float* __restrict__ in1, float* __restrict__ out,
+xcorr_eval_kernel(const float* __restrict__ in0, const float* __restrict__ in1, Out* __restrict__ out,
                   const float2* __restrict__ st0, const float2* __restrict__ st1, const uint8_t* __restrict__ g0,
                   const uint8_t* __restrict__ g1, const unsigned long long* __restrict__ hits, const unsigned* __restrict__ nhits,
                   unsigned cap, int H, int W, int D, int ws0, int ws1, int uoff) {
@@ -806,9 +988,9 @@ xcorr_eval_kernel(const float* __restrict__ in0, const float* __restrict__ in1, 
 // image.  An output is owned by the side with the larger grade (side 0 on ties) so it is done once.
 // Affected outputs are queued per warp and evaluated 32 at a time, so the expensive path runs with full
 // warps however sparse the hits are.
-template <int BS>
+template <int BS, typename Out>
 __global__ void __launch_bounds__(256)
-xcorr_fixup_kernel(const float* __restrict__ in0, const float* __restrict__ in1, float* __restrict__ out,
+xcorr_fixup_kernel(const float* __restrict__ in0, const float* __restrict__ in1, Out* __restrict__ out,
                    const float2* __restrict__ st0, const float2* __restrict__ st1, const uint8_t* __restrict__ g0,
                    const uint8_t* __restrict__ g1, const unsigned* __restrict__ list, const unsigned* __restrict__ count,
                    const unsigned* __restrict__ nhits, unsigned cap, int H, int W, int D, int ws0, int ws1, int uoff) {
@@ -861,6 +1043,56 @@ xcorr_fixup_kernel(const float* __restrict__ in0, const float* __restrict__ in1,
   if (nq > 0) drain(nq);
 }
 
+// c[k] = xcorr_fixed_value at d - 1 + k: the rare case of a flat window among the three, kept out of line so that its
+// registers do not count against the common path of xcorr_wta_finish_kernel
+template <int BS>
+__device__ __noinline__ void xcorr_fixed_three(const float* __restrict__ in0, const float* __restrict__ in1,
+                                               const float2* __restrict__ st0, const float2* __restrict__ st1,
+                                               const uint8_t* __restrict__ g0, const uint8_t* __restrict__ g1, int64_t b, int h,
+                                               int w, int d, int H, int W, int ws0, int ws1, int uoff, float (&c)[3]) {
+#pragma unroll 1
+  for (int k = 0; k < 3; ++k) c[k] = xcorr_fixed_value<BS>(in0, in1, st0, st1, g0, g1, b, h, w, d - 1 + k, H, W, ws0, ws1, uoff);
+}
+
+// Winner-take-all, last pass: one thread per pixel decodes d* and the score from its key.  The sub-pixel parabola takes
+// the scores at d* - 1, d*, d* + 1 in the fix-up's arithmetic (xcorr_fixed_value: centred form, reference arithmetic
+// for flat windows; the three centred ones in one pass) instead of keeping neighbours of every candidate.
+template <int BS>
+__global__ void __launch_bounds__(256, 3)
+xcorr_wta_finish_kernel(const float* __restrict__ in0, const float* __restrict__ in1, const float2* __restrict__ st0,
+                        const float2* __restrict__ st1, const uint8_t* __restrict__ g0, const uint8_t* __restrict__ g1,
+                        const unsigned long long* __restrict__ keys, float* __restrict__ disp, float* __restrict__ score,
+                        int64_t npix, int H, int W, int D, int ws0, int ws1, int uoff, int subpixel) {
+  for (int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; idx < npix; idx += (int64_t)gridDim.x * blockDim.x) {
+    const unsigned long long key = keys[idx];
+    const int d = wta_disp(key, D);
+    if (score) score[idx] = wta_score(key);
+    double delta = 0.0;
+    if (subpixel && d > 0 && d < D - 1) {
+      const int w = (int)(idx % W), h = (int)((idx / W) % H);
+      const int64_t b = idx / ((int64_t)W * H);
+      const int64_t i0 = (b * H + h) * ws0 + w, i1 = (b * H + h) * ws1 + (w - d + uoff);  // in1 window of d - 1 + k: i1 + 1 - k
+      float c[3];
+      if (g0[i0] >= XS_LEXACT || g1[i1 - 1] >= XS_LEXACT || g1[i1] >= XS_LEXACT || g1[i1 + 1] >= XS_LEXACT) {
+        xcorr_fixed_three<BS>(in0, in1, st0, st1, g0, g1, b, h, w, d, H, W, ws0, ws1, uoff, c);
+      } else {
+        const float2 s0 = __ldg(st0 + i0);
+        float mu1[3], sd1[3];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+          const float2 s1 = __ldg(st1 + i1 + 1 - k);
+          mu1[k] = s1.x;
+          sd1[k] = s1.y;
+        }
+        const int64_t plane = (int64_t)H * W;
+        xcorr_centred_three<BS>(in0 + b * plane, in1 + b * plane, H, W, h, w, d, s0.x * (1.0f / float(BS * BS)), s0.y, mu1, sd1, c);
+      }
+      delta = wta_subpixel(c[0], c[1], c[2]);
+    }
+    disp[idx] = (float)((double)d + delta);
+  }
+}
+
 // a non-blocking side stream and four events per host thread and device, for the fork / join inside one call
 struct SideStream {
   cudaStream_t stream = nullptr;
@@ -890,9 +1122,17 @@ static SideStream* side_stream() {
   return &s;
 }
 
+// Winner-take-all outputs of one launch (ctd_xcorr_disparity_f32): [B,1,H,W] each; score may be null.
+struct XcorrWta {
+  float* disp;
+  float* score;
+  int subpixel;
+};
+
+// One launch of the separable path for B images: the volume into `out`, or with `wta` the winner-take-all disparity.
 template <int BS>
 static bool xcorr_sep_launch(const float* in0, const float* in1, float* out, int64_t B, int64_t H, int64_t W, int64_t D,
-                             cudaStream_t st) {
+                             cudaStream_t st, const XcorrWta* wta = nullptr) {
   constexpr int R = BS / 2, XH = XsCfg<BS>::XH, TH = XsCfg<BS>::TH;
   const int64_t ndchunks = cdiv(D, XS_DT);
   const int64_t uoff = ndchunks * XS_DT, ws0 = cdiv(W, 4) * 4, ws1 = uoff + ws0;
@@ -903,11 +1143,14 @@ static bool xcorr_sep_launch(const float* in0, const float* in1, float* out, int
   // entries block 5 overflowed at batch 8 and ran the fallback kernel, 986 instead of 752 us (xcorr_hitcap_bs5.py).
   // g_xcorr_hitcap >= 0 overrides (tests force the overflow path with 0)
   const int64_t cap = (g_xcorr_hitcap >= 0 ? g_xcorr_hitcap : std::min<int64_t>(B * D * H * W / 32 + 1024, (int64_t)1 << 24)) / 2 * 2;  // even: the statistics planes behind it stay 16-byte aligned
-  const size_t words = (size_t)(2 * cap) + (size_t)(3 * n0 + 3 * n1 + 4) + (size_t)(n0 + n1 + 3) / 4;
+  // winner-take-all: one 64-bit key per pixel, an even count for the same reason
+  const int64_t nkeys = wta ? (B * H * W + 1) / 2 * 2 : 0;
+  const size_t words = (size_t)(2 * cap + 2 * nkeys) + (size_t)(3 * n0 + 3 * n1 + 4) + (size_t)(n0 + n1 + 3) / 4;
   float* scratch = static_cast<float*>(scratch_alloc(words * sizeof(float), st));
   if (!scratch) return false;
   unsigned long long* hits = reinterpret_cast<unsigned long long*>(scratch);  // 8-byte aligned: first
-  float2* st0 = reinterpret_cast<float2*>(hits + cap);
+  unsigned long long* keys = hits + cap;
+  float2* st0 = reinterpret_cast<float2*>(keys + nkeys);
   float2* st1 = st0 + n0;
   unsigned* list = reinterpret_cast<unsigned*>(st1 + n1);
   unsigned* count = list + n0 + n1;  // count[0]: listed windows, count[1]: untrusted outputs
@@ -915,62 +1158,82 @@ static bool xcorr_sep_launch(const float* in0, const float* in1, float* out, int
   uint8_t* g1 = g0 + n0;
   const size_t st_smem = sizeof(double) * 2 * (ST_H + 2 * R) * ST_W + sizeof(float) * (ST_H + 2 * R) * (ST_W + 2 * R);
   constexpr int TD = XS_TD;
-  const size_t smem = sizeof(float) * TH * (XS_AW + XS_BW) + (16 / TD) * sizeof(XsStatRing<XsNst<TD>::value>);
-  // the attribute belongs to the device (context), not to the process: set it on every call (a process may use several GPUs)
-  const bool attr_ok =
-      cudaFuncSetAttribute(xcorr_stats_kernel<BS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)st_smem) == cudaSuccess &&
-      cudaFuncSetAttribute(xcorr_sep_kernel<BS, TD, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) == cudaSuccess &&
-      cudaFuncSetAttribute(xcorr_sep_kernel<BS, TD, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) == cudaSuccess;
-  if (!attr_ok || cudaMemsetAsync(count, 0, 2 * sizeof(unsigned), st) != cudaSuccess) {
-    cudaGetLastError();
-    scratch_free(scratch, st);
-    return false;
-  }
-  // Fork / join inside the call (legal under stream capture: the side stream joins the capture through the events): the
-  // statistics of the two images run side by side, and the sweep over the listed windows -- which needs only the grades
-  // -- runs beside the main kernel instead of behind it.  The side stream and the events belong to the calling thread.
-  SideStream* ss = side_stream();
-  const bool fork = ss != nullptr && !g_xcorr_serial;
-  cudaStream_t sd = fork ? ss->stream : st;
-  if (fork) {
-    cudaEventRecord(ss->ev[0], st);
-    cudaStreamWaitEvent(sd, ss->ev[0], 0);
-  }
-  xcorr_stats_kernel<BS><<<dim3((unsigned)cdiv(ws1, ST_W), (unsigned)cdiv(H, ST_H), (unsigned)B), 256, st_smem, sd>>>(
-      in1, st1, g1, (int)H, (int)W, (int)ws1, (int)uoff, 1.0f, 0x80000000u, list, count);
-  xcorr_stats_kernel<BS><<<dim3((unsigned)cdiv(ws0, ST_W), (unsigned)cdiv(H, ST_H), (unsigned)B), 256, st_smem, st>>>(
-      in0, st0, g0, (int)H, (int)W, (int)ws0, 0, float(BS * BS), 0u, list, count);
-  if (fork) {
-    cudaEventRecord(ss->ev[1], sd);
-    cudaStreamWaitEvent(st, ss->ev[1], 0);   // the main kernel needs both statistics planes
-    cudaEventRecord(ss->ev[2], st);
-    cudaStreamWaitEvent(sd, ss->ev[2], 0);   // ... and so does the sweep
-  }
-  const int vec = (W % 4 == 0) && !((reinterpret_cast<uintptr_t>(in0) | reinterpret_cast<uintptr_t>(in1) |
-                                     reinterpret_cast<uintptr_t>(out)) & 15);
-  const dim3 sgrid((unsigned)cdiv(W, XS_W), (unsigned)cdiv(H, XH), (unsigned)(B * ndchunks));
-  if (!g_xcorr_nofix)
-    xcorr_sweep_kernel<<<148 * 8, 256, 0, sd>>>(g0, g1, list, count, hits, count + 1, (unsigned)cap, (int)H, (int)W, (int)D,
-                                               (int)ws0, (int)ws1, (int)uoff);
-  if (vec)
-    xcorr_sep_kernel<BS, TD, true><<<sgrid, 512 / TD, smem, st>>>(in0, in1, out, st0, st1, (int)H, (int)W, (int)D, (int)ws0,
-                                                                 (int)ws1, (int)uoff, (int)ndchunks);
-  else
-    xcorr_sep_kernel<BS, TD, false><<<sgrid, 512 / TD, smem, st>>>(in0, in1, out, st0, st1, (int)H, (int)W, (int)D, (int)ws0,
-                                                                  (int)ws1, (int)uoff, (int)ndchunks);
-  if (fork) {
-    cudaEventRecord(ss->ev[3], sd);
-    cudaStreamWaitEvent(st, ss->ev[3], 0);   // join: the evaluation of the hits overwrites outputs of the main kernel
-  }
-  if (!g_xcorr_nofix) {
-    xcorr_eval_kernel<BS><<<148 * 8, 256, 0, st>>>(in0, in1, out, st0, st1, g0, g1, hits, count + 1, (unsigned)cap, (int)H,
-                                                  (int)W, (int)D, (int)ws0, (int)ws1, (int)uoff);
-    xcorr_fixup_kernel<BS><<<148 * 3, 256, 0, st>>>(in0, in1, out, st0, st1, g0, g1, list, count, count + 1, (unsigned)cap,
-                                                   (int)H, (int)W, (int)D, (int)ws0, (int)ws1, (int)uoff);
-  }
-  count_launch(g_xcorr_nofix ? 3 : 6);
+  // o: the volume (float) or the key plane (unsigned long long); the kernels are instantiated for its type
+  auto run = [&](auto* o) -> bool {
+    using Out = std::remove_pointer_t<decltype(o)>;
+    constexpr bool WTA = std::is_same<Out, unsigned long long>::value;
+    const bool fix = WTA || !g_xcorr_nofix;  // the disparity needs the fix-up: untrusted outputs are not in the main kernel's maximum
+    const size_t smem = sizeof(float) * TH * (XS_AW + XS_BW) + (16 / TD) * sizeof(XsStatRing<XsNst<TD>::value>);
+    // the attribute belongs to the device (context), not to the process: set it on every call (a process may use several GPUs)
+    const bool attr_ok =
+        cudaFuncSetAttribute(xcorr_stats_kernel<BS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)st_smem) == cudaSuccess &&
+        cudaFuncSetAttribute(xcorr_sep_kernel<BS, TD, true, Out>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) == cudaSuccess &&
+        cudaFuncSetAttribute(xcorr_sep_kernel<BS, TD, false, Out>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) == cudaSuccess;
+    if (!attr_ok || cudaMemsetAsync(count, 0, 2 * sizeof(unsigned), st) != cudaSuccess ||
+        (WTA && cudaMemsetAsync(keys, 0, sizeof(unsigned long long) * nkeys, st) != cudaSuccess)) {
+      cudaGetLastError();
+      return false;
+    }
+    // Fork / join inside the call (legal under stream capture: the side stream joins the capture through the events): the
+    // statistics of the two images run side by side, and the sweep over the listed windows -- which needs only the grades
+    // -- runs beside the main kernel instead of behind it.  The side stream and the events belong to the calling thread.
+    SideStream* ss = side_stream();
+    const bool fork = ss != nullptr && !g_xcorr_serial;
+    cudaStream_t sd = fork ? ss->stream : st;
+    if (fork) {
+      cudaEventRecord(ss->ev[0], st);
+      cudaStreamWaitEvent(sd, ss->ev[0], 0);
+    }
+    xcorr_stats_kernel<BS><<<dim3((unsigned)cdiv(ws1, ST_W), (unsigned)cdiv(H, ST_H), (unsigned)B), 256, st_smem, sd>>>(
+        in1, st1, g1, (int)H, (int)W, (int)ws1, (int)uoff, 1.0f, 0x80000000u, list, count);
+    xcorr_stats_kernel<BS><<<dim3((unsigned)cdiv(ws0, ST_W), (unsigned)cdiv(H, ST_H), (unsigned)B), 256, st_smem, st>>>(
+        in0, st0, g0, (int)H, (int)W, (int)ws0, 0, float(BS * BS), 0u, list, count);
+    if (fork) {
+      cudaEventRecord(ss->ev[1], sd);
+      cudaStreamWaitEvent(st, ss->ev[1], 0);   // the main kernel needs both statistics planes
+      cudaEventRecord(ss->ev[2], st);
+      cudaStreamWaitEvent(sd, ss->ev[2], 0);   // ... and so does the sweep
+    }
+    const int vec = (W % 4 == 0) && !((reinterpret_cast<uintptr_t>(in0) | reinterpret_cast<uintptr_t>(in1) |
+                                       (WTA ? 0 : reinterpret_cast<uintptr_t>(o))) & 15);
+    const dim3 sgrid((unsigned)cdiv(W, XS_W), (unsigned)cdiv(H, XH), (unsigned)(B * ndchunks));
+    if (fix)
+      xcorr_sweep_kernel<<<148 * 8, 256, 0, sd>>>(g0, g1, list, count, hits, count + 1, (unsigned)cap, (int)H, (int)W, (int)D,
+                                                 (int)ws0, (int)ws1, (int)uoff);
+    if (vec)
+      xcorr_sep_kernel<BS, TD, true, Out><<<sgrid, 512 / TD, smem, st>>>(in0, in1, o, st0, st1, g0, g1, (int)H, (int)W, (int)D,
+                                                                        (int)ws0, (int)ws1, (int)uoff, (int)ndchunks);
+    else
+      xcorr_sep_kernel<BS, TD, false, Out><<<sgrid, 512 / TD, smem, st>>>(in0, in1, o, st0, st1, g0, g1, (int)H, (int)W, (int)D,
+                                                                         (int)ws0, (int)ws1, (int)uoff, (int)ndchunks);
+    if (fork) {
+      cudaEventRecord(ss->ev[3], sd);
+      cudaStreamWaitEvent(st, ss->ev[3], 0);   // join: the evaluation of the hits overwrites outputs of the main kernel
+    }
+    if (fix) {
+      xcorr_eval_kernel<BS, Out><<<148 * 8, 256, 0, st>>>(in0, in1, o, st0, st1, g0, g1, hits, count + 1, (unsigned)cap, (int)H,
+                                                         (int)W, (int)D, (int)ws0, (int)ws1, (int)uoff);
+      xcorr_fixup_kernel<BS, Out><<<148 * 3, 256, 0, st>>>(in0, in1, o, st0, st1, g0, g1, list, count, count + 1, (unsigned)cap,
+                                                          (int)H, (int)W, (int)D, (int)ws0, (int)ws1, (int)uoff);
+    }
+    if constexpr (WTA) {
+      const int64_t npix = B * H * W;
+      xcorr_wta_finish_kernel<BS><<<(unsigned)std::min<int64_t>(cdiv(npix, 256), 148 * 16), 256, 0, st>>>(
+          in0, in1, st0, st1, g0, g1, o, wta->disp, wta->score, npix, (int)H, (int)W, (int)D, (int)ws0, (int)ws1, (int)uoff,
+          wta->subpixel);
+    }
+    count_launch(WTA ? 7 : fix ? 6 : 3);
+    return true;
+  };
+  const bool ok = wta ? run(keys) : run(out);
   scratch_free(scratch, st);
-  return true;
+  return ok;
+}
+
+// Images per separable launch: as many as keep the fix-up's hit list (1/32 of the outputs, 16 M entries at most) at its
+// full relative size (see xcorrvol_impl).
+static int64_t xcorr_images_per_launch(int64_t D, int64_t H, int64_t W) {
+  return std::max<int64_t>(1, (((int64_t)1 << 24) - 1024) * 32 / std::max<int64_t>(D * H * W, 1));
 }
 
 template <typename T>
@@ -990,7 +1253,7 @@ static int xcorrvol_impl(const T* in0, const T* in1, T* out, int64_t B, int64_t 
     // relative size -- a large batch in one launch would overflow the list where many windows are flat (block 5) and fall
     // back to the slow fix-up kernel.  12 images at 480 x 640 x 128: launches that size lose nothing to tails.
     const int64_t per_image = D * H * W;
-    const int64_t nb_max = std::max<int64_t>(1, (((int64_t)1 << 24) - 1024) * 32 / std::max<int64_t>(per_image, 1));
+    const int64_t nb_max = xcorr_images_per_launch(D, H, W);
     bool done = true;
     for (int64_t b0 = 0; b0 < B && done; b0 += nb_max) {
       const int64_t nb = std::min(nb_max, B - b0);
@@ -1027,6 +1290,39 @@ static int xcorrvol_impl(const T* in0, const T* in1, T* out, int64_t B, int64_t 
   return check_launch("xcorrvol(generic)");
 }
 
+template <typename T>
+static int xcorr_disparity_impl(const T* in0, const T* in1, T* disp, T* score, int64_t B, int64_t C, int64_t H, int64_t W,
+                                int64_t D, int bs, int subpixel, cudaStream_t st) {
+  CTD_REQUIRE(B >= 0 && C >= 0 && H >= 0 && W >= 0 && D >= 0, "xcorr_disparity: negative size");
+  CTD_REQUIRE(bs >= 1 && bs <= 255, "xcorr_disparity: block_size %d out of range [1,255]", bs);
+  CTD_REQUIRE(H <= INT32_MAX && W <= INT32_MAX && D <= INT32_MAX && C <= INT32_MAX, "xcorr_disparity: dimension too large");
+  const int64_t npix = B * H * W;
+  if (npix == 0) return CTD_OK;
+  CTD_REQUIRE(D >= 1, "xcorr_disparity: n_disps must be >= 1");
+  CTD_REQUIRE(disp && (C == 0 || (in0 && in1)), "xcorr_disparity: null pointer");
+  if (sizeof(T) == 4 && C == 1 && !g_force_generic && (bs == 3 || bs == 5 || bs == 7 || bs == 9)) {
+    const float* f0 = reinterpret_cast<const float*>(in0);
+    const float* f1 = reinterpret_cast<const float*>(in1);
+    const int64_t nb_max = xcorr_images_per_launch(D, H, W);
+    bool done = true;
+    for (int64_t b0 = 0; b0 < B && done; b0 += nb_max) {
+      const int64_t nb = std::min(nb_max, B - b0), off = b0 * H * W;
+      const XcorrWta wta{reinterpret_cast<float*>(disp) + off, score ? reinterpret_cast<float*>(score) + off : nullptr, subpixel};
+      const float *q0 = f0 + off, *q1 = f1 + off;
+      done = bs == 9   ? xcorr_sep_launch<9>(q0, q1, nullptr, nb, H, W, D, st, &wta)
+             : bs == 7 ? xcorr_sep_launch<7>(q0, q1, nullptr, nb, H, W, D, st, &wta)
+             : bs == 5 ? xcorr_sep_launch<5>(q0, q1, nullptr, nb, H, W, D, st, &wta)
+                       : xcorr_sep_launch<3>(q0, q1, nullptr, nb, H, W, D, st, &wta);
+      if (!done && b0 > 0) return fail(CTD_ERR_CUDA, "xcorr_disparity: launch of images %lld.. failed", (long long)b0);
+    }
+    if (done) return check_launch("xcorr_disparity(separable)");
+  }
+  const int grid = (int)std::min<int64_t>(cdiv(npix, 256), 148 * 64);
+  xcorr_disparity_generic<T><<<grid, 256, 0, st>>>(in0, in1, disp, score, B, (int)C, (int)H, (int)W, (int)D, bs, subpixel);
+  count_launch();
+  return check_launch("xcorr_disparity(generic)");
+}
+
 }  // namespace ctd
 
 CTD_API int ctd_xcorrvol_f32(const float* in0, const float* in1, float* out, int64_t B, int64_t C, int64_t H,
@@ -1036,4 +1332,12 @@ CTD_API int ctd_xcorrvol_f32(const float* in0, const float* in1, float* out, int
 CTD_API int ctd_xcorrvol_f64(const double* in0, const double* in1, double* out, int64_t B, int64_t C, int64_t H,
                                 int64_t W, int64_t D, int bs, ctd_stream_t s) {
   return ctd::xcorrvol_impl<double>(in0, in1, out, B, C, H, W, D, bs, ctd::as_stream(s));
+}
+CTD_API int ctd_xcorr_disparity_f32(const float* in0, const float* in1, float* disp, float* score, int64_t B, int64_t C,
+                                    int64_t H, int64_t W, int64_t n_disps, int block_size, int subpixel, ctd_stream_t s) {
+  return ctd::xcorr_disparity_impl<float>(in0, in1, disp, score, B, C, H, W, n_disps, block_size, subpixel, ctd::as_stream(s));
+}
+CTD_API int ctd_xcorr_disparity_f64(const double* in0, const double* in1, double* disp, double* score, int64_t B, int64_t C,
+                                    int64_t H, int64_t W, int64_t n_disps, int block_size, int subpixel, ctd_stream_t s) {
+  return ctd::xcorr_disparity_impl<double>(in0, in1, disp, score, B, C, H, W, n_disps, block_size, subpixel, ctd::as_stream(s));
 }

@@ -111,6 +111,27 @@ def xcorrvol_cuda(in0, in1, n_disps, block_size):
     return out
 
 
+def xcorr_disparity_cuda(in0, in1, n_disps, block_size, subpixel=True):
+    """Winner-take-all disparity of xcorrvol_cuda's volume without writing it (ctd_xcorr_disparity_*).  in0, in1 [C,H,W]
+    -> (disp, score) [1,H,W]; batched: [B,C,H,W] -> [B,1,H,W]."""
+    _check_input_cuda(in0, "in0")
+    _check_input_cuda(in1, "in1")
+    _check(in0.dim() in (3, 4), "in0 has to be C x H x W (or B x C x H x W)")
+    _check(tuple(in0.shape) == tuple(in1.shape), "in0 and in1 have to be the same shape")
+    _same(in0, in1, "in0", "in1")
+    sfx = _real_suffix(in0, "xcorr_disparity")
+    batched = in0.dim() == 4
+    B = in0.size(0) if batched else 1
+    C, H, W = in0.shape[-3:]
+    shape = (B, 1, H, W) if batched else (1, H, W)
+    disp = torch.empty(shape, dtype=in0.dtype, device=in0.device)
+    score = torch.empty(shape, dtype=in0.dtype, device=in0.device)
+    with torch.cuda.device(in0.device):
+        _lib.call("ctd_xcorr_disparity" + sfx, in0.data_ptr(), in1.data_ptr(), disp.data_ptr(), score.data_ptr(), B, C, H, W,
+                  int(n_disps), int(block_size), int(bool(subpixel)), _stream(in0))
+    return disp, score
+
+
 def _photometric_args(es, ta, type):
     _check_input_cuda(es, "es")
     _check_input_cuda(ta, "ta")

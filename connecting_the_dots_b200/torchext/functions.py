@@ -77,6 +77,46 @@ def xcorrvol(in0, in1, n_disps, block_size):
     return XCorrVolFunction.apply(in0, in1, n_disps, block_size)
 
 
+def xcorr_disparity(in0, in1, n_disps, block_size, subpixel=True):
+    """Block-matching disparity from the xcorrvol cost volume, without writing the volume: (disp, score), [B,1,H,W] for a
+    [B,C,H,W] pair ([1,H,W] for the reference's [C,H,W]), in the input's dtype, not differentiable.  d* is the first d with
+    the largest score (winner-take-all), score the peak correlation there; with subpixel, disp = d* + the vertex offset of
+    the parabola through the scores at d* - 1, d*, d* + 1 (disparity_from_volume states it).  d* and score equal
+    disparity_from_volume(xcorrvol(in0, in1, n_disps, block_size)) exactly.  CUDA tensors only, float32 or float64."""
+    if not in0.is_cuda:
+        raise RuntimeError("torchext.xcorr_disparity: connecting_the_dots_b200 has no CPU implementation")
+    return ext_cuda.xcorr_disparity_cuda(in0, in1, n_disps, block_size, subpixel)
+
+
+def disparity_from_volume(vol, subpixel=True):
+    """Winner-take-all disparity of a cost volume [B,D,H,W] (or [D,H,W]) in plain torch, any device: the definition of
+    xcorr_disparity and its test oracle.  d* = the first d with vol[:, d] equal to the maximum over d; score = vol at d*;
+    with subpixel, c-, c0, c+ = vol at d* - 1, d*, d* + 1, den = c- - 2 c0 + c+ and disp = d* + clamp((c- - c+) / (2 den),
+    -0.5, 0.5), in float64, the offset 0 where d* = 0, d* = D - 1 or den >= 0.  Returns (disp, score), [B,1,H,W] (or
+    [1,H,W]), in vol's dtype.  For finite volumes; a column holding NaN gives d* = D - 1 (no error)."""
+    v = vol if vol.dim() == 4 else vol.unsqueeze(0)
+    D = v.size(1)
+    if D < 1:
+        raise RuntimeError("disparity_from_volume: the volume has no disparities")
+    idx = torch.arange(D, device=v.device).view(1, D, 1, 1)
+    # the first maximum (a column holding NaN has none: it gets d = D - 1, outside the finite-input contract)
+    d = torch.where(v == v.amax(dim=1, keepdim=True), idx, D).amin(dim=1, keepdim=True).clamp(max=D - 1)
+    score = v.gather(1, d)
+    disp = d.to(torch.float64)
+    if subpixel:
+        cm = v.gather(1, (d - 1).clamp(min=0)).double()
+        c0 = score.double()
+        cp = v.gather(1, (d + 1).clamp(max=D - 1)).double()
+        den = cm - 2 * c0 + cp
+        ok = (d > 0) & (d < D - 1) & (den < 0)
+        delta = torch.where(ok, (cm - cp) / (2 * torch.where(ok, den, -1.0)), 0.0).clamp(-0.5, 0.5)
+        disp = disp + delta
+    disp = disp.to(vol.dtype)
+    if vol.dim() == 3:
+        disp, score = disp[0], score[0]
+    return disp, score
+
+
 class PhotometricLossFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, es, ta, block_size, type, eps):

@@ -59,6 +59,17 @@ class XCorrVol(torch.nn.Module):
         return F.xcorrvol(in0, in1, self.n_disps, self.block_size)
 
 
+class XCorrDisparity(torch.nn.Module):
+    """forward(in0, in1) -> (disp, score) of xcorr_disparity: the winner-take-all disparity of XCorrVol's volume."""
+
+    def __init__(self, n_disps=128, block_size=9, subpixel=True):
+        super().__init__()
+        self.n_disps, self.block_size, self.subpixel = n_disps, block_size, subpixel
+
+    def forward(self, in0, in1):
+        return F.xcorr_disparity(in0, in1, self.n_disps, self.block_size, self.subpixel)
+
+
 class CrossCheck(torch.nn.Module):
     def forward(self, in0, in1):
         return F.crosscheck(in0, in1)

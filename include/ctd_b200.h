@@ -138,6 +138,28 @@ int ctd_xcorrvol_f32(const float* in0, const float* in1, float* out, int64_t B, 
 int ctd_xcorrvol_f64(const double* in0, const double* in1, double* out, int64_t B, int64_t C,
                      int64_t H, int64_t W, int64_t n_disps, int block_size, ctd_stream_t stream);
 
+/* ---- block-matching disparity from the XCorrVol cost volume (an addition: the reference has no consumer of the volume),
+ * without writing the volume.  With V[b,d,h,w] what ctd_xcorrvol_* writes for the same arguments (n_disps = D):
+ *   d*[b,h,w]        = the first d in [0, D) with V[b,d,h,w] = max_d V[b,d,h,w] (ties -> smallest d; +0.0 == -0.0),
+ *   score[b,0,h,w]   = V[b,d*,h,w], the peak normalised cross-correlation (a confidence),
+ *   disp[b,0,h,w]    = d* (subpixel = 0), or d* + delta (subpixel = 1) with c-, c0, c+ the scores at d*-1, d*, d*+1,
+ *                      den = c- - 2 c0 + c+, delta = (c- - c+) / (2 den) clamped to [-0.5, 0.5]; delta = 0 when d* = 0,
+ *                      d* = D-1 or den >= 0.
+ * disp and score [B,1,H,W], DEVICE pointers; score may be NULL.  n_disps >= 1 unless B*H*W = 0 (then CTD_OK, nothing runs).
+ * The integer disparity and the score equal the argmax and the maximum of the volume ctd_xcorrvol_* computes for the same
+ * inputs with the default options: fp32, C = 1, block 3/5/7/9 run one fused pass over the separable kernel's outputs
+ * (workspace grows with B*H*W, not B*D*H*W); every other case, and force_generic, runs a generic kernel, the exact argmax
+ * of the generic volume.  Not mirrored: the A/B options xcorr_direct and xcorr_nofix (the disparity always uses the
+ * separable kernel with its fix-up), and sizes the separable launch rejects (> 65535 row tiles or image x disparity-chunk
+ * launches, 2^31 statistics positions), where the volume falls back to its direct kernel and the disparity to the generic
+ * one -- equal to within the volume's 1e-5 there, not bit for bit.  In the fused path the sub-pixel scores are re-evaluated
+ * in the centred form, within ~1e-5 of the volume's.  The inputs must be finite: for non-finite inputs the
+ * result is unspecified (the call does not fault). */
+int ctd_xcorr_disparity_f32(const float* in0, const float* in1, float* disp, float* score, int64_t B, int64_t C, int64_t H,
+                            int64_t W, int64_t n_disps, int block_size, int subpixel, ctd_stream_t stream);
+int ctd_xcorr_disparity_f64(const double* in0, const double* in1, double* disp, double* score, int64_t B, int64_t C, int64_t H,
+                            int64_t W, int64_t n_disps, int block_size, int subpixel, ctd_stream_t stream);
+
 /* ---- ProjNNFunctor: ext.h:65-117, ext_cuda.cpp:47-69 (proj_nn_cuda).  K is a DEVICE pointer to
  * 9 values (row-major 3x3), like the reference's K tensor. */
 int ctd_proj_nn_f32(const float* xyz0, const float* xyz1, const float* K, int64_t* out, int64_t B,

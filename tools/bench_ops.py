@@ -3,11 +3,14 @@
 launching stream, rotating buffer sets larger than L2 where the op is HBM-bound).  Prints one JSON
 object; bench.py stays the contract benchmark, this is the per-op table that goes into profiles/.
 
-    python tools/bench_ops.py [--iters 30] [--only photometric,ssim,lcn,xcorrvol,proj_nn,nn,crosscheck]
+    python tools/bench_ops.py [--iters 30] [--only photometric,ssim,lcn,xcorrvol,xcorr_disparity,proj_nn,nn,crosscheck]
+
+The printed result names the GPU and its power limit, read in the same run.
 """
 import argparse
 import json
 import os
+import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -55,7 +58,19 @@ def timeit(fn, iters, warmup=5, nrep=NREP):
     return float(np.median(ts)), float(np.min(ts))
 
 
-ALL = "calib,photometric,ssim,warp,pyramid,geometric,disparity,lcn,xcorrvol,proj_nn,config4,nn,crosscheck,reduce,gpu_reference"
+def device_info(index):
+    """Name and power limit of the GPU the timings are taken on (nvidia-smi only reads them)."""
+    info = {"name": torch.cuda.get_device_name(index)}
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", str(index)],
+                             capture_output=True, text=True, timeout=60).stdout.strip()
+        info["nvidia_smi"] = out
+    except Exception as e:  # the timings stand without it, but say why it is missing
+        info["nvidia_smi"] = "unavailable: %s" % e
+    return info
+
+
+ALL = "calib,photometric,ssim,warp,pyramid,geometric,disparity,lcn,xcorrvol,xcorr_disparity,proj_nn,config4,nn,crosscheck,reduce,gpu_reference"
 
 
 def main():
@@ -64,7 +79,9 @@ def main():
     ap.add_argument("--only", default=ALL)
     ap.add_argument("--batch", type=int, default=8)
     args = ap.parse_args()
-    print(json.dumps(run(args.only, args.iters, args.batch)))
+    res = run(args.only, args.iters, args.batch)
+    res["device"] = device_info(0)
+    print(json.dumps(res))
 
 
 def run(only=ALL, iters=30, batch=8, device_index=0, verbose=True):
@@ -320,6 +337,39 @@ def run(only=ALL, iters=30, batch=8, device_index=0, verbose=True):
                 _lib.call("ctd_xcorrvol_f32", d["ta"].data_ptr(), d["pat_lcn"].data_ptr(), vols[i % 2].data_ptr(), B, 1, H, W, D, bs, st)
             add("xcorrvol_D128_bs%d" % bs, *timeit(f, max(3, args.iters // 6), warmup=1, nrep=2), (8 + 4 * D) * npx)
         del vols
+    if "xcorr_disparity" in only:
+        # the fused winner-take-all disparity (ctd_xcorr_disparity_f32, sub-pixel on) against what a caller does without it,
+        # on the same inputs in the same run: xcorrvol, then torch.max over d and the three-point parabola in torch
+        D = 128
+        vol = torch.empty(B, D, H, W, device=dev)
+        outs = [(torch.empty(B, 1, H, W, device=dev), torch.empty(B, 1, H, W, device=dev)) for _ in range(2)]
+        for bs in (9, 5):
+            def f(i, st, bs=bs):
+                d, (o_d, o_s) = sets[i % NS], outs[i % 2]
+                _lib.call("ctd_xcorr_disparity_f32", d["ta"].data_ptr(), d["pat_lcn"].data_ptr(), o_d.data_ptr(), o_s.data_ptr(),
+                          B, 1, H, W, D, bs, 1, st)
+            def g(i, st, bs=bs):
+                d = sets[i % NS]
+                _lib.call("ctd_xcorrvol_f32", d["ta"].data_ptr(), d["pat_lcn"].data_ptr(), vol.data_ptr(), B, 1, H, W, D, bs, st)
+                c0, di = vol.max(dim=1, keepdim=True)
+                cm, cp = vol.gather(1, (di - 1).clamp(min=0)), vol.gather(1, (di + 1).clamp(max=D - 1))
+                den = cm - 2 * c0 + cp
+                ok = (di > 0) & (di < D - 1) & (den < 0)
+                outs[i % 2][0].copy_(di + torch.where(ok, (cm - cp) / (2 * den), 0.0).clamp(-0.5, 0.5))
+                outs[i % 2][1].copy_(c0)
+            def f0(i, st, bs=bs):
+                d, (o_d, o_s) = sets[i % NS], outs[i % 2]
+                _lib.call("ctd_xcorr_disparity_f32", d["ta"].data_ptr(), d["pat_lcn"].data_ptr(), o_d.data_ptr(), o_s.data_ptr(),
+                          B, 1, H, W, D, bs, 0, st)
+            fused, unfused = "xcorr_disparity_D128_bs%d" % bs, "xcorrvol_then_torch_argmax_D128_bs%d" % bs
+            add(fused, *timeit(f, max(3, args.iters // 6), warmup=1, nrep=2), 16 * npx,
+                extra={"note": "in0, in1 in; disp (sub-pixel) and score out"})
+            add(fused + "_integer", *timeit(f0, max(3, args.iters // 6), warmup=1, nrep=2), 16 * npx,
+                extra={"note": "the same without sub-pixel refinement"})
+            add(unfused, *timeit(g, max(3, args.iters // 6), warmup=1, nrep=2), (8 + 8 * D + 16) * npx,
+                extra={"note": "xcorrvol writes the volume, torch.max reads it back, parabola from gathers"})
+            res["ops"][fused]["speedup_vs_volume_then_argmax"] = res["ops"][unfused]["ms_median"] / res["ops"][fused]["ms_median"]
+        del vol
     if "proj_nn" in only:
         T = 4
         xyz, K, poses = synth.make_clouds(T, H, W)
