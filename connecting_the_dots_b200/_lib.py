@@ -30,6 +30,8 @@ SIGNATURES = {
     "ctd_xcorrvol_f64": [_ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _int, _ptr],
     "ctd_xcorr_disparity_f32": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _int, _int, _ptr],
     "ctd_xcorr_disparity_f64": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _int, _int, _ptr],
+    "ctd_sgm_f32": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _f64, _f64, _int, _int, _ptr],
+    "ctd_sgm_f64": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _f64, _f64, _int, _int, _ptr],
     "ctd_proj_nn_f32": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _int, _ptr],
     "ctd_proj_nn_f64": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _int, _ptr],
     "ctd_nn_f32": [_ptr, _ptr, _ptr, _i64, _i64, _ptr],

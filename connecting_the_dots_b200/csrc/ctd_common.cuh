@@ -145,4 +145,12 @@ __device__ __forceinline__ void finish_masked_sums(double num, double den, doubl
 
 __device__ __forceinline__ bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
+// three-point parabola through the scores at d* - 1, d*, d* + 1: vertex offset in [-0.5, 0.5], 0 unless the peak is strict
+// (den < 0); fp64 with disparity_from_volume's operation order
+__device__ __forceinline__ double wta_subpixel(double cm, double c0, double cp) {
+  const double den = cm - 2.0 * c0 + cp;
+  if (!(den < 0.0)) return 0.0;
+  return fmin(fmax((cm - cp) / (2.0 * den), -0.5), 0.5);
+}
+
 }  // namespace ctd

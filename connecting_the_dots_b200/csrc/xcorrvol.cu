@@ -88,14 +88,6 @@ __device__ __forceinline__ float wta_score(unsigned long long key) {
 __device__ __forceinline__ int wta_disp(unsigned long long key, int D) {  // clamped: a key of 0 (no candidate) is never read out of range
   return (int)min(0xFFFFFFFFu - (unsigned)key, (unsigned)(D - 1));
 }
-// three-point parabola through the scores at d* - 1, d*, d* + 1: vertex offset in [-0.5, 0.5], 0 unless the peak is strict
-// (den < 0); fp64 like disparity_from_volume
-__device__ __forceinline__ double wta_subpixel(double cm, double c0, double cp) {
-  const double den = cm - 2.0 * c0 + cp;
-  if (!(den < 0.0)) return 0.0;
-  return fmin(fmax((cm - cp) / (2.0 * den), -0.5), 0.5);
-}
-
 // generic disparity: one thread per pixel sweeps d with xcorr_generic_one, so d* and the score are the exact argmax and
 // maximum of xcorrvol_generic's volume
 template <typename T>

@@ -132,6 +132,28 @@ def xcorr_disparity_cuda(in0, in1, n_disps, block_size, subpixel=True):
     return disp, score
 
 
+def sgm_cuda(vol, p1, p2, paths=8, subpixel=True, want_disparity=True):
+    """Semi-global matching over a score volume (ctd_sgm_*).  vol [B,D,H,W] (or [D,H,W]) -> (agg, disp, score): agg like
+    vol, disp and score [B,1,H,W] (or [1,H,W]), or None without want_disparity."""
+    _check_input_cuda(vol, "vol")
+    _check(vol.dim() in (3, 4), "vol has to be D x H x W (or B x D x H x W)")
+    sfx = _real_suffix(vol, "sgm")
+    batched = vol.dim() == 4
+    B = vol.size(0) if batched else 1
+    D, H, W = vol.shape[-3:]
+    agg = torch.empty_like(vol)
+    disp = score = None
+    if want_disparity:
+        shape = (B, 1, H, W) if batched else (1, H, W)
+        disp = torch.empty(shape, dtype=vol.dtype, device=vol.device)
+        score = torch.empty(shape, dtype=vol.dtype, device=vol.device)
+    with torch.cuda.device(vol.device):
+        _lib.call("ctd_sgm" + sfx, vol.data_ptr(), agg.data_ptr(), disp.data_ptr() if want_disparity else None,
+                  score.data_ptr() if want_disparity else None, B, D, H, W, float(p1), float(p2), int(paths),
+                  int(bool(subpixel)), _stream(vol))
+    return agg, disp, score
+
+
 def _photometric_args(es, ta, type):
     _check_input_cuda(es, "es")
     _check_input_cuda(ta, "ta")

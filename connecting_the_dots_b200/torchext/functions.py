@@ -117,6 +117,85 @@ def disparity_from_volume(vol, subpixel=True):
     return disp, score
 
 
+SGM_PATHS = {4: ((0, 1), (0, -1), (1, 0), (-1, 0)),
+             8: ((0, 1), (0, -1), (1, 0), (-1, 0), (1, 1), (1, -1), (-1, 1), (-1, -1))}
+
+
+def sgm_aggregate(vol, p1, p2, paths=8):
+    """Semi-global matching (Hirschmueller, PAMI 2008) over a score volume vol [B,D,H,W] (or [D,H,W]; higher is better, the
+    convention of xcorrvol: pass a cost volume negated): the aggregated volume A, same shape and dtype, equal bit for bit to
+    sgm_aggregate_pytorch, which states the definition.  Not differentiable.  CUDA tensors only, float32 or float64."""
+    if not vol.is_cuda:
+        raise RuntimeError("torchext.sgm_aggregate: connecting_the_dots_b200 has no CPU implementation")
+    return ext_cuda.sgm_cuda(vol, p1, p2, paths, want_disparity=False)[0]
+
+
+def sgm_disparity(vol, p1, p2, paths=8, subpixel=True):
+    """(disp, score) = disparity_from_volume(sgm_aggregate(vol, p1, p2, paths), subpixel), bit for bit, with the
+    winner-take-all fused into the last aggregation pass; A is allocated and dropped.  [B,1,H,W] (or [1,H,W]), not
+    differentiable, CUDA tensors only, float32 or float64."""
+    if not vol.is_cuda:
+        raise RuntimeError("torchext.sgm_disparity: connecting_the_dots_b200 has no CPU implementation")
+    _, disp, score = ext_cuda.sgm_cuda(vol, p1, p2, paths, subpixel)
+    return disp, score
+
+
+def _sgm_check(vol, p1, p2, paths):
+    if paths not in SGM_PATHS:
+        raise RuntimeError("sgm: paths must be 4 or 8, got %r" % (paths,))
+    if vol.dim() not in (3, 4) or vol.size(-3) < 1:
+        raise RuntimeError("sgm: vol has to be D x H x W (or B x D x H x W) with D >= 1")
+    if vol.dtype not in (torch.float32, torch.float64):
+        raise NotImplementedError("sgm: float32 or float64 volumes only")
+    t1, t2 = (torch.tensor(float(p), dtype=vol.dtype, device=vol.device) for p in (p1, p2))
+    if not (torch.isfinite(t1) and torch.isfinite(t2) and 0 <= t1 <= t2):
+        raise RuntimeError("sgm: penalties must be finite with 0 <= p1 <= p2 (p1 = %r, p2 = %r)" % (p1, p2))
+    return t1, t2
+
+
+def sgm_aggregate_pytorch(vol, p1, p2, paths=8):
+    """The definition of sgm_aggregate in plain torch, any device, in vol's dtype, and its test oracle.  For each path
+    direction r = (dy, dx) in the order of SGM_PATHS[paths] and q = p - r: L_r(p, d) = V(p, d) where q is outside the image,
+    else L_r(p, d) = V(p, d) + (m - M) with M = max_k L_r(q, k) and m = max(L_r(q, d), L_r(q, d-1) - p1, L_r(q, d+1) - p1,
+    M - p2) over the neighbours inside [0, D); p1, p2 converted once to vol's dtype.  A = (((L_0 + L_1) + L_2) + ...)."""
+    t1, t2 = _sgm_check(vol, p1, p2, paths)
+    v = vol if vol.dim() == 4 else vol.unsqueeze(0)
+    B, D, H, W = v.shape
+
+    def step(lq, cur, valid):
+        # lq: L_r(q, .) aligned with cur [B,D,N]; valid [N]: q inside the image
+        M = lq.amax(dim=1, keepdim=True)
+        ninf = torch.full_like(lq[:, :1], float("-inf"))
+        dn = torch.cat([ninf, lq[:, :-1]], 1) - t1     # L(q, d-1) - p1
+        up = torch.cat([lq[:, 1:], ninf], 1) - t1      # L(q, d+1) - p1
+        m = torch.maximum(torch.maximum(lq, dn), torch.maximum(up, M - t2))
+        return torch.where(valid, cur + (m - M), cur)
+
+    agg = None
+    for dy, dx in SGM_PATHS[paths]:
+        L = torch.empty_like(v)
+        if dy == 0:    # along rows: lines are [B,D,H] columns of pixels
+            ws = range(W) if dx > 0 else range(W - 1, -1, -1)
+            prev = None
+            for w in ws:
+                L[..., w] = v[..., w] if prev is None else step(prev, v[..., w], torch.ones(H, dtype=torch.bool, device=v.device))
+                prev = L[..., w]
+        else:          # row by row, the predecessor row shifted by dx
+            hs = range(H) if dy > 0 else range(H - 1, -1, -1)
+            prev = None
+            cols = torch.arange(W, device=v.device)
+            valid = (cols - dx >= 0) & (cols - dx < W)
+            for h in hs:
+                if prev is None:
+                    L[:, :, h] = v[:, :, h]
+                else:
+                    lq = prev if dx == 0 else torch.roll(prev, dx, dims=2)   # lq[..., w] = prev[..., w - dx]
+                    L[:, :, h] = step(lq, v[:, :, h], valid)
+                prev = L[:, :, h]
+        agg = L if agg is None else agg + L
+    return agg if vol.dim() == 4 else agg[0]
+
+
 class PhotometricLossFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, es, ta, block_size, type, eps):

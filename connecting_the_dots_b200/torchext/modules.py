@@ -70,6 +70,18 @@ class XCorrDisparity(torch.nn.Module):
         return F.xcorr_disparity(in0, in1, self.n_disps, self.block_size, self.subpixel)
 
 
+class SGMDisparity(torch.nn.Module):
+    """forward(in0, in1) -> (disp, score): xcorrvol(in0, in1, n_disps, block_size), then sgm_disparity over it.  The
+    default penalties (p1 = 0.2, p2 = 2.0 on the correlation scale, 8 paths) were tuned on two synthetic frames only."""
+
+    def __init__(self, n_disps=128, block_size=9, p1=0.2, p2=2.0, paths=8, subpixel=True):
+        super().__init__()
+        self.n_disps, self.block_size, self.p1, self.p2, self.paths, self.subpixel = n_disps, block_size, p1, p2, paths, subpixel
+
+    def forward(self, in0, in1):
+        return F.sgm_disparity(F.xcorrvol(in0, in1, self.n_disps, self.block_size), self.p1, self.p2, self.paths, self.subpixel)
+
+
 class CrossCheck(torch.nn.Module):
     def forward(self, in0, in1):
         return F.crosscheck(in0, in1)

@@ -160,6 +160,25 @@ int ctd_xcorr_disparity_f32(const float* in0, const float* in1, float* disp, flo
 int ctd_xcorr_disparity_f64(const double* in0, const double* in1, double* disp, double* score, int64_t B, int64_t C, int64_t H,
                             int64_t W, int64_t n_disps, int block_size, int subpixel, ctd_stream_t stream);
 
+/* ---- semi-global matching over a score volume (an addition: Hirschmueller, PAMI 2008).  vol [B,D,H,W], higher is better
+ * (the convention of ctd_xcorrvol_*; pass a cost volume negated).  p1, p2 are converted once to the volume's dtype.  For
+ * each path direction r = (dy, dx) and q = p - r:
+ *   L_r(p, d) = V(p, d)                    if q is outside the image (a path starts there),
+ *   L_r(p, d) = V(p, d) + (m - M)          otherwise, with M = max_k L_r(q, k) and
+ *               m = max(L_r(q, d), L_r(q, d-1) - p1, L_r(q, d+1) - p1, M - p2), leaving out neighbours outside [0, D).
+ * Path order: paths = 4: (0,+1) (0,-1) (+1,0) (-1,0); paths = 8: those, then (+1,+1) (+1,-1) (-1,+1) (-1,-1).
+ *   agg[b,d,h,w]   = A = (((L_0 + L_1) + L_2) + ...), summed in that order (required, caller-owned, must not overlap vol),
+ *   disp, score    = the winner-take-all of A exactly as ctd_xcorr_disparity_* states it for a volume (first maximum, score
+ *                    A at d*, optional fp64 three-point sub-pixel offset), [B,1,H,W]; each may be NULL.
+ * Every value is bit-equal to that definition (no multiplies, max is exact).  CTD_ERR_INVALID for paths other than 4 or
+ * 8, non-finite penalties, p1 < 0, p2 < p1, D < 1 (unless B*H*W = 0: then CTD_OK and nothing runs), D > 1024, agg
+ * overlapping vol.  DEVICE pointers; no scratch memory, no atomics, capture-safe.  The inputs must be finite: for
+ * non-finite inputs the result is unspecified (the call does not fault). */
+int ctd_sgm_f32(const float* vol, float* agg, float* disp, float* score, int64_t B, int64_t D, int64_t H, int64_t W,
+                double p1, double p2, int paths, int subpixel, ctd_stream_t stream);
+int ctd_sgm_f64(const double* vol, double* agg, double* disp, double* score, int64_t B, int64_t D, int64_t H, int64_t W,
+                double p1, double p2, int paths, int subpixel, ctd_stream_t stream);
+
 /* ---- ProjNNFunctor: ext.h:65-117, ext_cuda.cpp:47-69 (proj_nn_cuda).  K is a DEVICE pointer to
  * 9 values (row-major 3x3), like the reference's K tensor. */
 int ctd_proj_nn_f32(const float* xyz0, const float* xyz1, const float* K, int64_t* out, int64_t B,

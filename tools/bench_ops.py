@@ -3,7 +3,7 @@
 launching stream, rotating buffer sets larger than L2 where the op is HBM-bound).  Prints one JSON
 object; bench.py stays the contract benchmark, this is the per-op table that goes into profiles/.
 
-    python tools/bench_ops.py [--iters 30] [--only photometric,ssim,lcn,xcorrvol,xcorr_disparity,proj_nn,nn,crosscheck]
+    python tools/bench_ops.py [--iters 30] [--only photometric,ssim,lcn,xcorrvol,xcorr_disparity,sgm,proj_nn,nn,crosscheck]
 
 The printed result names the GPU and its power limit, read in the same run.
 """
@@ -70,7 +70,7 @@ def device_info(index):
     return info
 
 
-ALL = "calib,photometric,ssim,warp,pyramid,geometric,disparity,lcn,xcorrvol,xcorr_disparity,proj_nn,config4,nn,crosscheck,reduce,gpu_reference"
+ALL = "calib,photometric,ssim,warp,pyramid,geometric,disparity,lcn,xcorrvol,xcorr_disparity,sgm,proj_nn,config4,nn,crosscheck,reduce,gpu_reference"
 
 
 def main():
@@ -370,6 +370,51 @@ def run(only=ALL, iters=30, batch=8, device_index=0, verbose=True):
                 extra={"note": "xcorrvol writes the volume, torch.max reads it back, parabola from gathers"})
             res["ops"][fused]["speedup_vs_volume_then_argmax"] = res["ops"][unfused]["ms_median"] / res["ops"][fused]["ms_median"]
         del vol
+    if "sgm" in only:
+        # semi-global matching over the xcorrvol block-9 volume of the bench frames: the fused call (ctd_sgm_f32, sub-pixel
+        # on) at 4 and 8 paths, against sgm_aggregate followed by disparity_from_volume in the same run.  The volume is
+        # larger than L2 at batch 8 already, so one input serves every launch.
+        D = 128
+        vol = torch.empty(B, D, H, W, device=dev)
+        _lib.call("ctd_xcorrvol_f32", sets[0]["ta"].data_ptr(), sets[0]["pat_lcn"].data_ptr(), vol.data_ptr(), B, 1, H, W, D, 9,
+                  torch.cuda.current_stream().cuda_stream)
+        agg = torch.empty_like(vol)
+        o_d, o_s = torch.empty(B, 1, H, W, device=dev), torch.empty(B, 1, H, W, device=dev)
+        floor = (4 * D + 8) * npx
+        it = max(3, args.iters // 6)
+        for P in (4, 8):
+            def f(i, st, P=P):
+                _lib.call("ctd_sgm_f32", vol.data_ptr(), agg.data_ptr(), o_d.data_ptr(), o_s.data_ptr(), B, D, H, W, 0.2, 2.0, P, 1, st)
+
+            def g(i, st, P=P):
+                _lib.call("ctd_sgm_f32", vol.data_ptr(), agg.data_ptr(), None, None, B, D, H, W, 0.2, 2.0, P, 1, st)
+                d, s = tx.disparity_from_volume(agg, True)
+                o_d.copy_(d)
+                o_s.copy_(s)
+            fused, unfused = "sgm_disparity_%dpaths_D128" % P, "sgm_aggregate_then_disparity_from_volume_%dpaths_D128" % P
+            design = (3 * P - 1) * 4 * D * npx + 8 * npx
+            add(fused, *timeit(f, it, warmup=1, nrep=2), floor,
+                extra={"note": "algo_bytes: V in (4D B/px), disp and score out (8 B/px); A is written too (caller-owned)",
+                       "design_bytes": design})
+            res["ops"][fused]["frac_design_at_peak"] = design / res["ops"][fused]["ms_median"] / 1e6 / PEAK
+            res["ops"][fused]["achieved_design_gbs"] = design / res["ops"][fused]["ms_median"] / 1e6
+            add(unfused, *timeit(g, it, warmup=1, nrep=2), floor,
+                extra={"note": "the same aggregation without disp/score, then disparity_from_volume reads A back in torch"})
+            res["ops"][fused]["speedup_vs_unfused"] = res["ops"][unfused]["ms_median"] / res["ops"][fused]["ms_median"]
+        if B <= 8:
+            # the torch restatement on the GPU: launch-bound (a few ops per scan-line step), timed eagerly over two calls
+            tx.disparity_from_volume(tx.sgm_aggregate_pytorch(vol, 0.2, 2.0, 8), True)
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            torch.cuda.synchronize()
+            e0.record()
+            for _ in range(2):
+                tx.disparity_from_volume(tx.sgm_aggregate_pytorch(vol, 0.2, 2.0, 8), True)
+            e1.record()
+            torch.cuda.synchronize()
+            ms = e0.elapsed_time(e1) / 2
+            add("sgm_pytorch_restatement_8paths_D128", ms, ms, floor, extra={"note": "sgm_aggregate_pytorch + disparity_from_volume"})
+            res["ops"]["sgm_disparity_8paths_D128"]["speedup_vs_torch"] = ms / res["ops"]["sgm_disparity_8paths_D128"]["ms_median"]
+        del vol, agg
     if "proj_nn" in only:
         T = 4
         xyz, K, poses = synth.make_clouds(T, H, W)
