@@ -152,17 +152,23 @@ CTD_API int ctd_lcn_bwd_f32(const float* x, const float* lcn, const float* std_,
   if (N * H * W == 0) return CTD_OK;
   CTD_REQUIRE(x && lcn && std_ && grad_x, "lcn_bwd: null pointer");
   CTD_REQUIRE(radius < H && radius < W, "lcn_bwd: radius %d needs an image larger than %d x %d (ReflectionPad2d)", radius, (int)H, (int)W);
-  CTD_REQUIRE(H <= INT32_MAX && W <= INT32_MAX && N <= 65535, "lcn_bwd: dimension too large");
-  const int64_t n = N * H * W;
+  CTD_REQUIRE(H <= INT32_MAX && W <= INT32_MAX, "lcn_bwd: dimension too large");
+  const int64_t n = N * H * W, plane = H * W;
   float* scratch = static_cast<float*>(scratch_alloc(sizeof(float) * 2 * (size_t)n, st));
   if (!scratch) return fail(CTD_ERR_NOMEM, "lcn_bwd: no scratch memory for the coefficient planes");
   const float inv_n = 1.f / float((2 * radius + 1) * (2 * radius + 1));
   const int g1 = (int)std::min<int64_t>(cdiv(n, 256), 148 * 16);
   lcn_bwd_coeff_kernel<<<g1, 256, 0, st>>>(x, lcn, std_, g_lcn, g_std, scratch, scratch + n, n, epsilon, inv_n);
-  const dim3 grid((unsigned)cdiv(W, LB_TW), (unsigned)cdiv(H, LB_TH), (unsigned)N);
-  lcn_bwd_box_kernel<<<grid, 256, 0, st>>>(x, std_, g_lcn, scratch, scratch + n, grad_x, (int)H, (int)W, radius);
+  count_launch();
+  // the box kernel takes the image index from gridDim.z (at most 65535): chunks of images
+  for (int64_t b0 = 0; b0 < N; b0 += 65535) {
+    const int64_t nb = std::min<int64_t>(65535, N - b0), o = b0 * plane;
+    const dim3 grid((unsigned)cdiv(W, LB_TW), (unsigned)cdiv(H, LB_TH), (unsigned)nb);
+    lcn_bwd_box_kernel<<<grid, 256, 0, st>>>(x + o, std_ + o, g_lcn ? g_lcn + o : nullptr, scratch + o, scratch + n + o, grad_x + o,
+                                             (int)H, (int)W, radius);
+    count_launch();
+  }
   scratch_free(scratch, st);
-  count_launch(2);
   return check_launch("lcn_bwd");
 }
 

@@ -213,7 +213,8 @@ int ctd_pattern_similarity_f32(const float* pattern, const float* disp, const fl
                                ctd_stream_t stream);
 
 /* ---- LCN backward: what autograd produces for networks.LCN (model/networks.py:523-533) w.r.t. its input, given the
- * forward's input x, its outputs (lcn, std) and upstream gradients for both outputs (either may be NULL = zero). */
+ * forward's input x, its outputs (lcn, std) and upstream gradients for both outputs (either may be NULL = zero).
+ * radius <= 8 (CTD_ERR_INVALID above; the forward takes any radius); any number of images N. */
 int ctd_lcn_bwd_f32(const float* x, const float* lcn, const float* std, const float* grad_lcn, const float* grad_std,
                     float* grad_x, int64_t N, int64_t H, int64_t W, int radius, float epsilon, ctd_stream_t stream);
 
