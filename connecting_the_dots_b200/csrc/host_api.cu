@@ -85,10 +85,12 @@ struct Workspace {
   std::vector<Upload> uploads;
   // Downloads of the open batch that have been enqueued but not waited for: host ranges whose contents are not there
   // yet.  A later call of the batch that reads such a range (LCN's std as the mask of the loss, ProjNN's indices as
-  // CrossCheck's input) must not upload it -- the host still holds the old bytes.  An exact match (same address, same
-  // size: the chunks of two image-wise calls line up) is served from the producer's device buffer, with no copy at all:
-  // every kernel of a batch runs on the one compute stream, after its producer.  Any other overlap waits for the
-  // downloads to land and then uploads what the host really holds.
+  // CrossCheck's input) must not upload it -- the host still holds the old bytes.  The newest download that overlaps
+  // the range decides, since it lands last: an exact match (same address, same size: the chunks of two image-wise calls
+  // line up) is served from that producer's device buffer, with no copy at all -- every kernel of a batch runs on the
+  // one compute stream, after its producer.  Any other overlap waits for the downloads to land and then uploads what
+  // the host really holds.  A download also retires every entry of `uploads` it overlaps (note_download): that device
+  // copy no longer matches what the host will hold.
   std::vector<Upload> pending;
   uint64_t h2d_bytes = 0, h2d_saved = 0;  // statistics since ctd_host_begin_batch (ctd_host_batch_stats)
 
@@ -189,8 +191,15 @@ struct Workspace {
   int submit(std::string sig, const std::vector<const void*>& host_ptrs, std::function<int()> run);
   int end_batch(bool wait);
 
+  static bool overlaps(const Upload& u, const void* host, size_t bytes) {
+    const char *h0 = static_cast<const char*>(host), *p0 = static_cast<const char*>(u.host);
+    return h0 < p0 + u.bytes && p0 < h0 + bytes;
+  }
   void note_download(const void* host, size_t bytes, char* dev) {
-    if (deferred && bytes) pending.push_back({host, bytes, dev});
+    if (!deferred || !bytes) return;
+    uploads.erase(std::remove_if(uploads.begin(), uploads.end(), [&](const Upload& u) { return overlaps(u, host, bytes); }),
+                  uploads.end());
+    pending.push_back({host, bytes, dev});
   }
 
   // device address holding `bytes` bytes of `host`: the earlier upload of this batch, or `dst` after enqueuing the copy
@@ -198,22 +207,19 @@ struct Workspace {
     *dev = dst;
     if (bytes == 0) return CTD_OK;
     if (deferred) {
-      const char* h0 = static_cast<const char*>(host);
-      bool overlap = false;
-      for (const Upload& u : pending) {
-        if (u.host == host && u.bytes == bytes) {
-          *dev = u.dev;
+      for (auto p = pending.rbegin(); p != pending.rend(); ++p) {
+        if (!overlaps(*p, host, bytes)) continue;
+        if (p->host == host && p->bytes == bytes) {
+          *dev = p->dev;
           h2d_saved += bytes;
           return CTD_OK;
         }
-        const char* p0 = static_cast<const char*>(u.host);
-        overlap = overlap || (h0 < p0 + u.bytes && p0 < h0 + bytes);
-      }
-      if (overlap) {  // partial overlap with an output in flight: let the downloads finish, then the host copy is current
+        // partial overlap with an output in flight: let the downloads finish, then the host copy is current
         if (capturing) return CTD_RETRY_EAGER;
         CTD_CUDA(cudaStreamSynchronize(s_out));
         CTD_CUDA(cudaStreamSynchronize(stream));
         pending.clear();
+        break;
       }
       for (const Upload& u : uploads)
         if (u.host == host && u.bytes == bytes) {

@@ -264,7 +264,8 @@ int ctd_host_lcn_f32(const float* x, float* lcn, float* std, int64_t N, int64_t 
  * loss types, the gradient weights) is uploaded once.  An input that is an OUTPUT of an earlier call of the same batch
  * (LCN's std used as the loss mask, ProjNN's indices fed to CrossCheck) is taken from that call's device buffer when
  * address and size match exactly (no copy at all); any other overlap with an output still in flight first waits for
- * the downloads, then uploads what the host holds. */
+ * the downloads, then uploads what the host holds.  Later calls of a batch may overwrite an earlier call's inputs or
+ * outputs: the batch's results are those of the same calls made one at a time. */
 int ctd_host_begin_batch(void);
 int ctd_host_end_batch(void);
 /* Two batches in flight: ctd_host_end_batch_async() returns once the batch is enqueued, ctd_host_wait_batch() waits for the
