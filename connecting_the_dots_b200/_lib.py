@@ -32,6 +32,12 @@ SIGNATURES = {
     "ctd_xcorr_disparity_f64": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _int, _int, _ptr],
     "ctd_sgm_f32": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _f64, _f64, _int, _int, _ptr],
     "ctd_sgm_f64": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _f64, _f64, _int, _int, _ptr],
+    "ctd_census_transform_f32": [_ptr, _ptr, _i64, _i64, _i64, _i64, _int, _int, _ptr],
+    "ctd_census_transform_f64": [_ptr, _ptr, _i64, _i64, _i64, _i64, _int, _int, _ptr],
+    "ctd_census_vol_f32": [_ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _int, _int, _int, _ptr],
+    "ctd_census_vol_f64": [_ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _int, _int, _int, _ptr],
+    "ctd_census_disparity_f32": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _int, _int, _int, _int, _ptr],
+    "ctd_census_disparity_f64": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _int, _int, _int, _int, _ptr],
     "ctd_proj_nn_f32": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _int, _ptr],
     "ctd_proj_nn_f64": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _int, _ptr],
     "ctd_nn_f32": [_ptr, _ptr, _ptr, _i64, _i64, _ptr],

@@ -154,6 +154,55 @@ def sgm_cuda(vol, p1, p2, paths=8, subpixel=True, want_disparity=True):
     return agg, disp, score
 
 
+def census_transform_cuda(x, wh, ww):
+    """Census transform (ctd_census_transform_*): x [B,C,H,W] (or [C,H,W]) -> int64 of the same shape holding the uint64
+    bit patterns."""
+    _check_input_cuda(x, "x")
+    _check(x.dim() in (3, 4), "x has to be C x H x W (or B x C x H x W)")
+    sfx = _real_suffix(x, "census_transform")
+    B, C, H, W = x.shape if x.dim() == 4 else (1,) + tuple(x.shape)
+    out = torch.empty(x.shape, dtype=torch.int64, device=x.device)
+    with torch.cuda.device(x.device):
+        _lib.call("ctd_census_transform" + sfx, x.data_ptr(), out.data_ptr(), B, C, H, W, int(wh), int(ww), _stream(x))
+    return out
+
+
+def _census_pair(in0, in1, op):
+    _check_input_cuda(in0, "in0")
+    _check_input_cuda(in1, "in1")
+    _check(in0.dim() in (3, 4), "in0 has to be C x H x W (or B x C x H x W)")
+    _check(tuple(in0.shape) == tuple(in1.shape), "in0 and in1 have to be the same shape")
+    _same(in0, in1, "in0", "in1")
+    sfx = _real_suffix(in0, op)
+    B = in0.size(0) if in0.dim() == 4 else 1
+    return sfx, (B,) + tuple(in0.shape[-3:])
+
+
+def census_vol_cuda(in0, in1, n_disps, wh, ww, block_size):
+    """Census matching-score volume (ctd_census_vol_*): in0, in1 [B,C,H,W] -> [B,n_disps,H,W] (or [C,H,W] ->
+    [n_disps,H,W]), in the inputs' dtype."""
+    sfx, (B, C, H, W) = _census_pair(in0, in1, "census_vol")
+    shape = (B, int(n_disps), H, W) if in0.dim() == 4 else (int(n_disps), H, W)
+    out = torch.empty(shape, dtype=in0.dtype, device=in0.device)
+    with torch.cuda.device(in0.device):
+        _lib.call("ctd_census_vol" + sfx, in0.data_ptr(), in1.data_ptr(), out.data_ptr(), B, C, H, W, int(n_disps), int(wh),
+                  int(ww), int(block_size), _stream(in0))
+    return out
+
+
+def census_disparity_cuda(in0, in1, n_disps, wh, ww, block_size, subpixel=True):
+    """Winner-take-all disparity of census_vol_cuda's volume without writing it (ctd_census_disparity_*): (disp, score),
+    [B,1,H,W] (or [1,H,W])."""
+    sfx, (B, C, H, W) = _census_pair(in0, in1, "census_disparity")
+    shape = (B, 1, H, W) if in0.dim() == 4 else (1, H, W)
+    disp = torch.empty(shape, dtype=in0.dtype, device=in0.device)
+    score = torch.empty(shape, dtype=in0.dtype, device=in0.device)
+    with torch.cuda.device(in0.device):
+        _lib.call("ctd_census_disparity" + sfx, in0.data_ptr(), in1.data_ptr(), disp.data_ptr(), score.data_ptr(), B, C, H, W,
+                  int(n_disps), int(wh), int(ww), int(block_size), int(bool(subpixel)), _stream(in0))
+    return disp, score
+
+
 def _photometric_args(es, ta, type):
     _check_input_cuda(es, "es")
     _check_input_cuda(ta, "ta")

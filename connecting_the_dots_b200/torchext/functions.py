@@ -196,6 +196,117 @@ def sgm_aggregate_pytorch(vol, p1, p2, paths=8):
     return agg if vol.dim() == 4 else agg[0]
 
 
+def _census_check(op, window, block_size=1, C=0):
+    """The argument checks of the census entry points, with the C ABI's wording: (wh, ww) odd with 2 <= wh*ww <= 65,
+    block_size odd in [1, 15], C*(wh*ww-1)*block_size^2 <= 2^24."""
+    try:
+        wh, ww = (int(v) for v in window)
+    except (TypeError, ValueError):
+        raise RuntimeError("%s: window has to be a pair (wh, ww), got %r" % (op, window))
+    bs = int(block_size)
+    if wh < 1 or ww < 1 or wh % 2 == 0 or ww % 2 == 0:
+        raise RuntimeError("%s: window sides must be odd and positive, got %dx%d" % (op, wh, ww))
+    if not 2 <= wh * ww <= 65:
+        raise RuntimeError("%s: window %dx%d must have 2 to 65 taps" % (op, wh, ww))
+    if not (1 <= bs <= 15 and bs % 2 == 1):
+        raise RuntimeError("%s: block_size must be odd in [1,15], got %d" % (op, bs))
+    bound = C * (wh * ww - 1) * bs * bs
+    if bound > 1 << 24:
+        raise RuntimeError("%s: C*(wh*ww-1)*block_size^2 = %d exceeds 2^24 (scores would not be exact in float32)" % (op, bound))
+    return wh, ww, bs
+
+
+def _census_inputs(op, in0, in1, n_disps, window, block_size):
+    if in0.dim() not in (3, 4) or tuple(in0.shape) != tuple(in1.shape) or in0.dtype != in1.dtype:
+        raise RuntimeError("%s: in0 and in1 have to be C x H x W (or B x C x H x W) of the same shape and dtype" % op)
+    wh, ww, bs = _census_check(op, window, block_size, in0.size(-3))
+    B = in0.size(0) if in0.dim() == 4 else 1
+    if int(n_disps) < 1 and B * in0.size(-2) * in0.size(-1) > 0:
+        raise RuntimeError("%s: n_disps must be >= 1 (D = 0)" % op)
+    return wh, ww, bs
+
+
+def census_transform(x, window=(7, 9)):
+    """Census transform of each channel of x [B,C,H,W] (or [C,H,W]) over a window (wh, ww): int64 of x's shape holding the
+    uint64 bit pattern (bit 63 makes it negative), equal to census_transform_pytorch, which states the definition.  Not
+    differentiable.  CUDA tensors only, float32 or float64."""
+    if not x.is_cuda:
+        raise RuntimeError("torchext.census_transform: connecting_the_dots_b200 has no CPU implementation")
+    wh, ww, _ = _census_check("census_transform", window)
+    return ext_cuda.census_transform_cuda(x, wh, ww)
+
+
+def census_vol(in0, in1, n_disps, window=(7, 9), block_size=1):
+    """Census matching-score volume V [B,n_disps,H,W] (or [n_disps,H,W]) of in0 against in1 shifted by d, in the inputs'
+    dtype: minus the block_size^2 box sum of the Hamming distances of the census descriptors.  Higher is better (the
+    convention of xcorrvol), so sgm_disparity(census_vol(...), p1, p2) works as it is.  Equal bit for bit to
+    census_vol_pytorch, which states the definition.  Not differentiable.  CUDA tensors only, float32 or float64."""
+    if not in0.is_cuda:
+        raise RuntimeError("torchext.census_vol: connecting_the_dots_b200 has no CPU implementation")
+    wh, ww, bs = _census_inputs("census_vol", in0, in1, n_disps, window, block_size)
+    return ext_cuda.census_vol_cuda(in0, in1, n_disps, wh, ww, bs)
+
+
+def census_disparity(in0, in1, n_disps, window=(7, 9), block_size=9, subpixel=True):
+    """(disp, score) = disparity_from_volume(census_vol(in0, in1, n_disps, window, block_size), subpixel), bit for bit
+    including the sub-pixel offset, without writing the volume.  [B,1,H,W] (or [1,H,W]), not differentiable, CUDA tensors
+    only, float32 or float64."""
+    if not in0.is_cuda:
+        raise RuntimeError("torchext.census_disparity: connecting_the_dots_b200 has no CPU implementation")
+    wh, ww, bs = _census_inputs("census_disparity", in0, in1, n_disps, window, block_size)
+    return ext_cuda.census_disparity_cuda(in0, in1, n_disps, wh, ww, bs, subpixel)
+
+
+def census_transform_pytorch(x, window=(7, 9)):
+    """The definition of census_transform in plain torch, any device, and its test oracle.  Number the taps (i, j) of the
+    window, i in [0, wh), j in [0, ww), row-major, skipping the centre (wh//2, ww//2); bit k of T[b,c,h,w] is
+    x[b,c,clamp(h+i-wh//2),clamp(w+j-ww//2)] < x[b,c,h,w] (IEEE <: NaN on either side gives 0).  Higher bits are 0."""
+    wh, ww, _ = _census_check("census_transform", window)
+    xb = x if x.dim() == 4 else x.unsqueeze(0)
+    H, W = xb.shape[-2:]
+    rh, rw = wh // 2, ww // 2
+    taps = [(i, j) for i in range(wh) for j in range(ww) if (i, j) != (rh, rw)]
+    ti = torch.tensor([i - rh for i, _ in taps], device=x.device)
+    tj = torch.tensor([j - rw for _, j in taps], device=x.device)
+    rows = (torch.arange(H, device=x.device) + ti[:, None]).clamp(0, H - 1)     # [K,H]
+    cols = (torch.arange(W, device=x.device) + tj[:, None]).clamp(0, W - 1)     # [K,W]
+    bits = (xb[:, :, rows[:, :, None], cols[:, None, :]] < xb.unsqueeze(2)).long()  # [B,C,K,H,W]
+    shifts = torch.arange(len(taps), device=x.device).view(1, 1, -1, 1, 1)
+    t = (bits << shifts).sum(2)  # disjoint bits: the sum is their OR (bit 63 is the int64 sign)
+    return t if x.dim() == 4 else t[0]
+
+
+_POPCOUNT8 = torch.tensor([bin(i).count("1") for i in range(256)], dtype=torch.int32)
+
+
+def census_vol_pytorch(in0, in1, n_disps, window=(7, 9), block_size=1):
+    """The definition of census_vol in plain torch, any device, in the inputs' dtype, and its test oracle.  With T0, T1 =
+    census_transform_pytorch(in0, in1): Hm[b,d,h,w] = sum_c popcount(T0[b,c,h,w] ^ T1[b,c,h,clamp(w-d,0,W-1)]);
+    S[b,d,h,w] = sum over i, j in [0, bs) of Hm[b,d,clamp(h+i-bs//2),clamp(w+j-bs//2)]; V = -S.  census_disparity's
+    definition is disparity_from_volume(census_vol_pytorch(...))."""
+    wh, ww, bs = _census_inputs("census_vol", in0, in1, n_disps, window, block_size)
+    if in0.dtype not in (torch.float32, torch.float64):
+        raise NotImplementedError("census_vol: float32 or float64 inputs only")
+    a = in0 if in0.dim() == 4 else in0.unsqueeze(0)
+    b = in1 if in1.dim() == 4 else in1.unsqueeze(0)
+    B, C, H, W = a.shape
+    D, r = int(n_disps), bs // 2
+    t0, t1 = census_transform_pytorch(a, (wh, ww)), census_transform_pytorch(b, (wh, ww))
+    lut = _POPCOUNT8.to(a.device)
+    cols = torch.arange(W, device=a.device)
+    box_r = (torch.arange(H, device=a.device) + torch.arange(-r, r + 1, device=a.device)[:, None]).clamp(0, H - 1)  # [bs,H]
+    box_c = (cols + torch.arange(-r, r + 1, device=a.device)[:, None]).clamp(0, W - 1)                               # [bs,W]
+    vol = torch.empty(B, D, H, W, dtype=in0.dtype, device=in0.device)
+    for d in range(D):
+        x = (t0 ^ t1[..., (cols - d).clamp(min=0)]).contiguous()
+        hm = lut[x.view(torch.uint8).long()].view(B, C, H, W, 8).sum((1, 4))   # [B,H,W]
+        if r:
+            hm = hm[:, box_r].sum(1)          # [B,bs,H,W] -> rows summed
+            hm = hm[:, :, box_c].sum(2)       # [B,H,bs,W] -> columns summed
+        vol[:, d] = -(hm.to(in0.dtype))
+    return vol if in0.dim() == 4 else vol[0]
+
+
 class PhotometricLossFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, es, ta, block_size, type, eps):

@@ -82,6 +82,33 @@ class SGMDisparity(torch.nn.Module):
         return F.sgm_disparity(F.xcorrvol(in0, in1, self.n_disps, self.block_size), self.p1, self.p2, self.paths, self.subpixel)
 
 
+class CensusDisparity(torch.nn.Module):
+    """forward(in0, in1) -> (disp, score) of census_disparity: the winner-take-all disparity of census_vol's volume."""
+
+    def __init__(self, n_disps=128, window=(7, 9), block_size=9, subpixel=True):
+        super().__init__()
+        self.n_disps, self.window, self.block_size, self.subpixel = n_disps, tuple(window), block_size, subpixel
+
+    def forward(self, in0, in1):
+        return F.census_disparity(in0, in1, self.n_disps, self.window, self.block_size, self.subpixel)
+
+
+class CensusSGMDisparity(torch.nn.Module):
+    """forward(in0, in1) -> (disp, score): census_vol(in0, in1, n_disps, window, block_size), then sgm_disparity over it.
+    The default penalties (p1 = 6, p2 = 400 in Hamming units, 8 paths) were tuned on two synthetic frames only: a CPU sweep
+    of the definition over p1 in 3..16 and p2 in 100..1000 on synth.make_batch(2) put 0.911 (8 paths) and 0.913 (4 paths)
+    of the interior pixels within 2 px of the ground truth, against 0.849 and 0.789 at p1 = 10, p2 = 120."""
+
+    def __init__(self, n_disps=128, window=(7, 9), block_size=1, p1=6, p2=400, paths=8, subpixel=True):
+        super().__init__()
+        self.n_disps, self.window, self.block_size = n_disps, tuple(window), block_size
+        self.p1, self.p2, self.paths, self.subpixel = p1, p2, paths, subpixel
+
+    def forward(self, in0, in1):
+        vol = F.census_vol(in0, in1, self.n_disps, self.window, self.block_size)
+        return F.sgm_disparity(vol, self.p1, self.p2, self.paths, self.subpixel)
+
+
 class CrossCheck(torch.nn.Module):
     def forward(self, in0, in1):
         return F.crosscheck(in0, in1)

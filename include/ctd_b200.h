@@ -179,6 +179,42 @@ int ctd_sgm_f32(const float* vol, float* agg, float* disp, float* score, int64_t
 int ctd_sgm_f64(const double* vol, double* agg, double* disp, double* score, int64_t B, int64_t D, int64_t H, int64_t W,
                 double p1, double p2, int paths, int subpixel, ctd_stream_t stream);
 
+/* ---- census-transform stereo matching (an addition: Zabih & Woodfill 1994).  in0, in1 [B,C,H,W].  The window is
+ * (wh, ww), both odd, 2 <= wh*ww <= 65; rh = wh/2, rw = ww/2.  block_size = bs is odd, 1 <= bs <= 15; r = bs/2.
+ *   1. Census transform.  T[b,c,h,w] is a uint64.  Number the window taps (i, j), i in [0,wh), j in [0,ww), row-major,
+ *      skipping the centre (rh, rw).  Bit k, for the k-th tap, is
+ *      x[b,c,clamp(h+i-rh,0,H-1),clamp(w+j-rw,0,W-1)] < x[b,c,h,w].  Bits from wh*ww - 1 up are 0.  The comparison is
+ *      IEEE <, so a NaN on either side gives 0: non-finite input is defined.
+ *   2. Per-pixel Hamming cost.  Hm[b,d,h,w] = sum_c popcount(T0[b,c,h,w] XOR T1[b,c,h,clamp(w-d,0,W-1)]).
+ *   3. Aggregated cost.  S[b,d,h,w] = sum_{i,j in [0,bs)} Hm[b,d,clamp(h+i-r,0,H-1),clamp(w+j-r,0,W-1)] (a
+ *      replicate-padded box filter of the bs = 1 volume).
+ *   4. Score volume.  V = -S in the input's dtype: higher is better, the convention of ctd_xcorrvol_* and ctd_sgm_*.  |V|
+ *      <= C*(wh*ww-1)*bs^2, and calls where that bound exceeds 2^24 are rejected, so fp32 holds every value exactly.
+ *   5. Disparity.  (disp, score) = the winner-take-all of V as ctd_xcorr_disparity_* states it for a volume: the first
+ *      maximum of V (the smallest d among equal least costs), score = V at d*, and the optional fp64 three-point
+ *      sub-pixel offset, computed from the same integers, so the fused result is bit-equal to that of the volume.
+ * ctd_census_transform_* writes T (out [B,C,H,W] uint64).  ctd_census_vol_* writes V (out [B,n_disps,H,W]).
+ * ctd_census_disparity_* writes disp [B,1,H,W] and score [B,1,H,W] (score may be NULL) without writing V.
+ * CTD_ERR_INVALID, checked before any device work, for: an even or non-positive window side, wh*ww < 2 or > 65; an even
+ * block_size or one outside 1..15; the 2^24 bound; negative sizes; null pointers; n_disps < 1 when B*H*W > 0; an
+ * output that overlaps an input (or disp overlapping score).  B*H*W = 0 (B*C*H*W = 0 for the transform) is CTD_OK with
+ * nothing launched.  DEVICE pointers; descriptor scratch (2*B*C*H*W*8 bytes) comes from the library's stream-ordered
+ * pool; no atomics, no host synchronisation, capture-safe; 64-bit indexing.  One kernel path per entry point:
+ * "force_generic" does not apply. */
+int ctd_census_transform_f32(const float* in, uint64_t* out, int64_t B, int64_t C, int64_t H, int64_t W, int wh, int ww,
+                             ctd_stream_t stream);
+int ctd_census_transform_f64(const double* in, uint64_t* out, int64_t B, int64_t C, int64_t H, int64_t W, int wh, int ww,
+                             ctd_stream_t stream);
+int ctd_census_vol_f32(const float* in0, const float* in1, float* out, int64_t B, int64_t C, int64_t H, int64_t W,
+                       int64_t n_disps, int wh, int ww, int block_size, ctd_stream_t stream);
+int ctd_census_vol_f64(const double* in0, const double* in1, double* out, int64_t B, int64_t C, int64_t H, int64_t W,
+                       int64_t n_disps, int wh, int ww, int block_size, ctd_stream_t stream);
+int ctd_census_disparity_f32(const float* in0, const float* in1, float* disp, float* score, int64_t B, int64_t C, int64_t H,
+                             int64_t W, int64_t n_disps, int wh, int ww, int block_size, int subpixel, ctd_stream_t stream);
+int ctd_census_disparity_f64(const double* in0, const double* in1, double* disp, double* score, int64_t B, int64_t C,
+                             int64_t H, int64_t W, int64_t n_disps, int wh, int ww, int block_size, int subpixel,
+                             ctd_stream_t stream);
+
 /* ---- ProjNNFunctor: ext.h:65-117, ext_cuda.cpp:47-69 (proj_nn_cuda).  K is a DEVICE pointer to
  * 9 values (row-major 3x3), like the reference's K tensor. */
 int ctd_proj_nn_f32(const float* xyz0, const float* xyz1, const float* K, int64_t* out, int64_t B,

@@ -3,7 +3,7 @@
 launching stream, rotating buffer sets larger than L2 where the op is HBM-bound).  Prints one JSON
 object; bench.py stays the contract benchmark, this is the per-op table that goes into profiles/.
 
-    python tools/bench_ops.py [--iters 30] [--only photometric,ssim,lcn,xcorrvol,xcorr_disparity,sgm,proj_nn,nn,crosscheck]
+    python tools/bench_ops.py [--iters 30] [--only photometric,ssim,lcn,xcorrvol,xcorr_disparity,sgm,census_match,proj_nn,nn,crosscheck]
 
 The printed result names the GPU and its power limit, read in the same run.
 """
@@ -70,7 +70,14 @@ def device_info(index):
     return info
 
 
-ALL = "calib,photometric,ssim,warp,pyramid,geometric,disparity,lcn,xcorrvol,xcorr_disparity,sgm,proj_nn,config4,nn,crosscheck,reduce,gpu_reference"
+def census_traffic(B, C, H, W, D):
+    """Least HBM bytes of the census calls, from shapes: the volume writes 4 B per pixel and disparity and reads both fp32
+    inputs; the fused disparity reads the inputs and writes disp and score (16 B/px at C = 1)."""
+    npx = B * H * W
+    return {"volume": (4 * D + 8 * C) * npx, "disparity": (8 * C + 8) * npx}
+
+
+ALL = "calib,photometric,ssim,warp,pyramid,geometric,disparity,lcn,xcorrvol,xcorr_disparity,sgm,census_match,proj_nn,config4,nn,crosscheck,reduce,gpu_reference"
 
 
 def main():
@@ -415,6 +422,62 @@ def run(only=ALL, iters=30, batch=8, device_index=0, verbose=True):
             add("sgm_pytorch_restatement_8paths_D128", ms, ms, floor, extra={"note": "sgm_aggregate_pytorch + disparity_from_volume"})
             res["ops"]["sgm_disparity_8paths_D128"]["speedup_vs_torch"] = ms / res["ops"]["sgm_disparity_8paths_D128"]["ms_median"]
         del vol, agg
+    if "census_match" in only:
+        # census matching (7x9 window, D = 128) on the bench frames (ta against pat_lcn), in the same run on the same inputs:
+        # the volume at block 1 (what SGM consumes), the fused disparity at block 9 (sub-pixel on), the unfused pair
+        # census_vol(bs 9) + disparity_from_volume, the torch restatement on the GPU, and census_vol(bs 1) -> sgm_disparity.
+        D = 128
+        floors = census_traffic(B, 1, H, W, D)
+        vol = torch.empty(B, D, H, W, device=dev)
+        o_d, o_s = torch.empty(B, 1, H, W, device=dev), torch.empty(B, 1, H, W, device=dev)
+        it = max(3, args.iters // 6)
+
+        def vol_call(i, st, bs):
+            d = sets[i % NS]
+            _lib.call("ctd_census_vol_f32", d["ta"].data_ptr(), d["pat_lcn"].data_ptr(), vol.data_ptr(), B, 1, H, W, D, 7, 9, bs, st)
+
+        def f(i, st):
+            d = sets[i % NS]
+            _lib.call("ctd_census_disparity_f32", d["ta"].data_ptr(), d["pat_lcn"].data_ptr(), o_d.data_ptr(), o_s.data_ptr(),
+                      B, 1, H, W, D, 7, 9, 9, 1, st)
+
+        def g(i, st):
+            vol_call(i, st, 9)
+            dd, ss = tx.disparity_from_volume(vol, True)
+            o_d.copy_(dd)
+            o_s.copy_(ss)
+
+        def sgm(i, st):
+            vol_call(i, st, 1)
+            dd, ss = tx.sgm_disparity(vol, 6, 400, 8)
+            o_d.copy_(dd)
+            o_s.copy_(ss)
+        add("census_vol_D128_bs1", *timeit(lambda i, st: vol_call(i, st, 1), it, warmup=1, nrep=2), floors["volume"],
+            extra={"note": "algo_bytes: in0, in1 in (8 B/px), V out (4D B/px)"})
+        add("census_disparity_D128_bs9", *timeit(f, it, warmup=1, nrep=2), floors["disparity"],
+            extra={"note": "algo_bytes: in0, in1 in, disp and score out (16 B/px); the volume is never written"})
+        add("census_vol_bs9_then_disparity_from_volume_D128", *timeit(g, it, warmup=1, nrep=2), floors["volume"],
+            extra={"note": "census_vol(bs 9) writes V, disparity_from_volume reads it back in torch"})
+        res["ops"]["census_disparity_D128_bs9"]["speedup_vs_unfused"] = (
+            res["ops"]["census_vol_bs9_then_disparity_from_volume_D128"]["ms_median"] / res["ops"]["census_disparity_D128_bs9"]["ms_median"])
+        add("census_vol_bs1_then_sgm_disparity_8paths_D128", *timeit(sgm, it, warmup=1, nrep=2), floors["volume"],
+            extra={"note": "census_vol(bs 1) then sgm_disparity(p1 = 6, p2 = 400, 8 paths); algo_bytes is the volume's floor only"})
+        if B <= 8:
+            # the torch restatement on the GPU (a loop over d of gathers, XOR and a byte popcount table), timed eagerly
+            a, b = sets[0]["ta"], sets[0]["pat_lcn"]
+            tx.disparity_from_volume(tx.census_vol_pytorch(a, b, D, (7, 9), 9), True)
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            torch.cuda.synchronize()
+            e0.record()
+            for _ in range(2):
+                tx.disparity_from_volume(tx.census_vol_pytorch(a, b, D, (7, 9), 9), True)
+            e1.record()
+            torch.cuda.synchronize()
+            ms = e0.elapsed_time(e1) / 2
+            add("census_pytorch_restatement_bs9_D128", ms, ms, floors["volume"],
+                extra={"note": "disparity_from_volume(census_vol_pytorch(bs 9))"})
+            res["ops"]["census_disparity_D128_bs9"]["speedup_vs_torch"] = ms / res["ops"]["census_disparity_D128_bs9"]["ms_median"]
+        del vol
     if "proj_nn" in only:
         T = 4
         xyz, K, poses = synth.make_clouds(T, H, W)
