@@ -154,6 +154,25 @@ def sgm_cuda(vol, p1, p2, paths=8, subpixel=True, want_disparity=True):
     return agg, disp, score
 
 
+def disparity_check_cuda(vol, max_diff=1, uniqueness=0.0, subpixel=True):
+    """Left-right consistency and uniqueness checks over a score volume (ctd_disparity_check_*).  vol [B,D,H,W] (or
+    [D,H,W]) -> (disp, score, valid), [B,1,H,W] (or [1,H,W]); valid is torch.bool."""
+    _check_input_cuda(vol, "vol")
+    _check(vol.dim() in (3, 4), "vol has to be D x H x W (or B x D x H x W)")
+    sfx = _real_suffix(vol, "disparity_check")
+    batched = vol.dim() == 4
+    B = vol.size(0) if batched else 1
+    D, H, W = vol.shape[-3:]
+    shape = (B, 1, H, W) if batched else (1, H, W)
+    disp = torch.empty(shape, dtype=vol.dtype, device=vol.device)
+    score = torch.empty(shape, dtype=vol.dtype, device=vol.device)
+    valid = torch.empty(shape, dtype=torch.bool, device=vol.device)
+    with torch.cuda.device(vol.device):
+        _lib.call("ctd_disparity_check" + sfx, vol.data_ptr(), disp.data_ptr(), score.data_ptr(), None, None, valid.data_ptr(),
+                  B, D, H, W, int(max_diff), float(uniqueness), int(bool(subpixel)), _stream(vol))
+    return disp, score, valid
+
+
 def census_transform_cuda(x, wh, ww):
     """Census transform (ctd_census_transform_*): x [B,C,H,W] (or [C,H,W]) -> int64 of the same shape holding the uint64
     bit patterns."""

@@ -117,7 +117,87 @@ def disparity_from_volume(vol, subpixel=True):
     return disp, score
 
 
-SGM_PATHS = {4: ((0, 1), (0, -1), (1, 0), (-1, 0)),
+def _disparity_check_args(op, vol, uniqueness):
+    if vol.dim() not in (3, 4):
+        raise RuntimeError("%s: vol has to be D x H x W (or B x D x H x W)" % op)
+    u = float(uniqueness)
+    if not (u >= 0.0 and u != float("inf")):
+        raise RuntimeError("%s: uniqueness must be finite and >= 0, got %r" % (op, uniqueness))
+    return u
+
+
+def disparity_check(vol, max_diff=1, uniqueness=0.0, subpixel=True):
+    """Left-right consistency and uniqueness checks of the winner-take-all disparity of a score volume vol [B,D,H,W] (or
+    [D,H,W]; higher is better, the convention of xcorrvol, census_vol and sgm_aggregate), in one pass over the volume.
+    Returns (disp, score, valid), [B,1,H,W] (or [1,H,W]): disp and score equal disparity_from_volume(vol, subpixel) bit for
+    bit, valid (torch.bool) marks the pixels that pass both checks as disparity_check_pytorch states them.  max_diff < 0
+    turns the LR check off, uniqueness = 0 the uniqueness check.  Not differentiable.  CUDA tensors only, float32 or
+    float64."""
+    if not vol.is_cuda:
+        raise RuntimeError("torchext.disparity_check: connecting_the_dots_b200 has no CPU implementation")
+    u = _disparity_check_args("disparity_check", vol, uniqueness)
+    return ext_cuda.disparity_check_cuda(vol, int(max_diff), u, subpixel)
+
+
+def right_disparity_from_volume(vol, subpixel=True):
+    """Winner-take-all disparity of the right view of a score volume [B,D,H,W] (or [D,H,W]) in plain torch, any device:
+    part of disparity_check's definition and its test oracle.  For right pixel x, Dx = min(D, W - x) and VR[d,h,x] =
+    V[d,h,x+d] for d < Dx.  dR* = the first d in [0, Dx) with the largest VR, score = VR at dR*; with subpixel, c-, c0, c+
+    = VR at dR* - 1, dR*, dR* + 1 and disparity_from_volume's fp64 offset, 0 where dR* = 0, dR* = Dx - 1 or den >= 0.
+    Returns (disp, score), [B,1,H,W] (or [1,H,W]), in vol's dtype.  For volumes without NaN."""
+    v = vol if vol.dim() == 4 else vol.unsqueeze(0)
+    B, D, H, W = v.shape
+    if D < 1:
+        raise RuntimeError("right_disparity_from_volume: the volume has no disparities")
+    idx = torch.arange(D, device=v.device).view(1, D, 1, 1)
+    x = torch.arange(W, device=v.device).view(1, 1, 1, W)
+    cols = x + idx                                                  # [1,D,1,W]
+    ok = cols < W
+    vr = v.gather(3, cols.clamp(max=W - 1).expand(B, D, H, W))      # VR where ok, a clamped column elsewhere
+    best = torch.where(ok, vr, float("-inf")).amax(dim=1, keepdim=True)
+    d = torch.where(ok & (vr == best), idx, D).amin(dim=1, keepdim=True)
+    score = vr.gather(1, d)
+    disp = d.to(torch.float64)
+    if subpixel:
+        dx = (W - x).clamp(max=D)
+        cm = vr.gather(1, (d - 1).clamp(min=0)).double()
+        c0 = score.double()
+        cp = vr.gather(1, (d + 1).clamp(max=D - 1)).double()
+        den = cm - 2 * c0 + cp
+        ok = (d > 0) & (d < dx - 1) & (den < 0)
+        delta = torch.where(ok, (cm - cp) / (2 * torch.where(ok, den, -1.0)), 0.0).clamp(-0.5, 0.5)
+        disp = disp + delta
+    disp = disp.to(vol.dtype)
+    if vol.dim() == 3:
+        disp, score = disp[0], score[0]
+    return disp, score
+
+
+def disparity_check_pytorch(vol, max_diff=1, uniqueness=0.0, subpixel=True):
+    """The definition of disparity_check in plain torch, any device, and its test oracle.  (disp, score) =
+    disparity_from_volume(vol, subpixel); with d*L the integer left disparity and dR* that of right_disparity_from_volume,
+    valid = LR and uniqueness, where LR: max_diff < 0, or x = w - d*L >= 0 and |d*L - dR*(x)| <= max_diff; uniqueness:
+    uniqueness == 0, or no d has |d - d*L| >= 2, or (double)vol[d*L] - (double)max{vol[d] : |d - d*L| >= 2} >= uniqueness."""
+    u = _disparity_check_args("disparity_check", vol, uniqueness)
+    v = vol if vol.dim() == 4 else vol.unsqueeze(0)
+    B, D, H, W = v.shape
+    disp, score = disparity_from_volume(v, subpixel)
+    dl = disparity_from_volume(v, False)[0].long()
+    dr = right_disparity_from_volume(v, False)[0].long()
+    valid = torch.ones_like(dl, dtype=torch.bool)
+    if max_diff >= 0:
+        x = torch.arange(W, device=v.device).view(1, 1, 1, W) - dl
+        valid &= (x >= 0) & ((dl - dr.gather(3, x.clamp(min=0))).abs() <= max_diff)
+    if u != 0:
+        far = (torch.arange(D, device=v.device).view(1, D, 1, 1) - dl).abs() >= 2
+        second = torch.where(far, v, float("-inf")).amax(dim=1, keepdim=True)
+        valid &= ~far.any(dim=1, keepdim=True) | (score.double() - second.double() >= u)
+    if vol.dim() == 3:
+        disp, score, valid = disp[0], score[0], valid[0]
+    return disp, score, valid
+
+
+SGM_PATHS = {4:((0, 1), (0, -1), (1, 0), (-1, 0)),
              8: ((0, 1), (0, -1), (1, 0), (-1, 0), (1, 1), (1, -1), (-1, 1), (-1, -1))}
 
 

@@ -109,6 +109,19 @@ class CensusSGMDisparity(torch.nn.Module):
         return F.sgm_disparity(vol, self.p1, self.p2, self.paths, self.subpixel)
 
 
+class DisparityCheck(torch.nn.Module):
+    """forward(vol) -> (disp, score, valid) of disparity_check: the winner-take-all disparity of a score volume and the
+    mask of pixels that pass the left-right consistency and uniqueness checks.
+    DisparityCheck()(sgm_aggregate(census_vol(in0, in1, 128), 6, 400)) is a full classical stereo pipeline."""
+
+    def __init__(self, max_diff=1, uniqueness=0.0, subpixel=True):
+        super().__init__()
+        self.max_diff, self.uniqueness, self.subpixel = max_diff, uniqueness, subpixel
+
+    def forward(self, vol):
+        return F.disparity_check(vol, self.max_diff, self.uniqueness, self.subpixel)
+
+
 class CrossCheck(torch.nn.Module):
     def forward(self, in0, in1):
         return F.crosscheck(in0, in1)

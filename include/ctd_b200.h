@@ -215,6 +215,32 @@ int ctd_census_disparity_f64(const double* in0, const double* in1, double* disp,
                              int64_t H, int64_t W, int64_t n_disps, int wh, int ww, int block_size, int subpixel,
                              ctd_stream_t stream);
 
+/* ---- left-right consistency and uniqueness checks over a score volume (an addition: the post-processing of Hirschmueller's
+ * SGM and of OpenCV's StereoSGBM).  vol [B,D,H,W], higher is better (the convention of ctd_xcorrvol_*, ctd_census_vol_*
+ * and ctd_sgm_*); V[b,d,h,w] scores left pixel w against right pixel w - d.
+ *   1. Left view.  disp, score = the winner-take-all of V exactly as ctd_xcorr_disparity_* states it for a volume: d*L =
+ *      the first d with the largest V, score = V at d*L, optional fp64 three-point sub-pixel offset.
+ *   2. Right view.  For right pixel x, Dx = min(D, W - x) and VR[d,h,x] = V[d,h,x+d], d < Dx (the diagonal x + d <= W - 1:
+ *      never the clamped columns a volume holds for d > w).  dR* = the first d in [0, Dx) with the largest VR,
+ *      score_right = VR at dR*, disp_right = dR* plus the same offset with c-, c+ = V[dR*-1, h, x+dR*-1],
+ *      V[dR*+1, h, x+dR*+1]; the offset is 0 when dR* = 0, dR* = Dx - 1 or den >= 0.
+ *   3. valid[b,0,h,w] = 1 when both hold, else 0:
+ *      LR:          max_diff < 0 (check off), or x = w - d*L >= 0 and |d*L - dR*(x)| <= max_diff (integer indices);
+ *      uniqueness:  uniqueness == 0 (check off), or {d : |d - d*L| >= 2} is empty, or
+ *                   (double)V[d*L] - (double)second >= uniqueness, second = the maximum of V over that set.
+ * Only maxima, compares and those fp64 operations are involved, so every output is bit-equal to the definition.  Outputs
+ * [B,1,H,W] (valid as uint8), DEVICE pointers, each may be NULL.  CTD_ERR_INVALID, checked before any device work, for:
+ * negative sizes; a negative or non-finite uniqueness; D < 1 when B*H*W > 0; a null vol; an output overlapping vol or
+ * another output.  B*H*W = 0 is CTD_OK with nothing launched.  One pass over the volume; the right disparities of a row go
+ * through (grid x W x 4 bytes of) scratch from the library's stream-ordered pool; no atomics, no host synchronisation,
+ * capture-safe; 64-bit indexing.  The volume must not hold NaN: for it the result is unspecified (the call does not fault). */
+int ctd_disparity_check_f32(const float* vol, float* disp, float* score, float* disp_right, float* score_right,
+                            uint8_t* valid, int64_t B, int64_t D, int64_t H, int64_t W, int max_diff, double uniqueness,
+                            int subpixel, ctd_stream_t stream);
+int ctd_disparity_check_f64(const double* vol, double* disp, double* score, double* disp_right, double* score_right,
+                            uint8_t* valid, int64_t B, int64_t D, int64_t H, int64_t W, int max_diff, double uniqueness,
+                            int subpixel, ctd_stream_t stream);
+
 /* ---- ProjNNFunctor: ext.h:65-117, ext_cuda.cpp:47-69 (proj_nn_cuda).  K is a DEVICE pointer to
  * 9 values (row-major 3x3), like the reference's K tensor. */
 int ctd_proj_nn_f32(const float* xyz0, const float* xyz1, const float* K, int64_t* out, int64_t B,

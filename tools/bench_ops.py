@@ -3,7 +3,7 @@
 launching stream, rotating buffer sets larger than L2 where the op is HBM-bound).  Prints one JSON
 object; bench.py stays the contract benchmark, this is the per-op table that goes into profiles/.
 
-    python tools/bench_ops.py [--iters 30] [--only photometric,ssim,lcn,xcorrvol,xcorr_disparity,sgm,census_match,proj_nn,nn,crosscheck]
+    python tools/bench_ops.py [--iters 30] [--only photometric,ssim,lcn,xcorrvol,xcorr_disparity,sgm,census_match,disparity_check,proj_nn,nn,crosscheck]
 
 The printed result names the GPU and its power limit, read in the same run.
 """
@@ -77,7 +77,7 @@ def census_traffic(B, C, H, W, D):
     return {"volume": (4 * D + 8 * C) * npx, "disparity": (8 * C + 8) * npx}
 
 
-ALL = "calib,photometric,ssim,warp,pyramid,geometric,disparity,lcn,xcorrvol,xcorr_disparity,sgm,census_match,proj_nn,config4,nn,crosscheck,reduce,gpu_reference"
+ALL = "calib,photometric,ssim,warp,pyramid,geometric,disparity,lcn,xcorrvol,xcorr_disparity,sgm,census_match,disparity_check,proj_nn,config4,nn,crosscheck,reduce,gpu_reference"
 
 
 def main():
@@ -477,6 +477,47 @@ def run(only=ALL, iters=30, batch=8, device_index=0, verbose=True):
             add("census_pytorch_restatement_bs9_D128", ms, ms, floors["volume"],
                 extra={"note": "disparity_from_volume(census_vol_pytorch(bs 9))"})
             res["ops"]["census_disparity_D128_bs9"]["speedup_vs_torch"] = ms / res["ops"]["census_disparity_D128_bs9"]["ms_median"]
+        del vol
+    if "disparity_check" in only:
+        # left-right consistency and uniqueness checks over the census block-1 volume of the bench frames (7x9 window,
+        # D = 128): the fused call (disp, score and valid; max_diff = 1, uniqueness = 16), the torch restatement on the GPU
+        # and disparity_from_volume alone, in the same run.  The volume is larger than L2 at batch 8 already, so one input
+        # serves every launch; the floor is one read of it (4D B/px).
+        D = 128
+        vol = torch.empty(B, D, H, W, device=dev)
+        _lib.call("ctd_census_vol_f32", sets[0]["ta"].data_ptr(), sets[0]["pat_lcn"].data_ptr(), vol.data_ptr(), B, 1, H, W, D,
+                  7, 9, 1, torch.cuda.current_stream().cuda_stream)
+        o_d, o_s = torch.empty(B, 1, H, W, device=dev), torch.empty(B, 1, H, W, device=dev)
+        o_v = torch.empty(B, 1, H, W, dtype=torch.uint8, device=dev)
+        floor = 4 * D * npx
+        it = max(3, args.iters // 6)
+
+        def f(i, st):
+            _lib.call("ctd_disparity_check_f32", vol.data_ptr(), o_d.data_ptr(), o_s.data_ptr(), None, None, o_v.data_ptr(),
+                      B, D, H, W, 1, 16.0, 1, st)
+
+        def g(i, st):
+            dd, ss = tx.disparity_from_volume(vol, True)
+            o_d.copy_(dd)
+            o_s.copy_(ss)
+        add("disparity_check_D128", *timeit(f, it, warmup=2, nrep=4), floor,
+            extra={"note": "census_vol(bs 1) volume in (4D B/px, the floor); disp, score and valid out (9 B/px)"})
+        add("disparity_from_volume_D128", *timeit(g, it, warmup=2, nrep=4), floor,
+            extra={"note": "torch winner-take-all with sub-pixel offset only: no right view, no checks"})
+        tx.disparity_check_pytorch(vol, 1, 16.0)
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        torch.cuda.synchronize()
+        e0.record()
+        for _ in range(2):
+            tx.disparity_check_pytorch(vol, 1, 16.0)
+        e1.record()
+        torch.cuda.synchronize()
+        ms = e0.elapsed_time(e1) / 2
+        add("disparity_check_pytorch_D128", ms, ms, floor, extra={"note": "disparity_check_pytorch on the GPU, timed eagerly"})
+        r = res["ops"]["disparity_check_D128"]
+        r["speedup_vs_torch"] = ms / r["ms_median"]
+        r["ratio_vs_disparity_from_volume"] = res["ops"]["disparity_from_volume_D128"]["ms_median"] / r["ms_median"]
+        r["valid_frac"] = float(o_v.float().mean())
         del vol
     if "proj_nn" in only:
         T = 4
