@@ -12,9 +12,9 @@
 //   * census_match<T, R, WTA>: a CTA owns CM_ROWS rows x 128 columns of one image, a warp a row, a lane 4 adjacent
 //     pixels.  For each d in order it forms the Hamming plane of the tile plus its R = bs/2 halo (POPC of the XOR of the
 //     two descriptors per channel, read through L1), sums it by columns then by rows in shared memory (exact integer
-//     sums), and either stores the tile's row of V[d] (128-bit where aligned) or updates the lane's running best: least
-//     S, the first d that reached it, S at d* - 1 and S at d* + 1 (caught on the step after a new best).  R = 0 (bs = 1,
-//     the volume SGM consumes) is a compile-time case with no shared memory: the lane's own four pixels are the plane.
+//     sums), and either stores the tile's row of V[d] (128-bit where aligned) or steps the winner-take-all run
+//     (WtaRun, ctd_common.cuh) of each of the lane's pixels over -S as int.  R = 0 (bs = 1, the volume SGM consumes) is a
+//     compile-time case with no shared memory: the lane's own four pixels are the plane.
 // No atomics, no cudaMalloc (descriptor scratch comes from the library pool, stream-ordered), no host synchronisation:
 // every call is capture-safe.
 #include <algorithm>
@@ -122,10 +122,9 @@ census_match(const uint64_t* __restrict__ t0, const uint64_t* __restrict__ t1, T
     const int h = h0 + row, w = w0 + 4 * lane;
     const uint64_t* a0 = t0 + b * C * plane;
     const uint64_t* a1 = t1 + b * C * plane;
-    int best[4], bd[4], sm[4], sp[4], prev[4];
-    bool want_p[4];
+    WtaRun<int> run[4];  // over -S: its first maximum is the first minimum of S
 #pragma unroll
-    for (int k = 0; k < 4; ++k) best[k] = 0, bd[k] = 0, sm[k] = 0, sp[k] = 0, prev[k] = 0, want_p[k] = false;
+    for (int k = 0; k < 4; ++k) run[k].init();
     for (int d = 0; d < D; ++d) {
       int s[4];
       if constexpr (R == 0) {
@@ -195,14 +194,7 @@ census_match(const uint64_t* __restrict__ t0, const uint64_t* __restrict__ t1, T
           store4<T>(vol + (b * D + d) * plane + (int64_t)h * W + w, w, W, s);
         } else {
 #pragma unroll
-          for (int k = 0; k < 4; ++k) {
-            if (d == 0 || s[k] < best[k]) {
-              best[k] = s[k], bd[k] = d, sm[k] = prev[k], want_p[k] = true;
-            } else if (want_p[k]) {
-              sp[k] = s[k], want_p[k] = false;
-            }
-            prev[k] = s[k];
-          }
+          for (int k = 0; k < 4; ++k) run[k].step(-s[k], d);
         }
       }
     }
@@ -210,15 +202,9 @@ census_match(const uint64_t* __restrict__ t0, const uint64_t* __restrict__ t1, T
 #pragma unroll
       for (int k = 0; k < 4; ++k) {
         if (w + k >= W) break;
-        const int64_t px = b * plane + (int64_t)h * W + w + k;
-        if (score) score[px] = -(T)best[k];
-        if (disp) {
-          // the three scores -S in the volume's dtype, then disparity_from_volume's fp64 parabola
-          const double delta = subpixel && bd[k] > 0 && bd[k] < D - 1
-                                   ? wta_subpixel((double)(-(T)sm[k]), (double)(-(T)best[k]), (double)(-(T)sp[k]))
-                                   : 0.0;
-          disp[px] = (T)((double)bd[k] + delta);
-        }
+        // the score is -(T)S like the volume's (S = 0 is -0.0); the sign of a zero cm or cp does not change the offset
+        const WtaRun<int>& r = run[k];
+        wta_store<T>(disp, score, b * plane + (int64_t)h * W + w + k, r.bd, -(T)(-r.best), (T)r.cm, (T)r.cp, D, subpixel);
       }
     }
   }
@@ -228,9 +214,8 @@ template <typename T>
 int transform_launch(const T* in, uint64_t* out, int64_t nimg, int H, int W, int wh, int ww, cudaStream_t st) {
   const size_t smem = (size_t)(CT_ROWS + 2 * (wh / 2)) * (TILE_W + 2 * (ww / 2)) * sizeof(T);
   auto kernel = census_transform_kernel<T>;
-  // the attribute belongs to the device: set on every call (a process may use several GPUs)
-  if (smem > 48 * 1024 && cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-    return fail(CTD_ERR_CUDA, "census_transform: cannot raise the shared-memory limit to %zu bytes", smem);
+  const int rs = raise_smem_limit(kernel, smem, "census_transform");
+  if (rs != CTD_OK) return rs;
   const int64_t ntiles = nimg * cdiv(W, TILE_W) * cdiv(H, CT_ROWS);
   kernel<<<(unsigned)std::min<int64_t>(ntiles, INT32_MAX), 32 * CT_ROWS, smem, st>>>(in, out, nimg, H, W, wh, ww);
   count_launch();
@@ -263,11 +248,6 @@ int match_launch(const uint64_t* t0, const uint64_t* t1, T* vol, T* disp, T* sco
   return fail(CTD_ERR_INVALID, "census: block_size %d out of range", bs);
 }
 
-bool disjoint(const void* a, size_t na, const void* b, size_t nb) {
-  const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
-  return na == 0 || nb == 0 || x + na <= y || y + nb <= x;
-}
-
 // the checks every entry point shares, in the order the header lists them (before any device work)
 int check_window(const char* op, int64_t B, int64_t C, int64_t H, int64_t W, int wh, int ww, int bs) {
   CTD_REQUIRE(wh >= 1 && ww >= 1 && (wh & 1) && (ww & 1), "%s: window sides must be odd and positive, got %dx%d", op, wh, ww);
@@ -291,7 +271,7 @@ static int census_transform_impl(const T* in, uint64_t* out, int64_t B, int64_t 
   const int64_t n = B * C * H * W;
   if (n == 0) return CTD_OK;
   CTD_REQUIRE(in && out, "census_transform: null pointer");
-  CTD_REQUIRE(disjoint(in, n * sizeof(T), out, n * sizeof(uint64_t)), "census_transform: out overlaps in");
+  CTD_REQUIRE(ranges_disjoint(in, n * sizeof(T), out, n * sizeof(uint64_t)), "census_transform: out overlaps in");
   return transform_launch<T>(in, out, B * C, (int)H, (int)W, wh, ww, st);
 }
 
@@ -312,9 +292,9 @@ static int census_match_impl(bool is_vol, const T* in0, const T* in1, T* vol, T*
   const void* outs[3] = {vol, disp, score};
   const size_t nout[3] = {nvol, nmap, nmap};
   for (int i = 0; i < 3; ++i)
-    CTD_REQUIRE(!outs[i] || (disjoint(outs[i], nout[i], in0, nin) && disjoint(outs[i], nout[i], in1, nin)),
+    CTD_REQUIRE(ranges_disjoint(outs[i], nout[i], in0, nin) && ranges_disjoint(outs[i], nout[i], in1, nin),
                 "%s: an output overlaps an input", op);
-  CTD_REQUIRE(!score || disjoint(disp, nmap, score, nmap), "%s: disp overlaps score", op);
+  CTD_REQUIRE(ranges_disjoint(disp, nmap, score, nmap), "%s: disp overlaps score", op);
   const size_t words = (size_t)(npix * C);
   uint64_t* t = words ? static_cast<uint64_t*>(scratch_alloc(2 * words * sizeof(uint64_t), st)) : nullptr;
   CTD_REQUIRE(!words || t, "%s: no scratch memory for the descriptors (%zu bytes)", op, 2 * words * sizeof(uint64_t));

@@ -1,6 +1,9 @@
-// Shared helpers of libctd_b200: status/error plumbing, launch accounting, small device utilities.
+// Shared helpers of libctd_b200: status/error plumbing, launch accounting, small device utilities, and the winner-take-all
+// rule of the stereo-matching ops (WtaRun, wta_store).
 #pragma once
 #include <cuda_runtime.h>
+#include <limits.h>
+#include <math_constants.h>
 #include <stdint.h>
 #include <stdio.h>
 
@@ -145,12 +148,73 @@ __device__ __forceinline__ void finish_masked_sums(double num, double den, doubl
 
 __device__ __forceinline__ bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
+// [a, a + na) and [b, b + nb) (bytes) share no byte; a null pointer or an empty range overlaps nothing
+inline bool ranges_disjoint(const void* a, size_t na, const void* b, size_t nb) {
+  const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
+  return !a || !b || na == 0 || nb == 0 || x + na <= y || y + nb <= x;
+}
+
+// A kernel launched with more than 48 KB of dynamic shared memory has to opt in.  The attribute belongs to the device,
+// so it is set on every call (a process may use several GPUs).
+template <typename Kernel>
+int raise_smem_limit(Kernel kernel, size_t bytes, const char* op) {
+  if (bytes > 48 * 1024 && cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) != cudaSuccess)
+    return fail(CTD_ERR_CUDA, "%s: cannot raise the shared-memory limit to %zu bytes", op, bytes);
+  return CTD_OK;
+}
+
+// the value below every other: -inf for floating point, INT_MIN for int
+template <typename T>
+__device__ __forceinline__ T lowest();
+template <>
+__device__ __forceinline__ float lowest<float>() { return -CUDART_INF_F; }
+template <>
+__device__ __forceinline__ double lowest<double>() { return -CUDART_INF; }
+template <>
+__device__ __forceinline__ int lowest<int>() { return INT_MIN; }
+
+// Winner-take-all over scores fed in order d = 0, 1, ...: best = the largest score, bd = the first d that reached it
+// (d*), cm and cp = the scores at d* - 1 and d* + 1 (cp is caught on the step after d* while d* stands).  The lowest()
+// sentinels make d = 0 an ordinary step: any score beats them, and a column of lowest() keeps d* = 0.  Selects only.
+template <typename V>
+struct WtaRun {
+  V best, prev, cm, cp;
+  int bd;
+  __device__ __forceinline__ void init() {
+    best = prev = lowest<V>();
+    cm = cp = 0;
+    bd = 0;
+  }
+  // returns whether v is a new best (bd and best are then d and v; read bd before the call for the old d*)
+  __device__ __forceinline__ bool step(V v, int d) {
+    cp = d - 1 == bd ? v : cp;
+    const bool nb = v > best;
+    cm = nb ? prev : cm;
+    bd = nb ? d : bd;
+    best = nb ? v : best;
+    prev = v;
+    return nb;
+  }
+};
+
 // three-point parabola through the scores at d* - 1, d*, d* + 1: vertex offset in [-0.5, 0.5], 0 unless the peak is strict
 // (den < 0); fp64 with disparity_from_volume's operation order
 __device__ __forceinline__ double wta_subpixel(double cm, double c0, double cp) {
   const double den = cm - 2.0 * c0 + cp;
   if (!(den < 0.0)) return 0.0;
   return fmin(fmax((cm - cp) / (2.0 * den), -0.5), 0.5);
+}
+
+// The winner-take-all outputs of pixel px (either pointer may be null): score = c0, the score at d* = bd, and disp = d*
+// plus, with subpixel, the parabola's offset through cm, c0, cp where 0 < d* < lim - 1 (lim: the number of disparities
+// the pixel has).
+template <typename T>
+__device__ __forceinline__ void wta_store(T* disp, T* score, int64_t px, int bd, T c0, T cm, T cp, int lim, int subpixel) {
+  if (score) score[px] = c0;
+  if (disp) {
+    const double delta = subpixel && bd > 0 && bd < lim - 1 ? wta_subpixel((double)cm, (double)c0, (double)cp) : 0.0;
+    disp[px] = (T)((double)bd + delta);
+  }
 }
 
 }  // namespace ctd

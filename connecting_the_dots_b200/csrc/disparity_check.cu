@@ -11,17 +11,14 @@
 // pixel w and as a right pixel x at once.  The rows V[d,h,w0 .. w0+seg) of DC_DS = 4 consecutive d (and, for a chunk that
 // is not the last, the columns [w0+seg, w0+seg+d) the right pixels reach past it) fill one slot of a 4-slot shared ring
 // through coalesced cp.async copies (16 bytes where aligned), three slots ahead; one barrier per slot.  For each d the
-// thread then updates, with selects only,
-//   left:  best, first index, V at d*-1, V at d*+1 (caught on the step after a new best), the prefix maximum of V lagged
-//          by two steps (the uniqueness maximum below d*-1, taken at each new best) and the maximum over d >= d*+2
-//          (reset at each new best);
-//   right: best, first index, VR at d*-1 and at d*+1, from buf[x + d].
+// thread then steps two winner-take-all runs (WtaRun, ctd_common.cuh), the left one over buf[w] and the right one over
+// buf[x + d], and, for the left pixel, the uniqueness maxima: the prefix maximum of V lagged by two steps (the maximum
+// below d*-1, taken at each new best) and the maximum over d >= d*+2 (reset at each new best).
 // After the chunk's last d the right pixels store dR* in a per-CTA row of pool scratch; after one barrier each left pixel
 // reads dR*(w - d*L), which lies in this chunk or an earlier one of the same row.  Every element of V is read from global
 // memory once (twice for columns a wide row's right pixels reach across a chunk boundary).  No atomics, no host
 // synchronisation, scratch from the library's stream-ordered pool: every call is capture-safe.
 #include <cuda_pipeline.h>
-#include <math_constants.h>
 
 #include <algorithm>
 #include <cmath>
@@ -36,13 +33,6 @@ constexpr int DC_PPT = 4;       // pixels per thread
 constexpr int DC_MAXT = 256;    // threads per CTA at most: a chunk is at most 1024 columns
 constexpr int DC_DS = 4;        // disparities staged per ring slot (one barrier per DC_DS rows of V)
 constexpr int DC_STAGES = 4;    // ring slots; the copies of DC_STAGES - 1 groups are in flight
-
-template <typename T>
-__device__ __forceinline__ T dc_ninf();
-template <>
-__device__ __forceinline__ float dc_ninf<float>() { return -CUDART_INF_F; }
-template <>
-__device__ __forceinline__ double dc_ninf<double>() { return -CUDART_INF; }
 
 // columns [0, n) of a row starting at src into dst (16-byte aligned): 16-byte copies when src is aligned, then the tail
 template <typename T>
@@ -81,7 +71,7 @@ disparity_check_kernel(const T* __restrict__ vol, T* __restrict__ disp, T* __res
                        int stage_elems, int max_diff, double uniqueness, int subpixel) {
   extern __shared__ __align__(16) unsigned char dc_smem[];
   T* ring = reinterpret_cast<T*>(dc_smem);
-  const T ninf = dc_ninf<T>();
+  const T ninf = lowest<T>();
   const int seg = DC_PPT * blockDim.x, nch = (W + seg - 1) / seg, ngroups = (D + DC_DS - 1) / DC_DS;
   const int64_t nrows = B * H, plane = (int64_t)H * W;
   const bool lr_check = valid && max_diff >= 0;
@@ -113,10 +103,9 @@ disparity_check_kernel(const T* __restrict__ vol, T* __restrict__ disp, T* __res
     fslot = fslot + 1 == DC_STAGES ? 0 : fslot + 1;
   }
 
-  // left state of the thread's pixels (see the file comment), then right state
-  T lb[DC_PPT], lsm[DC_PPT], lsp[DC_PPT], lprev[DC_PPT], lpm[DC_PPT], lsec[DC_PPT], lfar[DC_PPT];
-  T rb[DC_PPT], rsm[DC_PPT], rsp[DC_PPT], rprev[DC_PPT];
-  int lbd[DC_PPT], rbd[DC_PPT];
+  // the runs of the thread's left and right pixels and the left pixels' uniqueness maxima (see the file comment)
+  WtaRun<T> L[DC_PPT], R[DC_PPT];
+  T lpm[DC_PPT], lsec[DC_PPT], lfar[DC_PPT];
   while (c.row < nrows) {
     __pipeline_wait_prior(DC_STAGES - 2);
     __syncthreads();  // group c's rows are in; every thread is done with the slot the next fetch overwrites
@@ -129,12 +118,11 @@ disparity_check_kernel(const T* __restrict__ vol, T* __restrict__ disp, T* __res
     cslot = cslot + 1 == DC_STAGES ? 0 : cslot + 1;
     const int w0 = c.ch * seg, aend = min(W, w0 + seg);
     if (c.g == 0) {
-      // the sentinels make d = 0 an ordinary step: -inf is beaten by any value, and a column of -inf keeps d* = 0
 #pragma unroll
       for (int k = 0; k < DC_PPT; ++k) {
-        lb[k] = lprev[k] = lpm[k] = lsec[k] = lfar[k] = rb[k] = rprev[k] = ninf;
-        lsm[k] = lsp[k] = rsm[k] = rsp[k] = 0;
-        lbd[k] = rbd[k] = 0;
+        L[k].init();
+        R[k].init();
+        lpm[k] = lsec[k] = lfar[k] = ninf;
       }
     }
 #pragma unroll
@@ -147,27 +135,16 @@ disparity_check_kernel(const T* __restrict__ vol, T* __restrict__ disp, T* __res
       for (int k = 0; k < DC_PPT; ++k) {
         const int p = threadIdx.x + k * blockDim.x, w = w0 + p;
         if (w < aend) {
-          // d == d* + 1 catches V at d* + 1; d >= d* + 2 feeds the uniqueness maximum above d*; both use the old d*
+          // d >= d* + 2 feeds the uniqueness maximum above d*, with the d* and the V at d - 1 of before the step
           const T v = buf[p];
-          const bool nb = v > lb[k];
-          lsp[k] = d - 1 == lbd[k] ? v : lsp[k];
-          lfar[k] = nb ? ninf : (d - 2 >= lbd[k] ? fmax(lfar[k], v) : lfar[k]);
+          const int bd = L[k].bd;
+          const T vm = L[k].prev;
+          const bool nb = L[k].step(v, d);
+          lfar[k] = nb ? ninf : (d - 2 >= bd ? fmax(lfar[k], v) : lfar[k]);
           lsec[k] = nb ? lpm[k] : lsec[k];
-          lsm[k] = nb ? lprev[k] : lsm[k];
-          lbd[k] = nb ? d : lbd[k];
-          lb[k] = nb ? v : lb[k];
-          lpm[k] = fmax(lpm[k], lprev[k]);
-          lprev[k] = v;
+          lpm[k] = fmax(lpm[k], vm);
           const int col = w + d;  // right pixel x = w reads VR[d] = V[d, x + d]
-          if (col < W) {
-            const T r = buf[col >= aend ? p + d - bshift : p + d];
-            const bool rn = r > rb[k];
-            rsp[k] = d - 1 == rbd[k] ? r : rsp[k];
-            rsm[k] = rn ? rprev[k] : rsm[k];
-            rbd[k] = rn ? d : rbd[k];
-            rb[k] = rn ? r : rb[k];
-            rprev[k] = r;
-          }
+          if (col < W) R[k].step(buf[col >= aend ? p + d - bshift : p + d], d);
         }
       }
     }
@@ -178,34 +155,22 @@ disparity_check_kernel(const T* __restrict__ vol, T* __restrict__ disp, T* __res
       for (int k = 0; k < DC_PPT; ++k) {
         const int x = w0 + threadIdx.x + k * blockDim.x;
         if (x >= aend) break;
-        if (lr_check) dr[x] = rbd[k];
-        if (score_r) score_r[base + x] = rb[k];
-        if (disp_r) {
-          const int dx = min(D, W - x);
-          const double delta = subpixel && rbd[k] > 0 && rbd[k] < dx - 1
-                                   ? wta_subpixel((double)rsm[k], (double)rb[k], (double)rsp[k])
-                                   : 0.0;
-          disp_r[base + x] = (T)((double)rbd[k] + delta);
-        }
+        if (lr_check) dr[x] = R[k].bd;
+        wta_store<T>(disp_r, score_r, base + x, R[k].bd, R[k].best, R[k].cm, R[k].cp, min(D, W - x), subpixel);
       }
       if (lr_check) __syncthreads();  // dR* of every x < aend of this row is in dr
 #pragma unroll
       for (int k = 0; k < DC_PPT; ++k) {
         const int w = w0 + threadIdx.x + k * blockDim.x;
         if (w >= aend) break;
-        if (score) score[base + w] = lb[k];
-        if (disp) {
-          const double delta = subpixel && lbd[k] > 0 && lbd[k] < D - 1
-                                   ? wta_subpixel((double)lsm[k], (double)lb[k], (double)lsp[k])
-                                   : 0.0;
-          disp[base + w] = (T)((double)lbd[k] + delta);
-        }
+        const int bd = L[k].bd;
+        wta_store<T>(disp, score, base + w, bd, L[k].best, L[k].cm, L[k].cp, D, subpixel);
         if (valid) {
-          const int x = w - lbd[k];
-          const bool lr = max_diff < 0 || (x >= 0 && abs(lbd[k] - dr[x]) <= max_diff);
-          const bool far_empty = lbd[k] < 2 && lbd[k] + 2 > D - 1;
+          const int x = w - bd;
+          const bool lr = max_diff < 0 || (x >= 0 && abs(bd - dr[x]) <= max_diff);
+          const bool far_empty = bd < 2 && bd + 2 > D - 1;
           const bool uq = uniqueness == 0.0 || far_empty ||
-                          (double)lb[k] - (double)fmax(lsec[k], lfar[k]) >= uniqueness;
+                          (double)L[k].best - (double)fmax(lsec[k], lfar[k]) >= uniqueness;
           valid[base + w] = lr && uq;
         }
       }
@@ -213,11 +178,6 @@ disparity_check_kernel(const T* __restrict__ vol, T* __restrict__ disp, T* __res
     c.next(ngroups, nch, D, H, W);
   }
   __pipeline_wait_prior(0);
-}
-
-bool dc_disjoint(const void* a, size_t na, const void* b, size_t nb) {
-  const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
-  return !a || !b || na == 0 || nb == 0 || x + na <= y || y + nb <= x;
 }
 
 }  // namespace
@@ -238,8 +198,8 @@ static int disparity_check_impl(const T* vol, T* disp, T* score, T* disp_r, T* s
   const void* outs[5] = {disp, score, disp_r, score_r, valid};
   const size_t nout[5] = {nmap, nmap, nmap, nmap, (size_t)npix};
   for (int i = 0; i < 5; ++i) {
-    CTD_REQUIRE(dc_disjoint(outs[i], nout[i], vol, nvol), "%s: an output overlaps vol", op);
-    for (int j = 0; j < i; ++j) CTD_REQUIRE(dc_disjoint(outs[i], nout[i], outs[j], nout[j]), "%s: two outputs overlap", op);
+    CTD_REQUIRE(ranges_disjoint(outs[i], nout[i], vol, nvol), "%s: an output overlaps vol", op);
+    for (int j = 0; j < i; ++j) CTD_REQUIRE(ranges_disjoint(outs[i], nout[i], outs[j], nout[j]), "%s: two outputs overlap", op);
   }
   if (!disp && !score && !disp_r && !score_r && !valid) return CTD_OK;
 
@@ -249,9 +209,8 @@ static int disparity_check_impl(const T* vol, T* disp, T* score, T* disp_r, T* s
   const int stage_elems = (W > seg ? 2 : 1) * seg;
   const size_t smem = (size_t)DC_STAGES * DC_DS * stage_elems * sizeof(T);
   auto kernel = disparity_check_kernel<T>;
-  // the attribute belongs to the device: set on every call (a process may use several GPUs)
-  if (smem > 48 * 1024 && cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-    return fail(CTD_ERR_CUDA, "%s: cannot raise the shared-memory limit to %zu bytes", op, smem);
+  const int rs = raise_smem_limit(kernel, smem, op);
+  if (rs != CTD_OK) return rs;
   int dev = 0, sms = 0, per_sm = 0;
   CTD_CUDA(cudaGetDevice(&dev));
   CTD_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));

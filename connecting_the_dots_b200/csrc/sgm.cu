@@ -18,11 +18,11 @@
 //   * sgm_lines: one vertical or diagonal path.  Lines are sheared columns k = w - dx*dy*h: a diagonal line's predecessor
 //     lies on the same line, so a line needs no data from its neighbours, and the 32/G lines of a warp read adjacent w.
 //     Each step loads the next row's V and A before it computes the current one.  The last pass in path order also takes
-//     the winner-take-all disparity and score of A (with disparity_from_volume's fp64 sub-pixel arithmetic).
+//     the winner-take-all disparity and score of A: the first maximum by a reduction over the group, stored through
+//     wta_store (ctd_common.cuh) with disparity_from_volume's fp64 sub-pixel offset.
 // No atomics, no scratch memory, no host synchronisation: every call is capture-safe and its result does not depend on
 // the launch configuration (every value is computed by the same operations in the same order whatever G, K or WT are).
 #include <cuda_pipeline.h>
-#include <math_constants.h>
 
 #include <algorithm>
 #include <cmath>
@@ -39,18 +39,11 @@ constexpr int SGM_HWARPS = 4;        // rows (warps) per sgm_horizontal CTA
 constexpr int SGM_SLAB_BYTES = 16384;  // shared slabs per warp (two tiles)
 constexpr int SGM_LTHREADS = 256;
 
-template <typename T>
-__device__ __forceinline__ T neg_inf();
-template <>
-__device__ __forceinline__ float neg_inf<float>() { return -CUDART_INF_F; }
-template <>
-__device__ __forceinline__ double neg_inf<double>() { return -CUDART_INF; }
-
 // One step of the recurrence for the line held by a group of G lanes (this lane is g).  L holds L_r(q, .) and M its maximum
 // on entry, L_r(p, .) and its maximum on exit; start: q is outside the image.  Every lane of the warp calls it.
 template <typename T, int K>
 __device__ __forceinline__ void sgm_step(T (&L)[K], const T (&v)[K], T& M, bool start, int g, int G, T p1, T p2) {
-  const T ninf = neg_inf<T>();
+  const T ninf = lowest<T>();
   const T lo = __shfl_up_sync(FULL, L[K - 1], 1, G);  // L(q, g*K - 1)
   const T hi = __shfl_down_sync(FULL, L[0], 1, G);    // L(q, g*K + K)
   const T mp2 = M - p2;
@@ -81,7 +74,7 @@ sgm_horizontal(const T* __restrict__ vol, T* __restrict__ agg, int64_t B, int D,
   extern __shared__ __align__(16) unsigned char sgm_smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   T* slabs = reinterpret_cast<T*>(sgm_smem) + (size_t)warp * 2 * D * WT;
-  const T ninf = neg_inf<T>();
+  const T ninf = lowest<T>();
   const int64_t plane = (int64_t)H * W, nrows = B * H;
   const int ntiles = (W + WT - 1) / WT, wshift = __ffs(WT) - 1;
   for (int64_t row = (int64_t)blockIdx.x * SGM_HWARPS + warp; row < nrows; row += (int64_t)gridDim.x * SGM_HWARPS) {
@@ -147,7 +140,7 @@ template <typename T, int K, bool WTA>
 __global__ void __launch_bounds__(SGM_LTHREADS)
 sgm_lines(const T* __restrict__ vol, T* __restrict__ agg, T* __restrict__ disp, T* __restrict__ score, int64_t B, int D,
           int H, int W, int dy, int dx, int G, T p1, T p2, int subpixel) {
-  const T ninf = neg_inf<T>();
+  const T ninf = lowest<T>();
   const int s = dx * dy;  // pixel (h, w) lies on line k = w - s*h
   const int64_t plane = (int64_t)H * W;
   const int64_t nk = W + (s != 0 ? (int64_t)H - 1 : 0), kmin = s > 0 ? -(int64_t)(H - 1) : 0;
@@ -222,14 +215,7 @@ sgm_lines(const T* __restrict__ vol, T* __restrict__ agg, T* __restrict__ disp, 
         }
         cm = __shfl_sync(FULL, cm, max(bd - 1, 0) / K, G);
         cp = __shfl_sync(FULL, cp, min(bd + 1, D - 1) / K, G);
-        if (in && g == 0) {
-          const int64_t px = b * plane + o;
-          if (score) score[px] = best;
-          if (disp) {
-            const double delta = subpixel && bd > 0 && bd < D - 1 ? wta_subpixel((double)cm, (double)best, (double)cp) : 0.0;
-            disp[px] = (T)((double)bd + delta);
-          }
-        }
+        if (in && g == 0) wta_store<T>(disp, score, b * plane + o, bd, best, cm, cp, D, subpixel);
       }
 #pragma unroll
       for (int j = 0; j < K; ++j) v[j] = vn[j], a[j] = an[j];
@@ -249,9 +235,8 @@ int horizontal_launch(const T* vol, T* agg, int64_t B, int D, int H, int W, T p1
   while (WT > 1 && (size_t)2 * D * WT * sizeof(T) > SGM_SLAB_BYTES) WT >>= 1;
   const size_t smem = (size_t)SGM_HWARPS * 2 * D * WT * sizeof(T);
   auto kernel = sgm_horizontal<T, K>;
-  // the attribute belongs to the device: set on every call (a process may use several GPUs)
-  if (smem > 48 * 1024 && cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-    return fail(CTD_ERR_CUDA, "sgm: cannot raise the shared-memory limit to %zu bytes", smem);
+  const int rs = raise_smem_limit(kernel, smem, "sgm");
+  if (rs != CTD_OK) return rs;
   const int64_t grid = std::min<int64_t>(cdiv(B * H, SGM_HWARPS), INT32_MAX);
   kernel<<<(unsigned)grid, 32 * SGM_HWARPS, smem, st>>>(vol, agg, B, D, H, W, WT, p1, p2);
   count_launch();
@@ -294,8 +279,8 @@ static int sgm_impl(const T* vol, T* agg, T* disp, T* score, int64_t B, int64_t 
   CTD_REQUIRE(D >= 1, "sgm: the volume has no disparities (D = 0)");
   CTD_REQUIRE(D <= SGM_MAX_D, "sgm: at most %d disparities, got %lld", SGM_MAX_D, (long long)D);
   CTD_REQUIRE(vol && agg, "sgm: null pointer");
-  const uintptr_t v0 = (uintptr_t)vol, a0 = (uintptr_t)agg, n = (uintptr_t)(B * D * H * W) * sizeof(T);
-  CTD_REQUIRE(a0 + n <= v0 || v0 + n <= a0, "sgm: agg overlaps vol");
+  const size_t n = (size_t)(B * D * H * W) * sizeof(T);
+  CTD_REQUIRE(ranges_disjoint(agg, n, vol, n), "sgm: agg overlaps vol");
   const int d = (int)D, h = (int)H, w = (int)W;
   // horizontal: a warp per row
   const int kh = pow2_at_least(cdiv(D, 32));

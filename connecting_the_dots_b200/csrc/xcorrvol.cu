@@ -88,8 +88,8 @@ __device__ __forceinline__ float wta_score(unsigned long long key) {
 __device__ __forceinline__ int wta_disp(unsigned long long key, int D) {  // clamped: a key of 0 (no candidate) is never read out of range
   return (int)min(0xFFFFFFFFu - (unsigned)key, (unsigned)(D - 1));
 }
-// generic disparity: one thread per pixel sweeps d with xcorr_generic_one, so d* and the score are the exact argmax and
-// maximum of xcorrvol_generic's volume
+// generic disparity: one thread per pixel sweeps d with xcorr_generic_one through a WtaRun, so d* and the score are the
+// exact argmax and maximum of xcorrvol_generic's volume
 template <typename T>
 __global__ void __launch_bounds__(256)
 xcorr_disparity_generic(const T* __restrict__ in0, const T* __restrict__ in1, T* __restrict__ disp, T* __restrict__ score,
@@ -99,22 +99,13 @@ xcorr_disparity_generic(const T* __restrict__ in0, const T* __restrict__ in1, T*
        idx += (int64_t)gridDim.x * blockDim.x) {
     const int w = idx % W, h = (idx / W) % H;
     const int64_t b = idx / ((int64_t)W * H);
-    T best = 0, prev = 0, cm = 0, cp = 0;  // cm, cp: V at best - 1 and best + 1
-    int bd = 0;
-    for (int d = 0; d < D; ++d) {
-      const T v = xcorr_generic_one<T>(in0, in1, b, C, H, W, h, w, d, bs);
-      if (d == 0 || v > best) {
-        best = v;
-        bd = d;
-        cm = prev;
-      } else if (d == bd + 1) {
-        cp = v;
-      }
-      prev = v;
-    }
-    if (score) score[idx] = best;
-    const double delta = subpixel && bd > 0 && bd < D - 1 ? wta_subpixel((double)cm, (double)best, (double)cp) : 0.0;
-    disp[idx] = (T)((double)bd + delta);
+    WtaRun<T> run;
+    run.init();
+    for (int d = 0; d < D; ++d) run.step(xcorr_generic_one<T>(in0, in1, b, C, H, W, h, w, d, bs), d);
+    // disp is never null here (xcorr_disparity_impl requires it); without the hint the fp32 build reloads two more
+    // spilled words per pixel
+    __builtin_assume(disp != nullptr);
+    wta_store<T>(disp, score, idx, run.bd, run.best, run.cm, run.cp, D, subpixel);
   }
 }
 

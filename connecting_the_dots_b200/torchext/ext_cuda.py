@@ -43,6 +43,24 @@ def _stream(t):
     return torch.cuda.current_stream(t.device).cuda_stream
 
 
+def _image_pair(in0, in1, op):
+    """Checks of an image pair [C,H,W] or [B,C,H,W]: (dtype suffix, B, C, H, W, batched)."""
+    _check_input_cuda(in0, "in0")
+    _check_input_cuda(in1, "in1")
+    _check(in0.dim() in (3, 4), "in0 has to be C x H x W (or B x C x H x W)")
+    _check(tuple(in0.shape) == tuple(in1.shape), "in0 and in1 have to be the same shape")
+    _same(in0, in1, "in0", "in1")
+    sfx = _real_suffix(in0, op)
+    batched = in0.dim() == 4
+    C, H, W = in0.shape[-3:]
+    return sfx, in0.size(0) if batched else 1, C, H, W, batched
+
+
+def _maps(ref, B, H, W, batched, dtype=None):
+    """One per-pixel output map on ref's device, [B,1,H,W] (or [1,H,W]), in ref's dtype unless one is given."""
+    return torch.empty((B, 1, H, W) if batched else (1, H, W), dtype=dtype or ref.dtype, device=ref.device)
+
+
 def nn_cuda(in0, in1):
     """ext_cuda.cpp:9-26.  in0 [N0,3], in1 [N1,3] -> int64 [N0] nearest-neighbour indices (or -1)."""
     _check_input_cuda(in0, "in0")
@@ -95,15 +113,7 @@ def proj_nn_cuda(xyz0, xyz1, K, patch_size):
 
 def xcorrvol_cuda(in0, in1, n_disps, block_size):
     """ext_cuda.cpp:73-86.  in0, in1 [C,H,W] -> [n_disps,H,W]; batched: [B,C,H,W] -> [B,n_disps,H,W]."""
-    _check_input_cuda(in0, "in0")
-    _check_input_cuda(in1, "in1")
-    _check(in0.dim() in (3, 4), "in0 has to be C x H x W (or B x C x H x W)")
-    _check(tuple(in0.shape) == tuple(in1.shape), "in0 and in1 have to be the same shape")
-    _same(in0, in1, "in0", "in1")
-    sfx = _real_suffix(in0, "xcorrvol")
-    batched = in0.dim() == 4
-    B = in0.size(0) if batched else 1
-    C, H, W = in0.shape[-3:]
+    sfx, B, C, H, W, batched = _image_pair(in0, in1, "xcorrvol")
     out = torch.empty((B, int(n_disps), H, W) if batched else (int(n_disps), H, W), dtype=in0.dtype, device=in0.device)
     with torch.cuda.device(in0.device):
         _lib.call("ctd_xcorrvol" + sfx, in0.data_ptr(), in1.data_ptr(), out.data_ptr(), B, C, H, W, int(n_disps),
@@ -114,18 +124,8 @@ def xcorrvol_cuda(in0, in1, n_disps, block_size):
 def xcorr_disparity_cuda(in0, in1, n_disps, block_size, subpixel=True):
     """Winner-take-all disparity of xcorrvol_cuda's volume without writing it (ctd_xcorr_disparity_*).  in0, in1 [C,H,W]
     -> (disp, score) [1,H,W]; batched: [B,C,H,W] -> [B,1,H,W]."""
-    _check_input_cuda(in0, "in0")
-    _check_input_cuda(in1, "in1")
-    _check(in0.dim() in (3, 4), "in0 has to be C x H x W (or B x C x H x W)")
-    _check(tuple(in0.shape) == tuple(in1.shape), "in0 and in1 have to be the same shape")
-    _same(in0, in1, "in0", "in1")
-    sfx = _real_suffix(in0, "xcorr_disparity")
-    batched = in0.dim() == 4
-    B = in0.size(0) if batched else 1
-    C, H, W = in0.shape[-3:]
-    shape = (B, 1, H, W) if batched else (1, H, W)
-    disp = torch.empty(shape, dtype=in0.dtype, device=in0.device)
-    score = torch.empty(shape, dtype=in0.dtype, device=in0.device)
+    sfx, B, C, H, W, batched = _image_pair(in0, in1, "xcorr_disparity")
+    disp, score = _maps(in0, B, H, W, batched), _maps(in0, B, H, W, batched)
     with torch.cuda.device(in0.device):
         _lib.call("ctd_xcorr_disparity" + sfx, in0.data_ptr(), in1.data_ptr(), disp.data_ptr(), score.data_ptr(), B, C, H, W,
                   int(n_disps), int(block_size), int(bool(subpixel)), _stream(in0))
@@ -144,9 +144,7 @@ def sgm_cuda(vol, p1, p2, paths=8, subpixel=True, want_disparity=True):
     agg = torch.empty_like(vol)
     disp = score = None
     if want_disparity:
-        shape = (B, 1, H, W) if batched else (1, H, W)
-        disp = torch.empty(shape, dtype=vol.dtype, device=vol.device)
-        score = torch.empty(shape, dtype=vol.dtype, device=vol.device)
+        disp, score = _maps(vol, B, H, W, batched), _maps(vol, B, H, W, batched)
     with torch.cuda.device(vol.device):
         _lib.call("ctd_sgm" + sfx, vol.data_ptr(), agg.data_ptr(), disp.data_ptr() if want_disparity else None,
                   score.data_ptr() if want_disparity else None, B, D, H, W, float(p1), float(p2), int(paths),
@@ -163,10 +161,7 @@ def disparity_check_cuda(vol, max_diff=1, uniqueness=0.0, subpixel=True):
     batched = vol.dim() == 4
     B = vol.size(0) if batched else 1
     D, H, W = vol.shape[-3:]
-    shape = (B, 1, H, W) if batched else (1, H, W)
-    disp = torch.empty(shape, dtype=vol.dtype, device=vol.device)
-    score = torch.empty(shape, dtype=vol.dtype, device=vol.device)
-    valid = torch.empty(shape, dtype=torch.bool, device=vol.device)
+    disp, score, valid = _maps(vol, B, H, W, batched), _maps(vol, B, H, W, batched), _maps(vol, B, H, W, batched, torch.bool)
     with torch.cuda.device(vol.device):
         _lib.call("ctd_disparity_check" + sfx, vol.data_ptr(), disp.data_ptr(), score.data_ptr(), None, None, valid.data_ptr(),
                   B, D, H, W, int(max_diff), float(uniqueness), int(bool(subpixel)), _stream(vol))
@@ -186,23 +181,11 @@ def census_transform_cuda(x, wh, ww):
     return out
 
 
-def _census_pair(in0, in1, op):
-    _check_input_cuda(in0, "in0")
-    _check_input_cuda(in1, "in1")
-    _check(in0.dim() in (3, 4), "in0 has to be C x H x W (or B x C x H x W)")
-    _check(tuple(in0.shape) == tuple(in1.shape), "in0 and in1 have to be the same shape")
-    _same(in0, in1, "in0", "in1")
-    sfx = _real_suffix(in0, op)
-    B = in0.size(0) if in0.dim() == 4 else 1
-    return sfx, (B,) + tuple(in0.shape[-3:])
-
-
 def census_vol_cuda(in0, in1, n_disps, wh, ww, block_size):
     """Census matching-score volume (ctd_census_vol_*): in0, in1 [B,C,H,W] -> [B,n_disps,H,W] (or [C,H,W] ->
     [n_disps,H,W]), in the inputs' dtype."""
-    sfx, (B, C, H, W) = _census_pair(in0, in1, "census_vol")
-    shape = (B, int(n_disps), H, W) if in0.dim() == 4 else (int(n_disps), H, W)
-    out = torch.empty(shape, dtype=in0.dtype, device=in0.device)
+    sfx, B, C, H, W, batched = _image_pair(in0, in1, "census_vol")
+    out = torch.empty((B, int(n_disps), H, W) if batched else (int(n_disps), H, W), dtype=in0.dtype, device=in0.device)
     with torch.cuda.device(in0.device):
         _lib.call("ctd_census_vol" + sfx, in0.data_ptr(), in1.data_ptr(), out.data_ptr(), B, C, H, W, int(n_disps), int(wh),
                   int(ww), int(block_size), _stream(in0))
@@ -212,10 +195,8 @@ def census_vol_cuda(in0, in1, n_disps, wh, ww, block_size):
 def census_disparity_cuda(in0, in1, n_disps, wh, ww, block_size, subpixel=True):
     """Winner-take-all disparity of census_vol_cuda's volume without writing it (ctd_census_disparity_*): (disp, score),
     [B,1,H,W] (or [1,H,W])."""
-    sfx, (B, C, H, W) = _census_pair(in0, in1, "census_disparity")
-    shape = (B, 1, H, W) if in0.dim() == 4 else (1, H, W)
-    disp = torch.empty(shape, dtype=in0.dtype, device=in0.device)
-    score = torch.empty(shape, dtype=in0.dtype, device=in0.device)
+    sfx, B, C, H, W, batched = _image_pair(in0, in1, "census_disparity")
+    disp, score = _maps(in0, B, H, W, batched), _maps(in0, B, H, W, batched)
     with torch.cuda.device(in0.device):
         _lib.call("ctd_census_disparity" + sfx, in0.data_ptr(), in1.data_ptr(), disp.data_ptr(), score.data_ptr(), B, C, H, W,
                   int(n_disps), int(wh), int(ww), int(block_size), int(bool(subpixel)), _stream(in0))

@@ -17,6 +17,11 @@ def _native(t, cuda_name, cpu_name):
     return getattr(ext_cuda, cuda_name) if t.is_cuda else getattr(ext_cpu, cpu_name)
 
 
+def _cuda_only(t, op):
+    if not t.is_cuda:
+        raise RuntimeError("torchext.%s: connecting_the_dots_b200 has no CPU implementation" % op)
+
+
 class NNFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, in0, in1):
@@ -83,9 +88,21 @@ def xcorr_disparity(in0, in1, n_disps, block_size, subpixel=True):
     the largest score (winner-take-all), score the peak correlation there; with subpixel, disp = d* + the vertex offset of
     the parabola through the scores at d* - 1, d*, d* + 1 (disparity_from_volume states it).  d* and score equal
     disparity_from_volume(xcorrvol(in0, in1, n_disps, block_size)) exactly.  CUDA tensors only, float32 or float64."""
-    if not in0.is_cuda:
-        raise RuntimeError("torchext.xcorr_disparity: connecting_the_dots_b200 has no CPU implementation")
+    _cuda_only(in0, "xcorr_disparity")
     return ext_cuda.xcorr_disparity_cuda(in0, in1, n_disps, block_size, subpixel)
+
+
+def _subpixel(src, d, lim):
+    """The sub-pixel offset of the winner-take-all disparity d [B,1,H,W] of src [B,D,H,W], in float64: with c-, c0, c+ =
+    src at d - 1, d, d + 1 and den = c- - 2 c0 + c+, clamp((c- - c+) / (2 den), -0.5, 0.5), and 0 where d = 0,
+    d >= lim - 1 (lim: the disparities the pixel has) or den >= 0."""
+    D = src.size(1)
+    cm = src.gather(1, (d - 1).clamp(min=0)).double()
+    c0 = src.gather(1, d).double()
+    cp = src.gather(1, (d + 1).clamp(max=D - 1)).double()
+    den = cm - 2 * c0 + cp
+    ok = (d > 0) & (d < lim - 1) & (den < 0)
+    return torch.where(ok, (cm - cp) / (2 * torch.where(ok, den, -1.0)), 0.0).clamp(-0.5, 0.5)
 
 
 def disparity_from_volume(vol, subpixel=True):
@@ -104,13 +121,7 @@ def disparity_from_volume(vol, subpixel=True):
     score = v.gather(1, d)
     disp = d.to(torch.float64)
     if subpixel:
-        cm = v.gather(1, (d - 1).clamp(min=0)).double()
-        c0 = score.double()
-        cp = v.gather(1, (d + 1).clamp(max=D - 1)).double()
-        den = cm - 2 * c0 + cp
-        ok = (d > 0) & (d < D - 1) & (den < 0)
-        delta = torch.where(ok, (cm - cp) / (2 * torch.where(ok, den, -1.0)), 0.0).clamp(-0.5, 0.5)
-        disp = disp + delta
+        disp = disp + _subpixel(v, d, D)
     disp = disp.to(vol.dtype)
     if vol.dim() == 3:
         disp, score = disp[0], score[0]
@@ -133,8 +144,7 @@ def disparity_check(vol, max_diff=1, uniqueness=0.0, subpixel=True):
     bit, valid (torch.bool) marks the pixels that pass both checks as disparity_check_pytorch states them.  max_diff < 0
     turns the LR check off, uniqueness = 0 the uniqueness check.  Not differentiable.  CUDA tensors only, float32 or
     float64."""
-    if not vol.is_cuda:
-        raise RuntimeError("torchext.disparity_check: connecting_the_dots_b200 has no CPU implementation")
+    _cuda_only(vol, "disparity_check")
     u = _disparity_check_args("disparity_check", vol, uniqueness)
     return ext_cuda.disparity_check_cuda(vol, int(max_diff), u, subpixel)
 
@@ -159,14 +169,7 @@ def right_disparity_from_volume(vol, subpixel=True):
     score = vr.gather(1, d)
     disp = d.to(torch.float64)
     if subpixel:
-        dx = (W - x).clamp(max=D)
-        cm = vr.gather(1, (d - 1).clamp(min=0)).double()
-        c0 = score.double()
-        cp = vr.gather(1, (d + 1).clamp(max=D - 1)).double()
-        den = cm - 2 * c0 + cp
-        ok = (d > 0) & (d < dx - 1) & (den < 0)
-        delta = torch.where(ok, (cm - cp) / (2 * torch.where(ok, den, -1.0)), 0.0).clamp(-0.5, 0.5)
-        disp = disp + delta
+        disp = disp + _subpixel(vr, d, (W - x).clamp(max=D))
     disp = disp.to(vol.dtype)
     if vol.dim() == 3:
         disp, score = disp[0], score[0]
@@ -205,8 +208,7 @@ def sgm_aggregate(vol, p1, p2, paths=8):
     """Semi-global matching (Hirschmueller, PAMI 2008) over a score volume vol [B,D,H,W] (or [D,H,W]; higher is better, the
     convention of xcorrvol: pass a cost volume negated): the aggregated volume A, same shape and dtype, equal bit for bit to
     sgm_aggregate_pytorch, which states the definition.  Not differentiable.  CUDA tensors only, float32 or float64."""
-    if not vol.is_cuda:
-        raise RuntimeError("torchext.sgm_aggregate: connecting_the_dots_b200 has no CPU implementation")
+    _cuda_only(vol, "sgm_aggregate")
     return ext_cuda.sgm_cuda(vol, p1, p2, paths, want_disparity=False)[0]
 
 
@@ -214,8 +216,7 @@ def sgm_disparity(vol, p1, p2, paths=8, subpixel=True):
     """(disp, score) = disparity_from_volume(sgm_aggregate(vol, p1, p2, paths), subpixel), bit for bit, with the
     winner-take-all fused into the last aggregation pass; A is allocated and dropped.  [B,1,H,W] (or [1,H,W]), not
     differentiable, CUDA tensors only, float32 or float64."""
-    if not vol.is_cuda:
-        raise RuntimeError("torchext.sgm_disparity: connecting_the_dots_b200 has no CPU implementation")
+    _cuda_only(vol, "sgm_disparity")
     _, disp, score = ext_cuda.sgm_cuda(vol, p1, p2, paths, subpixel)
     return disp, score
 
@@ -310,8 +311,7 @@ def census_transform(x, window=(7, 9)):
     """Census transform of each channel of x [B,C,H,W] (or [C,H,W]) over a window (wh, ww): int64 of x's shape holding the
     uint64 bit pattern (bit 63 makes it negative), equal to census_transform_pytorch, which states the definition.  Not
     differentiable.  CUDA tensors only, float32 or float64."""
-    if not x.is_cuda:
-        raise RuntimeError("torchext.census_transform: connecting_the_dots_b200 has no CPU implementation")
+    _cuda_only(x, "census_transform")
     wh, ww, _ = _census_check("census_transform", window)
     return ext_cuda.census_transform_cuda(x, wh, ww)
 
@@ -321,8 +321,7 @@ def census_vol(in0, in1, n_disps, window=(7, 9), block_size=1):
     dtype: minus the block_size^2 box sum of the Hamming distances of the census descriptors.  Higher is better (the
     convention of xcorrvol), so sgm_disparity(census_vol(...), p1, p2) works as it is.  Equal bit for bit to
     census_vol_pytorch, which states the definition.  Not differentiable.  CUDA tensors only, float32 or float64."""
-    if not in0.is_cuda:
-        raise RuntimeError("torchext.census_vol: connecting_the_dots_b200 has no CPU implementation")
+    _cuda_only(in0, "census_vol")
     wh, ww, bs = _census_inputs("census_vol", in0, in1, n_disps, window, block_size)
     return ext_cuda.census_vol_cuda(in0, in1, n_disps, wh, ww, bs)
 
@@ -331,8 +330,7 @@ def census_disparity(in0, in1, n_disps, window=(7, 9), block_size=9, subpixel=Tr
     """(disp, score) = disparity_from_volume(census_vol(in0, in1, n_disps, window, block_size), subpixel), bit for bit
     including the sub-pixel offset, without writing the volume.  [B,1,H,W] (or [1,H,W]), not differentiable, CUDA tensors
     only, float32 or float64."""
-    if not in0.is_cuda:
-        raise RuntimeError("torchext.census_disparity: connecting_the_dots_b200 has no CPU implementation")
+    _cuda_only(in0, "census_disparity")
     wh, ww, bs = _census_inputs("census_disparity", in0, in1, n_disps, window, block_size)
     return ext_cuda.census_disparity_cuda(in0, in1, n_disps, wh, ww, bs, subpixel)
 
@@ -451,8 +449,7 @@ class WeightedPhotometricLossFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, es, ta, mask, block_size, type, eps):
-        if not es.is_cuda:
-            raise RuntimeError("torchext.weighted_photometric_loss: connecting_the_dots_b200 has no CPU implementation")
+        _cuda_only(es, "weighted_photometric_loss")
         mask = mask.detach().contiguous()
         # grad_out = mask: the gradient comes back unnormalised and is divided by sum(mask) in backward
         out, grad_es, sums = ext_cuda.photometric_loss_forward_backward_masked(es.detach(), ta.detach(), mask, mask, block_size, type, eps)
@@ -477,8 +474,7 @@ SSIM_C1, SSIM_C2 = 0.01 ** 2, 0.03 ** 2
 class SSIMLossFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, es, ta, block_size, c1, c2):
-        if not es.is_cuda:
-            raise RuntimeError("torchext.ssim_loss: connecting_the_dots_b200 has no CPU implementation")
+        _cuda_only(es, "ssim_loss")
         es, ta = es.detach(), ta.detach()
         ctx.save_for_backward(es, ta)
         ctx.block_size, ctx.c1, ctx.c2 = block_size, c1, c2
@@ -526,8 +522,7 @@ class WeightedSSIMLossFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, es, ta, mask, block_size, c1, c2):
-        if not es.is_cuda:
-            raise RuntimeError("torchext.weighted_ssim_loss: connecting_the_dots_b200 has no CPU implementation")
+        _cuda_only(es, "weighted_ssim_loss")
         mask = mask.detach().contiguous()
         # grad_out = mask: the gradient comes back unnormalised and is divided by sum(mask) in backward
         out, grad_es, sums = ext_cuda.ssim_forward_backward_masked(es.detach(), ta.detach(), mask, mask, block_size, c1, c2)
@@ -552,8 +547,7 @@ class WarpPatternFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, pattern, disp):
-        if not disp.is_cuda:
-            raise RuntimeError("torchext.warp_pattern: connecting_the_dots_b200 has no CPU implementation")
+        _cuda_only(disp, "warp_pattern")
         pattern, disp = pattern.detach().contiguous(), disp.detach().contiguous()
         ctx.save_for_backward(pattern, disp)
         return ext_cuda.warp_pattern_forward(pattern, disp)
@@ -618,8 +612,7 @@ class ProjectionDepthSimilarityFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, depth0, depth1, R0, t0, R1, t1, K, ray, clamp):
-        if not depth0.is_cuda:
-            raise RuntimeError("torchext.projection_depth_similarity_loss: connecting_the_dots_b200 has no CPU implementation")
+        _cuda_only(depth0, "projection_depth_similarity_loss")
         c = lambda t: t.detach().contiguous()
         sums, g0, g1 = ext_cuda.depth_similarity(c(depth0), c(depth1), c(ray), c(K), c(R0), c(t0), c(R1), c(t1), clamp)
         ctx.save_for_backward(g0, g1)
@@ -655,8 +648,7 @@ class DisparityLossFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, disp, edge):
-        if not disp.is_cuda:
-            raise RuntimeError("torchext.disparity_loss: connecting_the_dots_b200 has no CPU implementation")
+        _cuda_only(disp, "disparity_loss")
         sums, gd, ge = ext_cuda.disparity_loss(disp.detach().contiguous(), None if edge is None else edge.detach().contiguous())
         ctx.has_edge = edge is not None
         ctx.save_for_backward(gd, ge if ge is not None else gd)
@@ -680,8 +672,7 @@ class LCNFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, radius, epsilon):
-        if not x.is_cuda:
-            raise RuntimeError("torchext.lcn: connecting_the_dots_b200 has no CPU implementation")
+        _cuda_only(x, "lcn")
         out, std = ext_cuda.lcn_forward(x, radius, epsilon)
         ctx.radius, ctx.epsilon = radius, epsilon
         if x.dtype == torch.float32 and x.requires_grad:
@@ -707,8 +698,7 @@ def lcn_normalize(img, kernel_size=4, epsilon=0.01):
     """The data generator's offline LCN, data/lcn/lcn.pyx:16-58 `normalize(img, kernel_size, epsilon)` (called at
     data/create_syn_data.py:182): img [M,N] (or a batch [B,M,N]) -> (img_lcn, img_std), a border of kernel_size pixels left
     at 0, std = sqrt of the centred two-pass variance.  Bit-identical to the Cython build; CUDA tensors only."""
-    if not img.is_cuda:
-        raise RuntimeError("torchext.lcn_normalize: connecting_the_dots_b200 has no CPU implementation")
+    _cuda_only(img, "lcn_normalize")
     return ext_cuda.lcn_cython(img.contiguous(), kernel_size, epsilon)
 
 
