@@ -1213,10 +1213,16 @@ static bool xcorr_sep_launch(const float* in0, const float* in1, float* out, int
   return ok;
 }
 
-// Images per separable launch: as many as keep the fix-up's hit list (1/32 of the outputs, 16 M entries at most) at its
-// full relative size (see xcorrvol_impl).
+// Images per separable launch (D, H, W >= 1): as many as keep the fix-up's hit list (1/32 of the outputs, 16 M entries at
+// most) at its full relative size (see xcorrvol_impl), and no more than xcorr_sep_launch takes in one launch -- gridDim.z
+// = images x disparity chunks <= 65535, statistics positions < 2^31.  A large batch is split into more launches instead
+// of leaving the separable path; xcorr_sep_launch refuses only sizes that one image already exceeds.
 static int64_t xcorr_images_per_launch(int64_t D, int64_t H, int64_t W) {
-  return std::max<int64_t>(1, (((int64_t)1 << 24) - 1024) * 32 / std::max<int64_t>(D * H * W, 1));
+  const int64_t ndchunks = cdiv(D, XS_DT), ws1 = ndchunks * XS_DT + cdiv(W, 4) * 4;
+  const int64_t hits = (((int64_t)1 << 24) - 1024) * 32 / (D * H * W);
+  const int64_t grid = 65535 / ndchunks;
+  const int64_t stats = (((int64_t)1 << 31) - 1) / (H * ws1);
+  return std::max<int64_t>(1, std::min({hits, grid, stats}));
 }
 
 template <typename T>

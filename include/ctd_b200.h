@@ -150,9 +150,11 @@ int ctd_xcorrvol_f64(const double* in0, const double* in1, double* out, int64_t 
  * inputs with the default options: fp32, C = 1, block 3/5/7/9 run one fused pass over the separable kernel's outputs
  * (workspace grows with B*H*W, not B*D*H*W); every other case, and force_generic, runs a generic kernel, the exact argmax
  * of the generic volume.  Not mirrored: the A/B options xcorr_direct and xcorr_nofix (the disparity always uses the
- * separable kernel with its fix-up), and sizes the separable launch rejects (> 65535 row tiles or image x disparity-chunk
- * launches, 2^31 statistics positions), where the volume falls back to its direct kernel and the disparity to the generic
- * one -- equal to within the volume's 1e-5 there, not bit for bit.  In the fused path the sub-pixel scores are re-evaluated
+ * separable kernel with its fix-up), and images that one separable launch cannot take even alone (H > 1048560, more than
+ * 65535 chunks of 16 disparities, or H * (16 ceil(D/16) + 4 ceil(W/4)) >= 2^31 window-statistics positions), where the
+ * volume falls back to its direct or generic kernel and the disparity to the generic one -- equal to within the volume's
+ * 1e-5 there, not bit for bit.  The batch size alone never leaves the separable path: both ops cut a batch into launches
+ * of as many images as one launch takes.  In the fused path the sub-pixel scores are re-evaluated
  * in the centred form, within ~1e-5 of the volume's.  The inputs must be finite: for non-finite inputs the
  * result is unspecified (the call does not fault). */
 int ctd_xcorr_disparity_f32(const float* in0, const float* in1, float* disp, float* score, int64_t B, int64_t C, int64_t H,

@@ -121,11 +121,12 @@ def _expect(ks, ran, among, what):
         assert got == set(ran), "%s: ran %s, expected %s (all kernels: %s)" % (what, sorted(got), sorted(ran), sorted({n for n, _ in ks}))
 
 
-def _expect_chunks(ks, name, B, chunk, what):
-    """`name` ran once per chunk of at most `chunk` images, the image index in gridDim.z."""
+def _expect_chunks(ks, name, B, chunk, what, zper=1):
+    """`name` ran once per chunk of at most `chunk` images, gridDim.z = the chunk's images x zper."""
     if _seen(ks, what):
         z = [g[2] for g in _grids(ks, name) if len(g) == 3]
-        assert z == [min(chunk, B - b0) for b0 in range(0, B, chunk)], "%s: %s grid.z per launch %s" % (what, name, z)
+        want = [min(chunk, B - b0) * zper for b0 in range(0, B, chunk)]
+        assert z == want, "%s: %s grid.z per launch %s, expected %s" % (what, name, z, want)
 
 
 # ---------------------------------------------------------------- 1. photometric loss, unaligned pointers
