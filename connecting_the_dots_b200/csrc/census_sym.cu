@@ -726,7 +726,7 @@ bool census_sym_launch(const float* es, const float* ta, const float* go, float*
                        int64_t B, int64_t C, int64_t H, int64_t W, int type, float eps, cudaStream_t st) {
   if (g_census_sym == 2) {
     const int64_t px = B * H * W;
-    // forward + backward in one call: the tile kernel with packed fp32 taps wins at every size measured (r02_census_stream_ab.json)
+    // forward + backward in one call: the tile kernel with packed fp32 taps wins at every size measured (DESIGN §4.2)
     if (px < CS_MIN_PIXELS || (out != nullptr && gi != nullptr)) return false;
   }
   if (!g_census_sym || g_force_generic || C != 1 || B < 1 || H < 16 || W < 16 || H * W >= (int64_t)1 << 30 || (type != 2 && type != 3)) return false;

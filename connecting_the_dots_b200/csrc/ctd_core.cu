@@ -16,13 +16,6 @@ int g_host_graphs = 0;        // host-buffer API: 1 = capture repeated batches i
 int g_host_chunks_graph = 2;  // image chunks per call in a batch that is captured (measured: finer chunks lose on the bus even with no host cost)
 int g_host_chunks_batch = 2;  // ... inside ctd_host_begin_batch / end_batch, where neighbouring calls already overlap
 int g_host_chunks = 4;     // host-buffer API: image chunks per call (copies below ~2 MB lose PCIe efficiency)
-extern int g_census_pairs;
-extern int g_census_sym;
-extern int g_census_stream;
-extern int g_xcorr_serial;
-extern int g_proj_nn_tile;
-extern int g_census_sym_noguard;
-extern int g_census_sym_dbg;
 int g_disable_tma = 0;    // tests / A-B runs: use the shared-memory tile kernels instead of the TMA ones
 static std::atomic<uint64_t> g_launches{0};
 
@@ -186,6 +179,32 @@ int check_launch(const char* what) {
   return CTD_OK;
 }
 
+extern int g_census_sym;          // census_sym.cu
+extern int g_census_sym_dbg;      // census_sym.cu
+extern int g_census_sym_noguard;  // census_sym.cu
+extern int g_xcorr_serial;        // xcorrvol.cu
+
+// The names ctd_set_option accepts and the variable each one sets (meanings and defaults where they are defined).
+static const struct {
+  const char* name;
+  int* value;
+} k_options[] = {
+    {"force_generic", &g_force_generic},
+    {"disable_tma", &g_disable_tma},
+    {"census_sym", &g_census_sym},
+    {"census_sym_dbg", &g_census_sym_dbg},
+    {"census_sym_noguard", &g_census_sym_noguard},
+    {"xcorr_direct", &g_xcorr_direct},
+    {"xcorr_serial", &g_xcorr_serial},
+    {"xcorr_hitcap", &g_xcorr_hitcap},
+    {"xcorr_nofix", &g_xcorr_nofix},
+    {"host_graphs", &g_host_graphs},
+    {"host_chunks", &g_host_chunks},
+    {"host_chunks_batch", &g_host_chunks_batch},
+    {"host_chunks_graph", &g_host_chunks_graph},
+    {"ms_force_scratch", &g_ms_force_scratch},
+};
+
 }  // namespace ctd
 
 CTD_API const char* ctd_last_error(void) { return ctd::err_buf(); }
@@ -193,73 +212,11 @@ CTD_API const char* ctd_version(void) { return "ctd_b200 0.1 (sm_100a)"; }
 CTD_API uint64_t ctd_launch_count(void) { return ctd::g_launches.load(std::memory_order_relaxed); }
 
 CTD_API int ctd_set_option(const char* name, int value) {
-  if (name && !strcmp(name, "force_generic")) {
-    ctd::g_force_generic = value;
-    return CTD_OK;
-  }
-  if (name && !strcmp(name, "xcorr_direct")) {
-    ctd::g_xcorr_direct = value;
-    return CTD_OK;
-  }
-  if (name && !strcmp(name, "xcorr_nofix")) {
-    ctd::g_xcorr_nofix = value;
-    return CTD_OK;
-  }
-  if (name && !strcmp(name, "xcorr_hitcap")) {
-    ctd::g_xcorr_hitcap = value;
-    return CTD_OK;
-  }
-  if (name && !strcmp(name, "host_graphs")) {
-    ctd::g_host_graphs = value;
-    return CTD_OK;
-  }
-  if (name && !strcmp(name, "host_chunks_graph")) {
-    ctd::g_host_chunks_graph = value;
-    return CTD_OK;
-  }
-  if (name && !strcmp(name, "host_chunks_batch")) {
-    ctd::g_host_chunks_batch = value;
-    return CTD_OK;
-  }
-  if (name && !strcmp(name, "host_chunks")) {
-    ctd::g_host_chunks = value;
-    return CTD_OK;
-  }
-  if (name && !strcmp(name, "census_pairs")) {
-    ctd::g_census_pairs = value;
-    return CTD_OK;
-  }
-  if (name && !strcmp(name, "census_stream")) {
-    ctd::g_census_stream = value;
-    return CTD_OK;
-  }
-  if (name && !strcmp(name, "census_sym")) {
-    ctd::g_census_sym = value;
-    return CTD_OK;
-  }
-  if (name && !strcmp(name, "xcorr_serial")) {
-    ctd::g_xcorr_serial = value;
-    return CTD_OK;
-  }
-  if (name && !strcmp(name, "proj_nn_tile")) {
-    ctd::g_proj_nn_tile = value;
-    return CTD_OK;
-  }
-  if (name && !strcmp(name, "ms_force_scratch")) {
-    ctd::g_ms_force_scratch = value;
-    return CTD_OK;
-  }
-  if (name && !strcmp(name, "census_sym_dbg")) {
-    ctd::g_census_sym_dbg = value;
-    return CTD_OK;
-  }
-  if (name && !strcmp(name, "census_sym_noguard")) {
-    ctd::g_census_sym_noguard = value;
-    return CTD_OK;
-  }
-  if (name && !strcmp(name, "disable_tma")) {
-    ctd::g_disable_tma = value;
-    return CTD_OK;
+  for (const auto& o : ctd::k_options) {
+    if (name && !strcmp(name, o.name)) {
+      *o.value = value;
+      return CTD_OK;
+    }
   }
   return ctd::fail(CTD_ERR_INVALID, "ctd_set_option: unknown option '%s'", name ? name : "(null)");
 }

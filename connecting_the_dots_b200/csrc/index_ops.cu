@@ -251,171 +251,6 @@ proj_nn_fixed_kernel(const T* __restrict__ xyz0, const T* __restrict__ xyz1, con
   out[i] = best < 0 ? (int64_t)-1 : b * (int64_t)hw + best;
 }
 
-// 2-D query tiles with the candidates' window of xyz1 staged in shared memory (float, fixed patch sizes).  A CTA owns
-// 32 x 32 query pixels (four per thread); neighbouring queries project to neighbouring pixels of the other frame (smooth geometry), so the
-// union of their PS x PS patches is a window little larger than the tile wherever the motion takes it.  The CTA finds
-// that window (bounding box of the patches that touch the image), stages its rows -- contiguous runs of 12-byte points,
-// coalesced -- and every candidate becomes three conflict-free shared-memory loads (stride 3 words) instead of three
-// global gathers whose 32 lanes straddle three or four 128-byte lines each.  A tile whose window does not fit (wild
-// geometry) scans global memory exactly like proj_nn_fixed_kernel.  Same arithmetic, same scan order, same indices.
-constexpr int PT_W = 32, PT_H = 32, PT_QPT = 4, PT_CAP = 3072;  // query tile, queries per thread, staged points (36 KB)
-
-template <int PS>
-__global__ void __launch_bounds__(PT_W* PT_H / PT_QPT)
-proj_nn_tile_kernel(const float* __restrict__ xyz0, const float* __restrict__ xyz1, const float* __restrict__ K,
-                    int64_t* __restrict__ out, int H, int W, int tiles_x, int tiles_y) {
-  __shared__ float win[PT_CAP * 3];
-  __shared__ int s_box[4];  // min ub, max ub, min vb, max vb over the queries whose patch touches the image
-  constexpr int ROWS = PT_H / PT_QPT;  // thread (lx, ly) owns the queries of tile rows ly, ly + ROWS, ...
-  const int tid = threadIdx.x, lx = tid % PT_W, ly = tid / PT_W;
-  const int tile = blockIdx.x % (tiles_x * tiles_y);
-  const int64_t b = blockIdx.x / (tiles_x * tiles_y);
-  const int px = (tile % tiles_x) * PT_W + lx, py0 = (tile / tiles_x) * PT_H + ly;
-  const unsigned hw = (unsigned)H * (unsigned)W;
-  const float* img1 = xyz1 + b * (int64_t)hw * 3;
-  if (tid == 0) {
-    s_box[0] = INT32_MAX;
-    s_box[1] = INT32_MIN;
-    s_box[2] = INT32_MAX;
-    s_box[3] = INT32_MIN;
-  }
-  float k[9];
-#pragma unroll
-  for (int j = 0; j < 9; ++j) k[j] = __ldg(K + j);
-  constexpr int half = PS / 2;
-  float x[PT_QPT], y[PT_QPT], z[PT_QPT];
-  int ub[PT_QPT], vb[PT_QPT];
-  bool valid[PT_QPT];
-#pragma unroll
-  for (int m = 0; m < PT_QPT; ++m) {  // all query loads in flight together
-    const int py = py0 + m * ROWS;
-    valid[m] = px < W && py < H;
-    x[m] = y[m] = z[m] = 0.f;
-    if (valid[m]) {
-      const float* q = xyz0 + (b * (int64_t)hw + (int64_t)py * W + px) * 3;
-      x[m] = __ldg(q);
-      y[m] = __ldg(q + 1);
-      z[m] = __ldg(q + 2);
-    }
-  }
-  int a0 = INT32_MAX, a1 = INT32_MIN, c0 = INT32_MAX, c1 = INT32_MIN;
-#pragma unroll
-  for (int m = 0; m < PT_QPT; ++m) {
-    const float den = k[6] * x[m] + k[7] * y[m] + k[8] * z[m];
-    const float u = (k[0] * x[m] + k[1] * y[m] + k[2] * z[m]) / den;
-    const float v = (k[3] * x[m] + k[4] * y[m] + k[5] * z[m]) / den;
-    const int u0 = x86_double_to_int((double)u + 0.5);
-    const int v0 = x86_double_to_int((double)v + 0.5);
-    // INT_MIN (x86's answer to NaN / out of range) must stay far outside the image after the offsets are added
-    ub[m] = u0 < -(1 << 30) ? -(1 << 30) : u0 - half;
-    vb[m] = v0 < -(1 << 30) ? -(1 << 30) : v0 - half;
-    if (valid[m] && ub[m] > -PS && ub[m] < W && vb[m] > -PS && vb[m] < H) {  // some candidate lies inside the image
-      a0 = min(a0, ub[m]);
-      a1 = max(a1, ub[m]);
-      c0 = min(c0, vb[m]);
-      c1 = max(c1, vb[m]);
-    }
-  }
-  __syncthreads();
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    a0 = min(a0, __shfl_xor_sync(0xffffffffu, a0, o));
-    a1 = max(a1, __shfl_xor_sync(0xffffffffu, a1, o));
-    c0 = min(c0, __shfl_xor_sync(0xffffffffu, c0, o));
-    c1 = max(c1, __shfl_xor_sync(0xffffffffu, c1, o));
-  }
-  if ((tid & 31) == 0 && a0 <= a1) {
-    atomicMin(&s_box[0], a0);
-    atomicMax(&s_box[1], a1);
-    atomicMin(&s_box[2], c0);
-    atomicMax(&s_box[3], c1);
-  }
-  __syncthreads();
-  const int wx0 = max(s_box[0], 0), wx1 = min(s_box[1] + PS - 1, W - 1);
-  const int wy0 = max(s_box[2], 0), wy1 = min(s_box[3] + PS - 1, H - 1);
-  const int ww = wx1 - wx0 + 1, wh = wy1 - wy0 + 1;
-  const bool staged = s_box[0] <= s_box[1] && ww > 0 && wh > 0 && (int64_t)ww * wh <= PT_CAP;  // block-uniform
-  if (staged) {
-    const int rowlen = ww * 3;
-    for (int r = tid >> 5; r < wh; r += (PT_W * PT_H / PT_QPT) / 32) {
-      const float* src = img1 + ((unsigned)(wy0 + r) * (unsigned)W + (unsigned)wx0) * 3u;
-      float* dst = win + r * rowlen;
-      for (int c = tid & 31; c < rowlen; c += 32) dst[c] = __ldg(src + c);
-    }
-  }
-  __syncthreads();
-#pragma unroll
-  for (int m = 0; m < PT_QPT; ++m) {
-    if (!valid[m]) continue;
-    float best_d = 1e9f;
-    int best = -1;
-#pragma unroll
-    for (int pv = 0; pv < PS; ++pv) {
-      const int v1 = vb[m] + pv;
-      const bool vok = v1 >= 0 && v1 < H;
-      float qx[PS], qy[PS], qz[PS];
-#pragma unroll
-      for (int pu = 0; pu < PS; ++pu) {
-        const int u1 = ub[m] + pu;
-        const bool ok = vok && u1 >= 0 && u1 < W;
-        if (staged) {
-          const float* q = win + (ok ? (v1 - wy0) * ww + (u1 - wx0) : 0) * 3;
-          qx[pu] = ok ? q[0] : INFINITY;
-          qy[pu] = ok ? q[1] : 0.f;
-          qz[pu] = ok ? q[2] : 0.f;
-        } else {
-          const float* q = img1 + (unsigned)(ok ? v1 * W + u1 : 0) * 3u;
-          qx[pu] = ok ? __ldg(q) : INFINITY;
-          qy[pu] = ok ? __ldg(q + 1) : 0.f;
-          qz[pu] = ok ? __ldg(q + 2) : 0.f;
-        }
-      }
-#pragma unroll
-      for (int pu = 0; pu < PS; ++pu) {
-        const float dd = (x[m] - qx[pu]) * (x[m] - qx[pu]) + (y[m] - qy[pu]) * (y[m] - qy[pu]) + (z[m] - qz[pu]) * (z[m] - qz[pu]);
-        if (dd < best_d) {
-          best_d = dd;
-          best = (vb[m] + pv) * W + (ub[m] + pu);
-        }
-      }
-    }
-    out[b * (int64_t)hw + (int64_t)(py0 + m * ROWS) * W + px] = best < 0 ? (int64_t)-1 : b * (int64_t)hw + best;
-  }
-}
-
-template <typename T>
-struct ProjNNTile {
-  static bool launch(const T*, const T*, const T*, int64_t*, int64_t, int64_t, int64_t, int, cudaStream_t) { return false; }
-};
-// ctd_set_option("proj_nn_tile", 1): route float calls through the tile kernel.  OFF by default: measured on B200 (12 frame
-// pairs of 480x640, profiles/r02_proj_nn_tile.json) it is SLOWER than the row-segment kernel with global gathers -- patch 3:
-// 67 us (32x32 tiles, four queries per thread; 77 us with 32x8 tiles) against 55 us, patch 5: 158 against 107 us.  The
-// gathers of the row kernel mostly hit L1, and a tile pays two more dependent phases per CTA (bounding box, staging).
-int g_proj_nn_tile = 0;
-template <>
-struct ProjNNTile<float> {
-  static bool launch(const float* xyz0, const float* xyz1, const float* K, int64_t* out, int64_t B, int64_t H, int64_t W, int ps,
-                     cudaStream_t st) {
-    if (!g_proj_nn_tile) return false;
-    const int64_t tx = cdiv(W, PT_W), ty = cdiv(H, PT_H), n = B * tx * ty;
-    if (n > INT32_MAX) return false;
-#define CTD_PT_CASE(PS)                                                                                                          \
-  case PS:                                                                                                                       \
-    proj_nn_tile_kernel<PS><<<(unsigned)n, PT_W * PT_H / PT_QPT, 0, st>>>(xyz0, xyz1, K, out, (int)H, (int)W, (int)tx, (int)ty);          \
-    return true;
-    switch (ps) {
-      CTD_PT_CASE(1)
-      CTD_PT_CASE(2)
-      CTD_PT_CASE(3)
-      CTD_PT_CASE(5)
-      CTD_PT_CASE(7)
-      CTD_PT_CASE(9)
-      default: return false;
-    }
-#undef CTD_PT_CASE
-  }
-};
-
 template <typename T>
 static int proj_nn_impl(const T* xyz0, const T* xyz1, const T* K, int64_t* out, int64_t B, int64_t H, int64_t W,
                         int ps, cudaStream_t st) {
@@ -428,10 +263,6 @@ static int proj_nn_impl(const T* xyz0, const T* xyz1, const T* K, int64_t* out, 
   CTD_REQUIRE(cdiv(total, PN_THREADS) <= INT32_MAX, "proj_nn: too many pixels");
   const unsigned grid = (unsigned)cdiv(total, PN_THREADS);
   const bool fixed = !g_force_generic && H * W < ((int64_t)1 << 31) / 3;
-  if (fixed && ProjNNTile<T>::launch(xyz0, xyz1, K, out, B, H, W, ps, st)) {
-    count_launch();
-    return check_launch("proj_nn(tile)");
-  }
 #define CTD_PN_CASE(PS)                                                                                             \
   case PS:                                                                                                          \
     proj_nn_fixed_kernel<T, PS><<<grid, PN_THREADS, 0, st>>>(xyz0, xyz1, K, out, total, (int)H, (int)W);           \

@@ -31,24 +31,13 @@ int box9_tma_fwd_bwd(const float* es, const float* ta, const float* go, float* o
 int masked_sums_launch(const float* diff, const float* mask, int64_t n, float* out2, cudaStream_t st);
 int box9_tma_fwd_bwd_masked(const float* es, const float* ta, const float* go, const float* mask, float* out, float* gi,
                             float* sums2, int64_t B, int64_t C, int64_t H, int64_t W, int type, cudaStream_t st);
-int census_pairs_fwd(const float* es, const float* ta, float* out, int64_t B, int64_t C, int64_t H, int64_t W, int type,
-                     float eps, cudaStream_t st);
-// census_sym.cu: every pixel pair evaluated once (forward, backward or both, optional masked sums); false = not taken
+// census_sym.cu: every pixel pair evaluated once (forward, backward or both, optional masked sums); false = not taken.
+// Two kernels serve census_mse / census_sad at block size 9: this pair-symmetric one and the tile kernels below, which
+// take every call it refuses.  The choice is census_sym_launch's size rule: by default it takes forward-only and
+// backward-only calls from ~6 images (CS_MIN_PIXELS) and leaves fused forward+backward calls to the tile kernels;
+// ctd_set_option("census_sym", 0 / 1) sends every call to the tile kernels / to it where the shape allows.
 bool census_sym_launch(const float* es, const float* ta, const float* go, float* out, float* gi, const float* mask, float* sums2,
                        int64_t B, int64_t C, int64_t H, int64_t W, int type, float eps, cudaStream_t st);
-// census_stream.cu: persistent CTAs, tiles through a cp.async ring, packed fp32 taps (calls with a backward); false = not taken
-bool census_stream_launch(const float* es, const float* ta, const float* go, float* out, float* gi, const float* mask, float* sums2,
-                          int64_t B, int64_t C, int64_t H, int64_t W, int type, float eps, cudaStream_t st);
-extern int g_census_sym;
-// The census kernels that take whole calls: the pair-symmetric one by its own size rule (forward-only and backward-only
-// calls from ~6 images, or when forced by option), the streaming one when switched on (census_stream.cu: measured equal to the
-// tile kernels below, which take whatever is left).
-static bool census_fast_launch(const float* es, const float* ta, const float* go, float* out, float* gi, const float* mask,
-                               float* sums2, int64_t B, int64_t C, int64_t H, int64_t W, int type, float eps, cudaStream_t st) {
-  if (g_census_sym == 1 && census_sym_launch(es, ta, go, out, gi, mask, sums2, B, C, H, W, type, eps, st)) return true;
-  if (gi && census_stream_launch(es, ta, go, out, gi, mask, sums2, B, C, H, W, type, eps, st)) return true;
-  return census_sym_launch(es, ta, go, out, gi, mask, sums2, B, C, H, W, type, eps, st);
-}
 
 // ------------------------------------------------------------------------------------------
 // generic kernels (any block size, channel count, size; float or double)
@@ -1063,7 +1052,6 @@ CTD_API int ctd_photometric_fwd_f32(const float* es, const float* ta, float* out
   if (type <= 1 && box9_tma_fwd(es, ta, out, B, C, H, W, type, st)) return check_launch("photometric_fwd(tma)");
   if (type >= 2 && es && ta && out && census_sym_launch(es, ta, nullptr, out, nullptr, nullptr, nullptr, B, C, H, W, type, eps, st))
     return check_launch("photometric_fwd(census, pair-symmetric)");
-  if (type >= 2 && census_pairs_fwd(es, ta, out, B, C, H, W, type, eps, st)) return check_launch("photometric_fwd(census pairs)");
   const int vec = vec_ok(W, es, ta, out, out);
   for (int64_t b0 = 0; b0 < B; b0 += 32768) {
     const int nb = (int)std::min<int64_t>(32768, B - b0);
@@ -1097,7 +1085,7 @@ CTD_API int ctd_photometric_bwd_f32(const float* es, const float* ta, const floa
   if (int rc = check_common(es, ta, gi, B, C, H, W, bs, type)) return rc;
   CTD_REQUIRE(go, "photometric_bwd: null grad_out");
   if (type <= 1 && box9_tma_bwd(es, ta, go, gi, B, C, H, W, type, st)) return check_launch("photometric_bwd(tma)");
-  if (type >= 2 && es && ta && gi && census_fast_launch(es, ta, go, nullptr, gi, nullptr, nullptr, B, C, H, W, type, eps, st))
+  if (type >= 2 && es && ta && gi && census_sym_launch(es, ta, go, nullptr, gi, nullptr, nullptr, B, C, H, W, type, eps, st))
     return check_launch("photometric_bwd(census, pair-symmetric)");
   const int vec = vec_ok(W, es, ta, go, gi);
   for (int64_t b0 = 0; b0 < B; b0 += 32768) {
@@ -1129,8 +1117,8 @@ CTD_API int ctd_photometric_fwd_bwd_f32(const float* es, const float* ta, const 
   if (type >= 2 && type <= 3 && fast9_ok(bs, H, W) && C >= 1 && B >= 1) {
     if (int rc = check_common(es, ta, gi, B, C, H, W, bs, type)) return rc;
     CTD_REQUIRE(go && out, "photometric_fwd_bwd: null pointer");
-    if (es && ta && gi && census_fast_launch(es, ta, go, out, gi, nullptr, nullptr, B, C, H, W, type, eps, st))
-      return check_launch("photometric_fwd_bwd(census, whole-call kernel)");
+    if (es && ta && gi && census_sym_launch(es, ta, go, out, gi, nullptr, nullptr, B, C, H, W, type, eps, st))
+      return check_launch("photometric_fwd_bwd(census, pair-symmetric)");
     const int vec = vec_ok(W, es, ta, go, gi) && (reinterpret_cast<uintptr_t>(out) & 15) == 0;
     for (int64_t b0 = 0; b0 < B; b0 += 32768) {
       const int nb = (int)std::min<int64_t>(32768, B - b0);
@@ -1162,8 +1150,8 @@ CTD_API int ctd_photometric_fwd_bwd_masked_f32(const float* es, const float* ta,
   if (fast9_ok(bs, H, W) && C >= 1 && B >= 1 && B <= 32768) {
     if (type <= 1 && box9_tma_fwd_bwd_masked(es, ta, go, mask, out, gi, sums2, B, C, H, W, type, st))
       return check_launch("photometric_fwd_bwd_masked(box, fused)");
-    if (type >= 2 && es && ta && gi && census_fast_launch(es, ta, go, out, gi, mask, sums2, B, C, H, W, type, eps, st))
-      return check_launch("photometric_fwd_bwd_masked(census, whole-call kernel)");
+    if (type >= 2 && es && ta && gi && census_sym_launch(es, ta, go, out, gi, mask, sums2, B, C, H, W, type, eps, st))
+      return check_launch("photometric_fwd_bwd_masked(census, pair-symmetric)");
     if (type >= 2) {
       const int vec = vec_ok(W, es, ta, go, gi) && ((reinterpret_cast<uintptr_t>(out) | reinterpret_cast<uintptr_t>(mask)) & 15) == 0;
       if (census_bwd_launch(es, ta, go, gi, out, (int)B, C, H, W, type, eps, vec, st, mask, sums2)) {

@@ -60,7 +60,7 @@ SHAPES = [  # B, C, H, W, bs -- ragged widths (scalar path), multi-tile, tiny (g
     (2, 1, 33, 132, 9), (1, 1, 40, 67, 9), (1, 2, 64, 256, 9), (1, 1, 9, 9, 9), (3, 1, 70, 200, 9),
     (1, 3, 17, 23, 9), (1, 1, 5, 6, 9), (1, 1, 3, 3, 9), (2, 1, 20, 31, 5), (1, 2, 16, 16, 4), (1, 1, 12, 40, 1),
     (1, 1, 8, 300, 9), (1, 1, 300, 12, 9),
-    # census pair kernels: one full 120-column strip exactly, full + leftover strip, packed leftover strips only
+    # more census widths and heights: 120, 160 and 44 columns, 16 x 16
     (1, 1, 48, 120, 9), (2, 1, 40, 160, 9), (3, 1, 100, 44, 9), (1, 1, 16, 16, 9),
 ]
 
@@ -98,47 +98,6 @@ def test_photometric_generic_kernels_agree(tx, ty):
     fwd2, bwd2 = photometric_both(tx, es, ta, go, 9, ty, 0.3)
     assert_close(fwd2, fwd, what="fast vs generic fwd")
     assert_close(bwd2, bwd, what="fast vs generic bwd")
-
-
-@pytest.mark.parametrize("ty", (2, 3))
-def test_census_pair_kernels_match_gather_kernels(tx, ty):
-    """A/B inside the library: the pair-symmetric census kernels against the shared-memory gather kernels."""
-    from connecting_the_dots_b200 import _lib
-    rng = np.random.RandomState(11)
-    es = rng.randn(2, 1, 150, 280).astype(np.float32)
-    ta = (es + 0.5 * rng.randn(2, 1, 150, 280)).astype(np.float32)
-    go = rng.rand(2, 1, 150, 280).astype(np.float32)
-    _lib.set_option("census_sym", 0)   # the gather-era kernels: forward-only pair kernel vs shared-memory gather
-    _lib.set_option("census_pairs", 1)
-    try:
-        fwd, bwd = photometric_both(tx, es, ta, go, 9, ty, 0.5)
-        _lib.set_option("census_pairs", 0)
-        fwd0, bwd0 = photometric_both(tx, es, ta, go, 9, ty, 0.5)
-    finally:
-        _lib.set_option("census_pairs", 2)
-        _lib.set_option("census_sym", 2)
-    assert_close(fwd, fwd0, what="pairs vs gather fwd")
-    assert_close(bwd, bwd0, what="pairs vs gather bwd")
-    assert_close(fwd, oracle.photometric_loss_forward(es, ta, 9, ty, 0.5), what="pairs vs oracle fwd")
-
-
-@pytest.mark.parametrize("shape", [(1, 1, 48, 120), (2, 1, 40, 160), (3, 1, 100, 44), (1, 1, 16, 16), (2, 1, 33, 132)])
-def test_census_pair_kernel_strip_layouts(tx, shape):
-    """Forced pair kernel on widths that give one exact strip, a full + a leftover strip, packed leftover strips."""
-    from connecting_the_dots_b200 import _lib
-    B, C, H, W = shape
-    rng = np.random.RandomState(W)
-    es = rng.randn(B, C, H, W).astype(np.float32)
-    ta = (es + 0.7 * rng.randn(B, C, H, W)).astype(np.float32)
-    _lib.set_option("census_sym", 0)
-    _lib.set_option("census_pairs", 1)
-    try:
-        for ty in (2, 3):
-            got = tx.photometric_loss(cu(es), cu(ta), 9, TYPES[ty], 0.5).cpu().numpy()
-            assert_close(got, oracle.photometric_loss_forward(es, ta, 9, ty, 0.5), what="pairs fwd %s" % TYPES[ty])
-    finally:
-        _lib.set_option("census_pairs", 2)
-        _lib.set_option("census_sym", 2)
 
 
 SYM_SHAPES = [(1, 16, 16), (2, 33, 132), (1, 40, 67), (1, 130, 200), (1, 250, 48), (3, 128, 36), (1, 129, 150), (2, 61, 301)]
@@ -234,17 +193,17 @@ def test_census_pair_symmetric_kernel_exact_sign_decisions(tx):
             _lib.set_option("census_sym", 2)
 
 
-STREAM_SHAPES = [(1, 9, 12), (2, 16, 64), (1, 10, 72), (3, 21, 132), (1, 130, 200), (2, 61, 300), (1, 250, 48), (5, 40, 68)]
+TILE_SHAPES = [(1, 9, 12), (2, 16, 64), (1, 10, 72), (3, 21, 132), (1, 130, 200), (2, 61, 300), (1, 250, 48), (5, 40, 68),
+               (2, 150, 280)]
 
 
-@pytest.mark.gpu
-@pytest.mark.parametrize("shape", STREAM_SHAPES)
+@pytest.mark.parametrize("shape", TILE_SHAPES)
 @pytest.mark.parametrize("ty", (2, 3))
-def test_census_streaming_kernel_vs_oracle(tx, shape, ty):
-    """census_stream.cu (persistent CTAs, cp.async tile ring, packed fp32 taps, deferred second pass for border / near-tie pixels)
-    through the three entry points with a backward, against the oracle: images smaller than a tile, ragged last tile
-    column (width a multiple of 4 but not of 64) and last tile row (height not a multiple of 8), more tiles than one CTA
-    round, every pixel of the smallest image ON the border."""
+def test_census_tile_kernel_vs_oracle(tx, shape, ty):
+    """The census tile kernels of photometric.cu (census_sym = 0: every call) through all four entry points against the
+    oracle, one launch each: images smaller than a 64 x 16 tile, ragged last tile column (width not a multiple of 64)
+    and last tile row (height not a multiple of 16), widths that are / are not multiples of four, several images,
+    every pixel of the smallest image ON the border."""
     B, H, W = shape
     rng = np.random.RandomState(H * 1000 + W + ty)
     es = rng.randn(B, 1, H, W).astype(np.float32)
@@ -253,31 +212,25 @@ def test_census_streaming_kernel_vs_oracle(tx, shape, ty):
     mask = (rng.rand(B, 1, H, W) + 0.5).astype(np.float32)
     from connecting_the_dots_b200 import _lib
     _lib.set_option("census_sym", 0)
-    _lib.set_option("census_stream", 1)   # opt-in kernel
     try:
         n0 = _lib.launch_count()
         r = _census_all_entry_points(tx, es, ta, go, mask, ty)
         assert _lib.launch_count() - n0 == 4, "one kernel per entry point"
-        _lib.set_option("census_stream", 0)   # A/B partner: the tile kernel of photometric.cu (the default)
-        tile = _census_all_entry_points(tx, es, ta, go, mask, ty)
     finally:
-        _lib.set_option("census_stream", 0)
         _lib.set_option("census_sym", 2)
     of, ob = oracle.photometric_loss_forward(es, ta, 9, ty, 0.5), oracle.photometric_loss_backward(es, ta, go, 9, ty, 0.5)
-    for k in ("f_fwd", "m_fwd"):
+    for k in ("fwd", "f_fwd", "m_fwd"):
         assert_close(r[k], of, what=k)
     for k in ("bwd", "f_bwd", "m_bwd"):
         assert_close(r[k], ob, what=k)
-        assert_close(r[k], tile[k], what=k + " vs tile kernel")
     want = np.array([(mask.astype(np.float64) * of).sum(), mask.astype(np.float64).sum()])
     assert np.abs(r["sums"] - want).max() <= 1e-5 * np.abs(want).max()
 
 
-@pytest.mark.gpu
-def test_census_streaming_kernel_exact_sign_decisions_and_determinism(tx):
-    """Quantised images (many window terms exactly zero or equal up to rounding), a constant image (EVERY pixel goes
-    through the in-warp correction) and the bench frames, whose flat regions tie exactly: census_sad's sign() decisions
-    have to be the reference's, and two runs have to agree bit for bit."""
+def test_census_tile_kernel_exact_sign_decisions_and_determinism(tx):
+    """The census tile kernels (census_sym = 0) on quantised images (many window terms exactly zero or equal up to
+    rounding), a constant image (every pair a tie) and the bench frames, whose flat regions tie exactly: census_sad's
+    sign() decisions have to be the reference's, and two runs have to agree bit for bit."""
     from connecting_the_dots_b200 import _lib, synth
     rng = np.random.RandomState(11)
     B, H, W = 2, 70, 120
@@ -287,7 +240,6 @@ def test_census_streaming_kernel_exact_sign_decisions_and_determinism(tx):
     d = synth.make_batch(1, 96, 128)
     cases = [(es, ta, go), (es, es.copy(), go), (np.full_like(es, 0.25), np.full_like(es, 0.75), go), (d["es"], d["ta"], d["go"])]
     _lib.set_option("census_sym", 0)
-    _lib.set_option("census_stream", 1)
     try:
         for e, t, g in cases:
             fwd, bwd = photometric_both(tx, e, t, g, 9, 3, 0.5)
@@ -297,7 +249,6 @@ def test_census_streaming_kernel_exact_sign_decisions_and_determinism(tx):
             scale = max(float(np.abs(ob).max()), 1e-30)
             assert float(np.abs(bwd - ob).max()) <= 1e-5 * scale + 1e-12, "quantised bwd"
     finally:
-        _lib.set_option("census_stream", 0)
         _lib.set_option("census_sym", 2)
 
 
@@ -754,11 +705,10 @@ def test_proj_nn_vs_oracle(tx, dt):
 
 
 @pytest.mark.parametrize("ps", (1, 2, 3, 5, 7, 9))
-def test_proj_nn_tile_kernel_matches_oracle_and_row_kernel(tx, ps):
-    """The shared-memory tile kernel (window of xyz1 staged per 32x8 query tile) against the oracle and the row-segment
-    kernel: smooth geometry (window staged), wild geometry (projections all over the image: window too large, global
-    fallback inside the same kernel), queries that miss the image, ragged image sizes."""
-    from connecting_the_dots_b200 import _lib, synth
+def test_proj_nn_fixed_kernel_vs_oracle(tx, ps):
+    """The fixed-patch row kernel against the oracle on a ragged image size: smooth geometry, wild geometry (projections
+    all over the image, NaN, zero depth, points behind the camera) and queries that all miss the image."""
+    from connecting_the_dots_b200 import synth
     xyz, K, poses = synth.make_clouds(2, 61, 83, seed=3)
     cases = [(synth.transform(xyz[0], poses[1])[None], xyz[1][None], K)]
     rng = np.random.RandomState(ps)
@@ -770,15 +720,8 @@ def test_proj_nn_tile_kernel_matches_oracle_and_row_kernel(tx, ps):
     far = (xyz[0] + np.float32([5.0, 0, 0]))[None]                                        # everything projects outside
     cases.append((far.astype(np.float32), xyz[1][None], K))
     for x0, x1, K_ in cases:
-        want = oracle.proj_nn(x0, x1, K_, ps)
-        row = tx.proj_nn(cu(x0), cu(x1), cu(K_), ps).cpu().numpy()     # default: row-segment kernel
-        assert np.array_equal(row, want)
-        _lib.set_option("proj_nn_tile", 1)
-        try:
-            got = tx.proj_nn(cu(x0), cu(x1), cu(K_), ps).cpu().numpy()
-        finally:
-            _lib.set_option("proj_nn_tile", 0)
-        assert np.array_equal(got, want)
+        got = tx.proj_nn(cu(x0), cu(x1), cu(K_), ps).cpu().numpy()
+        assert np.array_equal(got, oracle.proj_nn(x0, x1, K_, ps))
 
 
 def test_nn_golden_and_split(tx, golden):

@@ -1,5 +1,5 @@
-"""A/B timings of the census kernels at the bench size, every entry point: pair-symmetric (census_sym.cu), streaming
-(census_stream.cu), tile (photometric.cu) and the automatic dispatch.  python tools/experiments/census_sym_ab.py [batch]"""
+"""A/B timings of the census kernels at the bench size, every entry point: pair-symmetric (census_sym.cu), tile
+(photometric.cu) and the automatic dispatch.  python tools/experiments/census_sym_ab.py [batch]"""
 import os, sys, json
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
@@ -20,9 +20,7 @@ for s in range(NS):
     d["o1"], d["o2"], d["sums"] = torch.empty(B, 1, H, W, device=dev), torch.empty(B, 1, H, W, device=dev), torch.zeros(2, device=dev)
     sets.append(d)
 res = {}
-DEFAULTS = {"census_sym": 2, "census_stream": 0}
-for label, opts in (("sym", {"census_sym": 1}), ("stream", {"census_sym": 0, "census_stream": 1}), ("tile", {"census_sym": 0, "census_stream": 0}), ("auto", {})) + tuple(
-        ("stream_dbg%d" % int(a), {"census_sym": 0, "census_stream": int(a)}) for a in sys.argv[2:]):
+for label, opts in (("sym", {"census_sym": 1}), ("tile", {"census_sym": 0}), ("auto", {})):
     for k, v in opts.items():
         _lib.set_option(k, v)
     for ty in (2, 3):
@@ -38,6 +36,5 @@ for label, opts in (("sym", {"census_sym": 1}), ("stream", {"census_sym": 0, "ce
                       d["o1"].data_ptr(), d["o2"].data_ptr(), d["sums"].data_ptr(), B, 1, H, W, 9, ty, 0.5, st)
         for name, f in (("fwd", fwd), ("bwd", bwd), ("fused_masked", fused)):
             res["%s_t%d_%s" % (label, ty, name)] = round(timeit(f, 10)[0] * 1e3, 1)
-    for k in opts:
-        _lib.set_option(k, DEFAULTS.get(k, 0))
+    _lib.set_option("census_sym", 2)
 print(json.dumps(res, indent=1))
