@@ -13,7 +13,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, "csrc")
 OBJ = os.path.join(CSRC, "build")
 LIB = os.path.join(PKG, "libctd_b200.so")
-SOURCES = ["ctd_core.cu", "photometric.cu", "photometric_tma.cu", "census_sym.cu", "lcn.cu", "lcn_extra.cu", "xcorrvol.cu", "index_ops.cu", "reduce.cu", "warp.cu", "geometric.cu", "disparity_loss.cu", "ssim.cu", "sgm.cu", "census_match.cu", "disparity_check.cu", "host_api.cu"]
+SOURCES = ["ctd_core.cu", "photometric.cu", "photometric_tma.cu", "census_sym.cu", "lcn.cu", "lcn_extra.cu", "xcorrvol.cu", "index_ops.cu", "reduce.cu", "warp.cu", "geometric.cu", "disparity_loss.cu", "ssim.cu", "sgm.cu", "census_match.cu", "disparity_check.cu", "speckle.cu", "host_api.cu"]
 HEADERS = [os.path.join(CSRC, "ctd_common.cuh"), os.path.join(CSRC, "ctd_tma.cuh"), os.path.join(PKG, "..", "include", "ctd_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 # -fmad=false: the reference's CPU build has no fused multiply-adds and the index ops must match it

@@ -40,6 +40,8 @@ SIGNATURES = {
     "ctd_census_disparity_f64": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _int, _int, _int, _int, _ptr],
     "ctd_disparity_check_f32": [_ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _int, _f64, _int, _ptr],
     "ctd_disparity_check_f64": [_ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _int, _f64, _int, _ptr],
+    "ctd_speckle_filter_f32": [_ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _f64, _ptr],
+    "ctd_speckle_filter_f64": [_ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _f64, _ptr],
     "ctd_proj_nn_f32": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _int, _ptr],
     "ctd_proj_nn_f64": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _int, _ptr],
     "ctd_nn_f32": [_ptr, _ptr, _ptr, _i64, _i64, _ptr],

@@ -168,6 +168,24 @@ def disparity_check_cuda(vol, max_diff=1, uniqueness=0.0, subpixel=True):
     return disp, score, valid
 
 
+def speckle_filter_cuda(disp, valid, max_size, max_diff):
+    """Speckle filter of a disparity map (ctd_speckle_filter_*).  disp [B,1,H,W] (or [1,H,W]), valid None or bool of the
+    same shape -> valid_out, torch.bool of disp's shape."""
+    _check_input_cuda(disp, "disp")
+    _check(disp.dim() in (3, 4) and disp.size(-3) == 1, "disp has to be 1 x H x W (or B x 1 x H x W)")
+    sfx = _real_suffix(disp, "speckle_filter")
+    if valid is not None:
+        _check_input_cuda(valid, "valid")
+        _check(valid.dtype == torch.bool and tuple(valid.shape) == tuple(disp.shape), "valid has to be a bool tensor of disp's shape")
+        _check(valid.device == disp.device, "disp and valid must be on the same device")
+    H, W = disp.shape[-2:]
+    out = torch.empty(disp.shape, dtype=torch.bool, device=disp.device)
+    with torch.cuda.device(disp.device):
+        _lib.call("ctd_speckle_filter" + sfx, disp.data_ptr(), None if valid is None else valid.data_ptr(), out.data_ptr(),
+                  disp.size(0) if disp.dim() == 4 else 1, H, W, int(max_size), float(max_diff), _stream(disp))
+    return out
+
+
 def census_transform_cuda(x, wh, ww):
     """Census transform (ctd_census_transform_*): x [B,C,H,W] (or [C,H,W]) -> int64 of the same shape holding the uint64
     bit patterns."""

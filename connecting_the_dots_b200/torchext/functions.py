@@ -200,6 +200,77 @@ def disparity_check_pytorch(vol, max_diff=1, uniqueness=0.0, subpixel=True):
     return disp, score, valid
 
 
+def _speckle_args(op, disp, valid, max_size, max_diff):
+    if disp.dim() not in (3, 4) or disp.size(-3) != 1:
+        raise RuntimeError("%s: disp has to be 1 x H x W (or B x 1 x H x W)" % op)
+    ext_cuda._real_suffix(disp, op)
+    if valid is not None:
+        if valid.dtype != torch.bool or tuple(valid.shape) != tuple(disp.shape):
+            raise RuntimeError("%s: valid has to be a bool tensor of disp's shape" % op)
+        if valid.device != disp.device:
+            raise RuntimeError("%s: disp and valid must be on the same device" % op)
+    n, md = int(max_size), float(max_diff)
+    if n != max_size or n < 0:
+        raise RuntimeError("%s: max_size must be an integer >= 0, got %r" % (op, max_size))
+    if not (md >= 0.0 and md != float("inf")):
+        raise RuntimeError("%s: max_diff must be finite and >= 0, got %r" % (op, max_diff))
+    return n, md
+
+
+def speckle_filter(disp, valid=None, max_size=100, max_diff=1.0):
+    """Speckle filter of a disparity map disp [B,1,H,W] (or [1,H,W]): drop the connected regions of nearly equal disparity
+    with at most max_size pixels, as speckle_filter_pytorch states it.  valid (bool, disp's shape; None: every pixel) marks
+    the pixels that take part.  Returns valid_out (bool, disp's shape); disp is not modified.  Not differentiable.  CUDA
+    tensors only, float32 or float64."""
+    _cuda_only(disp, "speckle_filter")
+    n, md = _speckle_args("speckle_filter", disp, valid, max_size, max_diff)
+    return ext_cuda.speckle_filter_cuda(disp, valid, n, md)
+
+
+def speckle_filter_pytorch(disp, valid=None, max_size=100, max_diff=1.0):
+    """The definition of speckle_filter in plain torch, any device, and its test oracle.
+
+    Inputs: disp [B,1,H,W] (or [1,H,W]), float32 or float64; valid, the same shape, bool, None meaning every pixel is
+    valid; an integer max_size >= 0; a finite max_diff >= 0.
+    Adjacency: pixels p and q of the same image are adjacent when all of these hold: they are 4-neighbours
+    (|dh| + |dw| = 1); both are valid; |(double)disp[p] - (double)disp[q]| <= max_diff, evaluated in fp64.  A NaN disparity
+    is therefore adjacent to nothing.  Adjacency is not transitive in value: 0, 1, 2 in a row with max_diff = 1 form one
+    component.
+    Components: they are the connected components of that graph.  A valid pixel with no adjacent pixel is a component of
+    size 1.
+    Output: valid_out[p] = valid[p] && size(component of p) > max_size, and disp is not modified.  This equals OpenCV's
+    filterSpeckles(disp, newVal, max_size, max_diff) with invalid pixels preset to newVal.  max_size = 0 returns valid
+    unchanged.
+    Exactness: component membership does not depend on the algorithm that finds it, and sizes are integer counts.  So the
+    output is bit-equal to the definition, deterministic, and independent of the order in which atomics land.
+
+    Components are found by min-label hooking with pointer jumping (scatter_reduce "amin") until a fixed point."""
+    n, md = _speckle_args("speckle_filter", disp, valid, max_size, max_diff)
+    d = disp.reshape(-1, disp.size(-2), disp.size(-1)).double()
+    ok = torch.ones(d.shape, dtype=torch.bool, device=d.device) if valid is None else valid.reshape(d.shape)
+    B, H, W = d.shape
+    idx = torch.arange(B * H * W, device=d.device).view(B, H, W)
+    right = ok[:, :, :-1] & ok[:, :, 1:] & ((d[:, :, :-1] - d[:, :, 1:]).abs() <= md)
+    down = ok[:, :-1] & ok[:, 1:] & ((d[:, :-1] - d[:, 1:]).abs() <= md)
+    src = torch.cat([idx[:, :, :-1][right], idx[:, :-1][down]])
+    dst = torch.cat([idx[:, :, 1:][right], idx[:, 1:][down]])
+    lab = idx.view(-1)  # lab[x] <= x, a pixel of x's component; lab[lab] == lab after every round
+    while True:
+        ls, ld = lab[src], lab[dst]
+        m = torch.minimum(ls, ld)
+        new = lab.scatter_reduce(0, ls, m, "amin").scatter_reduce(0, ld, m, "amin")  # hook each edge's roots to the smaller
+        while True:
+            jumped = new[new]
+            if torch.equal(jumped, new):
+                break
+            new = jumped
+        if torch.equal(new, lab):  # every edge joins two pixels of one label: lab is the component's smallest pixel
+            break
+        lab = new
+    size = torch.bincount(lab, minlength=lab.numel())[lab].view(B, H, W)
+    return (ok & (size > n)).view(disp.shape)
+
+
 SGM_PATHS = {4:((0, 1), (0, -1), (1, 0), (-1, 0)),
              8: ((0, 1), (0, -1), (1, 0), (-1, 0), (1, 1), (1, -1), (-1, 1), (-1, -1))}
 

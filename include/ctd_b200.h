@@ -243,6 +243,31 @@ int ctd_disparity_check_f64(const double* vol, double* disp, double* score, doub
                             uint8_t* valid, int64_t B, int64_t D, int64_t H, int64_t W, int max_diff, double uniqueness,
                             int subpixel, ctd_stream_t stream);
 
+/* ---- speckle filter of a disparity map (an addition: OpenCV's filterSpeckles, the speckleWindowSize / speckleRange step
+ * of StereoSGBM, the peak filter of Hirschmueller's SGM): drop small connected regions of nearly equal disparity.
+ *   Inputs.  disp [B,1,H,W], float or double; valid, the same shape, uint8, nonzero meaning valid, NULL meaning every
+ *            pixel is valid; an integer max_size >= 0; a finite max_diff >= 0.
+ *   Adjacency.  Pixels p and q of the same image are adjacent when all of these hold: they are 4-neighbours
+ *            (|dh| + |dw| = 1); both are valid; |(double)disp[p] - (double)disp[q]| <= max_diff, evaluated in fp64.  A NaN
+ *            disparity is therefore adjacent to nothing.  Adjacency is not transitive in value: 0, 1, 2 in a row with
+ *            max_diff = 1 form one component.
+ *   Components.  They are the connected components of that graph.  A valid pixel with no adjacent pixel is a component of
+ *            size 1.
+ *   Output.  valid_out[p] = valid[p] && size(component of p) > max_size (uint8, 0 or 1), and disp is not modified.  This
+ *            equals OpenCV's filterSpeckles(disp, newVal, max_size, max_diff) with invalid pixels preset to newVal.
+ *            max_size = 0 returns valid unchanged.
+ *   Exactness.  Component membership does not depend on the algorithm that finds it, and sizes are integer counts.  So
+ *            the output is bit-equal to the definition, deterministic, and independent of the order in which atomics land.
+ * DEVICE pointers.  valid_out == NULL makes the call a no-op.  B*H*W = 0 is CTD_OK with nothing launched.  CTD_ERR_INVALID,
+ * checked before any device work, for: negative sizes; H*W > INT32_MAX (labels are image-local int32); a null disp;
+ * max_size < 0; a negative or non-finite max_diff; valid_out overlapping disp or valid.  Union-find labelling in four
+ * launches whatever the sizes; labels and sizes (8 bytes per pixel of int32) come from the library's stream-ordered
+ * scratch pool; integer atomics only, no host synchronisation, capture-safe; 64-bit indexing over the batch. */
+int ctd_speckle_filter_f32(const float* disp, const uint8_t* valid, uint8_t* valid_out, int64_t B, int64_t H, int64_t W,
+                           int64_t max_size, double max_diff, ctd_stream_t stream);
+int ctd_speckle_filter_f64(const double* disp, const uint8_t* valid, uint8_t* valid_out, int64_t B, int64_t H, int64_t W,
+                           int64_t max_size, double max_diff, ctd_stream_t stream);
+
 /* ---- ProjNNFunctor: ext.h:65-117, ext_cuda.cpp:47-69 (proj_nn_cuda).  K is a DEVICE pointer to
  * 9 values (row-major 3x3), like the reference's K tensor. */
 int ctd_proj_nn_f32(const float* xyz0, const float* xyz1, const float* K, int64_t* out, int64_t B,

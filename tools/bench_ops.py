@@ -3,7 +3,7 @@
 launching stream, rotating buffer sets larger than L2 where the op is HBM-bound).  Prints one JSON
 object; bench.py stays the contract benchmark, this is the per-op table that goes into profiles/.
 
-    python tools/bench_ops.py [--iters 30] [--only photometric,ssim,lcn,xcorrvol,xcorr_disparity,sgm,census_match,disparity_check,proj_nn,nn,crosscheck]
+    python tools/bench_ops.py [--iters 30] [--only photometric,ssim,lcn,xcorrvol,xcorr_disparity,sgm,census_match,disparity_check,speckle,proj_nn,nn,crosscheck]
 
 The printed result names the GPU and its power limit, read in the same run.
 """
@@ -77,7 +77,7 @@ def census_traffic(B, C, H, W, D):
     return {"volume": (4 * D + 8 * C) * npx, "disparity": (8 * C + 8) * npx}
 
 
-ALL = "calib,photometric,ssim,warp,pyramid,geometric,disparity,lcn,xcorrvol,xcorr_disparity,sgm,census_match,disparity_check,proj_nn,config4,nn,crosscheck,reduce,gpu_reference"
+ALL = "calib,photometric,ssim,warp,pyramid,geometric,disparity,lcn,xcorrvol,xcorr_disparity,sgm,census_match,disparity_check,speckle,proj_nn,config4,nn,crosscheck,reduce,gpu_reference"
 
 
 def main():
@@ -519,6 +519,39 @@ def run(only=ALL, iters=30, batch=8, device_index=0, verbose=True):
         r["ratio_vs_disparity_from_volume"] = res["ops"]["disparity_from_volume_D128"]["ms_median"] / r["ms_median"]
         r["valid_frac"] = float(o_v.float().mean())
         del vol
+    if "speckle" in only:
+        # speckle filter (max_size 200, max_diff 1) of the census block-9 integer disparities of the bench frames (7x9
+        # window, D = 128) after disparity_check(max_diff 1): the fused call against speckle_filter_pytorch on the GPU.  The
+        # floor is disp and valid in, valid_out out (6 B/px); labels and sizes add 8 B/px of scratch, written once and
+        # read about once.  One input serves every launch: at batch 8 it and the scratch (54 MB in all) fit in L2.
+        vol = torch.empty(B, 128, H, W, device=dev)
+        _lib.call("ctd_census_vol_f32", sets[0]["ta"].data_ptr(), sets[0]["pat_lcn"].data_ptr(), vol.data_ptr(), B, 1, H, W, 128,
+                  7, 9, 9, torch.cuda.current_stream().cuda_stream)
+        disp, _, ok = tx.disparity_check(vol, 1, 0.0, subpixel=False)
+        del vol
+        o_v = torch.empty(B, 1, H, W, dtype=torch.uint8, device=dev)
+
+        def f(i, st):
+            _lib.call("ctd_speckle_filter_f32", disp.data_ptr(), ok.data_ptr(), o_v.data_ptr(), B, H, W, 200, 1.0, st)
+        add("speckle_filter", *timeit(f, args.iters), 6 * npx,
+            extra={"note": "disp (4 B/px) and valid (1 B/px) in, valid_out (1 B/px) out; 4 launches",
+                   "scratch_bytes": 16 * npx})
+        ref = tx.speckle_filter_pytorch(disp, ok, 200, 1.0)
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        torch.cuda.synchronize()
+        e0.record()
+        for _ in range(3):
+            tx.speckle_filter_pytorch(disp, ok, 200, 1.0)
+        e1.record()
+        torch.cuda.synchronize()
+        ms = e0.elapsed_time(e1) / 3
+        add("speckle_filter_pytorch", ms, ms, 6 * npx, extra={"note": "speckle_filter_pytorch on the GPU, timed eagerly"})
+        r = res["ops"]["speckle_filter"]
+        r["speedup_vs_torch"] = ms / r["ms_median"]
+        r["bit_equal_to_torch"] = bool(torch.equal(o_v.bool(), ref))
+        r["valid_in_frac"] = float(ok.float().mean())
+        r["valid_out_frac"] = float(o_v.float().mean())
+        del disp, ok, ref
     if "proj_nn" in only:
         T = 4
         xyz, K, poses = synth.make_clouds(T, H, W)
