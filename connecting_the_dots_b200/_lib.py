@@ -42,6 +42,10 @@ SIGNATURES = {
     "ctd_disparity_check_f64": [_ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _int, _f64, _int, _ptr],
     "ctd_speckle_filter_f32": [_ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _f64, _ptr],
     "ctd_speckle_filter_f64": [_ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _f64, _ptr],
+    "ctd_corr_softargmax_fwd_f32": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _f64, _ptr],
+    "ctd_corr_softargmax_fwd_f64": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _f64, _ptr],
+    "ctd_corr_softargmax_bwd_f32": [_ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _f64, _ptr],
+    "ctd_corr_softargmax_bwd_f64": [_ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _f64, _ptr],
     "ctd_proj_nn_f32": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _int, _ptr],
     "ctd_proj_nn_f64": [_ptr, _ptr, _ptr, _ptr, _i64, _i64, _i64, _int, _ptr],
     "ctd_nn_f32": [_ptr, _ptr, _ptr, _i64, _i64, _ptr],

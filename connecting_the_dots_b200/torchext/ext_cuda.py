@@ -186,6 +186,34 @@ def speckle_filter_cuda(disp, valid, max_size, max_diff):
     return out
 
 
+def corr_softargmax_fwd_cuda(f0, f1, n_disps, temperature):
+    """Correlation soft-argmax disparity (ctd_corr_softargmax_fwd_*).  f0, f1 [C,H,W] -> (disp, lse) [1,H,W]; batched:
+    [B,C,H,W] -> [B,1,H,W].  lse is the log-sum-exp of the scaled scores, saved for the backward."""
+    sfx, B, C, H, W, batched = _image_pair(f0, f1, "corr_softargmax")
+    disp, lse = _maps(f0, B, H, W, batched), _maps(f0, B, H, W, batched)
+    with torch.cuda.device(f0.device):
+        _lib.call("ctd_corr_softargmax_fwd" + sfx, f0.data_ptr(), f1.data_ptr(), disp.data_ptr(), lse.data_ptr(), B, C, H, W,
+                  int(n_disps), float(temperature), _stream(f0))
+    return disp, lse
+
+
+def corr_softargmax_bwd_cuda(f0, f1, disp, lse, grad_disp, n_disps, temperature, need_f0=True, need_f1=True):
+    """Gradients of corr_softargmax_fwd_cuda (ctd_corr_softargmax_bwd_*): (grad_f0, grad_f1), each like f0 or None when
+    not asked for."""
+    sfx, B, C, H, W, batched = _image_pair(f0, f1, "corr_softargmax")
+    for t, name in ((disp, "disp"), (lse, "lse"), (grad_disp, "grad_disp")):
+        _check_input_cuda(t, name)
+        _check(tuple(t.shape) == ((B, 1, H, W) if batched else (1, H, W)), "%s has to be f0's shape with one channel" % name)
+        _same(f0, t, "f0", name)
+    g0 = torch.empty_like(f0) if need_f0 else None
+    g1 = torch.empty_like(f1) if need_f1 else None
+    with torch.cuda.device(f0.device):
+        _lib.call("ctd_corr_softargmax_bwd" + sfx, f0.data_ptr(), f1.data_ptr(), disp.data_ptr(), lse.data_ptr(),
+                  grad_disp.data_ptr(), None if g0 is None else g0.data_ptr(), None if g1 is None else g1.data_ptr(), B, C, H, W,
+                  int(n_disps), float(temperature), _stream(f0))
+    return g0, g1
+
+
 def census_transform_cuda(x, wh, ww):
     """Census transform (ctd_census_transform_*): x [B,C,H,W] (or [C,H,W]) -> int64 of the same shape holding the uint64
     bit patterns."""

@@ -271,6 +271,83 @@ def speckle_filter_pytorch(disp, valid=None, max_size=100, max_diff=1.0):
     return (ok & (size > n)).view(disp.shape)
 
 
+def _corr_args(op, f0, f1, n_disps, temperature):
+    if f0.dim() not in (3, 4) or tuple(f0.shape) != tuple(f1.shape) or f0.dtype != f1.dtype:
+        raise RuntimeError("%s: f0 and f1 have to be C x H x W (or B x C x H x W) of the same shape and dtype" % op)
+    if f0.device != f1.device:
+        raise RuntimeError("%s: f0 and f1 must be on the same device" % op)
+    ext_cuda._real_suffix(f0, op)
+    D, tau = int(n_disps), float(temperature)
+    B = f0.size(0) if f0.dim() == 4 else 1
+    if B * f0.size(-2) * f0.size(-1) > 0 and (D != n_disps or D < 1 or f0.size(-3) < 1):
+        raise RuntimeError("%s: n_disps must be an integer >= 1 and C >= 1, got n_disps %r, C %d" % (op, n_disps, f0.size(-3)))
+    if not (tau > 0.0 and tau != float("inf")):
+        raise RuntimeError("%s: temperature must be finite and > 0, got %r" % (op, temperature))
+    return D, tau
+
+
+class CorrSoftArgmaxFunction(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, f0, f1, n_disps, temperature):
+        f0, f1 = f0.detach(), f1.detach()
+        disp, lse = ext_cuda.corr_softargmax_fwd_cuda(f0, f1, n_disps, temperature)
+        ctx.save_for_backward(f0, f1, disp, lse)
+        ctx.n_disps, ctx.temperature = n_disps, temperature
+        return disp
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_disp):
+        f0, f1, disp, lse = ctx.saved_tensors
+        g0, g1 = ext_cuda.corr_softargmax_bwd_cuda(f0, f1, disp, lse, grad_disp.contiguous(), ctx.n_disps, ctx.temperature,
+                                                   ctx.needs_input_grad[0], ctx.needs_input_grad[1])
+        return g0, g1, None, None
+
+
+def corr_softargmax(f0, f1, n_disps, temperature=1.0):
+    """Soft-argmax disparity of the correlation of two feature maps f0, f1 [B,C,H,W] (or [C,H,W]) over n_disps
+    disparities, as corr_softargmax_pytorch states it: [B,1,H,W] (or [1,H,W]) in the input dtype, differentiable w.r.t.
+    f0 and f1 (once).  The score volume is never written: the forward keeps an online softmax per pixel, the backward
+    recomputes the scores.  CUDA tensors only, float32 or float64, contiguous."""
+    _cuda_only(f0, "corr_softargmax")
+    D, tau = _corr_args("corr_softargmax", f0, f1, n_disps, temperature)
+    return CorrSoftArgmaxFunction.apply(f0, f1, D, tau)
+
+
+def corr_softargmax_pytorch(f0, f1, n_disps, temperature=1.0):
+    """The definition of corr_softargmax in plain torch, any device, differentiable through autograd, and its test oracle.
+
+    Inputs.  f0, f1: [B,C,H,W] (or [C,H,W]), same shape, dtype (float32 or float64) and device, contiguous; n_disps = D >= 1;
+    temperature = tau, finite and > 0.
+    Scores.  For pixel (b,h,w), let Dw = min(D, w + 1).  Only w - d >= 0 is a correspondence: there is no clamped column and
+    no zero padding.  For d < Dw, s_d = (sum_c f0[b,c,h,w] * f1[b,c,h,w-d]) / C.  This is the DispNetC / FlowNet
+    correlation normalisation.  Higher is better, the convention of xcorrvol and census_vol.
+    Soft-argmax.  m = max_d s_d/tau; lse = m + log sum_{d<Dw} exp(s_d/tau - m); p_d = exp(s_d/tau - lse);
+    disp = sum_{d<Dw} d * p_d.  Output disp is [B,1,H,W] (or [1,H,W]) in the input dtype.  At w = 0, disp = 0.
+    Gradient.  d disp / d s_d = p_d * (d - disp) / tau, chained through s_d to both f0 and f1.  Either input may not require
+    grad.  Double backward is not supported (once_differentiable).
+    Non-finite input is outside the contract.  The result is unspecified, but the call must not fault.
+    Sums of products in a different order differ in the last bits, so this op is checked against a tolerance, not bit for
+    bit.
+
+    Builds the masked [B,D,H,W] score volume (-inf where d >= Dw) and applies logsumexp and softmax."""
+    D, tau = _corr_args("corr_softargmax", f0, f1, n_disps, temperature)
+    a = f0 if f0.dim() == 4 else f0.unsqueeze(0)
+    b = f1 if f1.dim() == 4 else f1.unsqueeze(0)
+    B, C, H, W = a.shape
+    if B * H * W == 0:
+        return torch.zeros(f0.shape[:-3] + (1, H, W), dtype=f0.dtype, device=f0.device)
+    cols = []
+    for d in range(min(D, W)):
+        s = (a[..., d:] * b[..., :W - d]).sum(1) / C                   # [B,H,W-d]
+        cols.append(torch.nn.functional.pad(s, (d, 0), value=float("-inf")))
+    v = torch.stack(cols, 1) / tau                                      # [B,Deff,H,W]
+    p = torch.softmax(v, dim=1)
+    idx = torch.arange(v.size(1), device=v.device, dtype=v.dtype).view(1, -1, 1, 1)
+    disp = (p * idx).sum(1, keepdim=True)
+    return disp if f0.dim() == 4 else disp[0]
+
+
 SGM_PATHS = {4:((0, 1), (0, -1), (1, 0), (-1, 0)),
              8: ((0, 1), (0, -1), (1, 0), (-1, 0), (1, 1), (1, -1), (-1, 1), (-1, -1))}
 

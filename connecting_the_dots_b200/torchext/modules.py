@@ -122,6 +122,18 @@ class DisparityCheck(torch.nn.Module):
         return F.disparity_check(vol, self.max_diff, self.uniqueness, self.subpixel)
 
 
+class CorrSoftArgmax(torch.nn.Module):
+    """forward(f0, f1) -> disp of corr_softargmax: the differentiable soft-argmax disparity of the 1-D correlation of two
+    feature maps over n_disps disparities at a softmax temperature."""
+
+    def __init__(self, n_disps=128, temperature=1.0):
+        super().__init__()
+        self.n_disps, self.temperature = n_disps, temperature
+
+    def forward(self, f0, f1):
+        return F.corr_softargmax(f0, f1, self.n_disps, self.temperature)
+
+
 class CrossCheck(torch.nn.Module):
     def forward(self, in0, in1):
         return F.crosscheck(in0, in1)

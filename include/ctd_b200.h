@@ -268,6 +268,38 @@ int ctd_speckle_filter_f32(const float* disp, const uint8_t* valid, uint8_t* val
 int ctd_speckle_filter_f64(const double* disp, const uint8_t* valid, uint8_t* valid_out, int64_t B, int64_t H, int64_t W,
                            int64_t max_size, double max_diff, ctd_stream_t stream);
 
+/* ---- correlation soft-argmax disparity (an addition: the differentiable matching head of DispNetC / ActiveStereoNet), fused
+ * forward and backward that never write the B x D x H x W score volume.
+ *   Inputs.  f0, f1: [B,C,H,W] (or [C,H,W]), same shape, dtype (float or double) and device, contiguous; n_disps = D >= 1;
+ *            temperature = tau, finite and > 0.
+ *   Scores.  For pixel (b,h,w), let Dw = min(D, w + 1).  Only w - d >= 0 is a correspondence: there is no clamped column
+ *            and no zero padding.  For d < Dw, s_d = (sum_c f0[b,c,h,w] * f1[b,c,h,w-d]) / C.  This is the DispNetC /
+ *            FlowNet correlation normalisation.  Higher is better, the convention of xcorrvol and census_vol.
+ *   Soft-argmax.  m = max_d s_d/tau; lse = m + log sum_{d<Dw} exp(s_d/tau - m); p_d = exp(s_d/tau - lse);
+ *            disp = sum_{d<Dw} d * p_d.  Output disp is [B,1,H,W] (or [1,H,W]) in the input dtype.  At w = 0, disp = 0.
+ *   Gradient.  d disp / d s_d = p_d * (d - disp) / tau, chained through s_d to both f0 and f1.  Either input may not
+ *            require grad.  Double backward is not supported (once_differentiable).
+ *   Non-finite input is outside the contract.  The result is unspecified, but the call must not fault.
+ * Sums of products in a different order differ in the last bits, so this op is checked against a tolerance, not bit for
+ * bit.
+ * DEVICE pointers.  fwd writes disp and lse ([B,1,H,W] each, lse saved for bwd).  bwd takes grad_disp [B,1,H,W] and writes
+ * grad_f0 and grad_f1 ([B,C,H,W], overwritten); either may be NULL (that half is skipped), both NULL is a no-op.
+ * B*H*W = 0 is CTD_OK with nothing launched.  CTD_ERR_INVALID, checked before any device work, for: negative sizes; C < 1
+ * or D < 1 when B*H*W > 0; a temperature that is non-positive or non-finite; C or H > INT32_MAX, W > INT32_MAX / 4; null
+ * required pointers; any output overlapping an input or another output.  One launch for fwd, one per gradient for bwd;
+ * no scratch memory, no atomics (the gradients are bit-identical from run to run), no host synchronisation,
+ * capture-safe; 64-bit indexing over the batch. */
+int ctd_corr_softargmax_fwd_f32(const float* f0, const float* f1, float* disp, float* lse, int64_t B, int64_t C, int64_t H,
+                                int64_t W, int64_t n_disps, double temperature, ctd_stream_t stream);
+int ctd_corr_softargmax_fwd_f64(const double* f0, const double* f1, double* disp, double* lse, int64_t B, int64_t C,
+                                int64_t H, int64_t W, int64_t n_disps, double temperature, ctd_stream_t stream);
+int ctd_corr_softargmax_bwd_f32(const float* f0, const float* f1, const float* disp, const float* lse,
+                                const float* grad_disp, float* grad_f0, float* grad_f1, int64_t B, int64_t C, int64_t H,
+                                int64_t W, int64_t n_disps, double temperature, ctd_stream_t stream);
+int ctd_corr_softargmax_bwd_f64(const double* f0, const double* f1, const double* disp, const double* lse,
+                                const double* grad_disp, double* grad_f0, double* grad_f1, int64_t B, int64_t C, int64_t H,
+                                int64_t W, int64_t n_disps, double temperature, ctd_stream_t stream);
+
 /* ---- ProjNNFunctor: ext.h:65-117, ext_cuda.cpp:47-69 (proj_nn_cuda).  K is a DEVICE pointer to
  * 9 values (row-major 3x3), like the reference's K tensor. */
 int ctd_proj_nn_f32(const float* xyz0, const float* xyz1, const float* K, int64_t* out, int64_t B,

@@ -3,7 +3,7 @@
 launching stream, rotating buffer sets larger than L2 where the op is HBM-bound).  Prints one JSON
 object; bench.py stays the contract benchmark, this is the per-op table that goes into profiles/.
 
-    python tools/bench_ops.py [--iters 30] [--only photometric,ssim,lcn,xcorrvol,xcorr_disparity,sgm,census_match,disparity_check,speckle,proj_nn,nn,crosscheck]
+    python tools/bench_ops.py [--iters 30] [--only photometric,ssim,lcn,xcorrvol,xcorr_disparity,sgm,census_match,disparity_check,speckle,corr_softargmax,proj_nn,nn,crosscheck]
 
 The printed result names the GPU and its power limit, read in the same run.
 """
@@ -70,6 +70,17 @@ def device_info(index):
     return info
 
 
+def sm_clock_mhz(index):
+    """Current and maximum SM clock of the GPU (MHz), read by nvidia-smi; torch's reading where nvidia-smi is missing."""
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=clocks.sm,clocks.max.sm", "--format=csv,noheader,nounits", "-i",
+                              str(index)], capture_output=True, text=True, timeout=60).stdout.strip()
+        cur, mx = (float(v) for v in out.split(","))
+    except Exception:
+        cur = mx = float(torch.cuda.clock_rate(index))
+    return {"current_mhz": cur, "max_mhz": mx}
+
+
 def census_traffic(B, C, H, W, D):
     """Least HBM bytes of the census calls, from shapes: the volume writes 4 B per pixel and disparity and reads both fp32
     inputs; the fused disparity reads the inputs and writes disp and score (16 B/px at C = 1)."""
@@ -77,7 +88,7 @@ def census_traffic(B, C, H, W, D):
     return {"volume": (4 * D + 8 * C) * npx, "disparity": (8 * C + 8) * npx}
 
 
-ALL = "calib,photometric,ssim,warp,pyramid,geometric,disparity,lcn,xcorrvol,xcorr_disparity,sgm,census_match,disparity_check,speckle,proj_nn,config4,nn,crosscheck,reduce,gpu_reference"
+ALL = "calib,photometric,ssim,warp,pyramid,geometric,disparity,lcn,xcorrvol,xcorr_disparity,sgm,census_match,disparity_check,speckle,corr_softargmax,proj_nn,config4,nn,crosscheck,reduce,gpu_reference"
 
 
 def main():
@@ -552,6 +563,87 @@ def run(only=ALL, iters=30, batch=8, device_index=0, verbose=True):
         r["valid_in_frac"] = float(ok.float().mean())
         r["valid_out_frac"] = float(o_v.float().mean())
         del disp, ok, ref
+    if "corr_softargmax" in only:
+        # correlation soft-argmax, D = 128, fp32: C = 1 (ta against pat_lcn of the bench frames) and C = 32 (random
+        # features).  Forward alone and forward + backward (both gradients) through the C ABI, against
+        # corr_softargmax_pytorch with autograd on the same GPU.  Floors from shapes: HBM bytes (8C + 8 forward, 16C + 12
+        # backward per pixel) at PEAK, and FMAs at 148 SMs x 128 FP32 lanes x the maximum SM clock.  FMAs: C per score
+        # (scores = sum over pixels of min(D, w + 1)) forward; the backward needs at least one recompute and one FMA per
+        # score and channel for each gradient, so forward + backward is at least 4 C per score.  (The kernels recompute
+        # the scores once per gradient, 5 C per score in all.)  The larger floor bounds the call.
+        # One input set serves every launch: at C = 32 it is far larger than L2, at C = 1 (20 MB at batch 8) it fits.
+        D, tau = 128, 1.0
+        clk = sm_clock_mhz(device_index)
+        fma_rate = 148 * 128 * clk["max_mhz"] * 1e6
+        scores = B * H * sum(min(D, w + 1) for w in range(W))
+        g = torch.Generator(device=dev).manual_seed(0)
+        for C in (1, 32):
+            if C == 1:
+                f0, f1 = sets[0]["ta"], sets[0]["pat_lcn"]
+            else:
+                f0 = torch.randn(B, C, H, W, device=dev, generator=g)
+                f1 = torch.randn(B, C, H, W, device=dev, generator=g)
+            gd = torch.randn(B, 1, H, W, device=dev, generator=g)
+            disp, lse = torch.empty(B, 1, H, W, device=dev), torch.empty(B, 1, H, W, device=dev)
+            g0, g1 = torch.empty_like(f0), torch.empty_like(f1)
+
+            def fwd(i, st):
+                _lib.call("ctd_corr_softargmax_fwd_f32", f0.data_ptr(), f1.data_ptr(), disp.data_ptr(), lse.data_ptr(), B, C, H,
+                          W, D, tau, st)
+
+            def fwd_bwd(i, st):
+                fwd(i, st)
+                _lib.call("ctd_corr_softargmax_bwd_f32", f0.data_ptr(), f1.data_ptr(), disp.data_ptr(), lse.data_ptr(),
+                          gd.data_ptr(), g0.data_ptr(), g1.data_ptr(), B, C, H, W, D, tau, st)
+            floors = {"fwd": ((8 * C + 8) * npx, C * scores), "fwd_bwd": ((24 * C + 20) * npx, 4 * C * scores)}
+            for name, fn in (("fwd", fwd), ("fwd_bwd", fwd_bwd)):
+                ms, ms_min = timeit(fn, args.iters, nrep=3)
+                by, fm = floors[name]
+                t_hbm, t_fma = by / PEAK / 1e6, fm / fma_rate * 1e3
+                add("corr_softargmax_%s_C%d" % (name, C), ms, ms_min, by,
+                    extra={"fma": fm, "floor_ms_hbm": t_hbm, "floor_ms_fma": t_fma,
+                           "bound": "fma" if t_fma > t_hbm else "hbm", "frac_of_floor": max(t_hbm, t_fma) / ms})
+
+            def peak(fn):
+                torch.cuda.synchronize()
+                base_mem = torch.cuda.memory_allocated(dev)
+                torch.cuda.reset_peak_memory_stats(dev)
+                fn()
+                torch.cuda.synchronize()
+                return torch.cuda.max_memory_allocated(dev) - base_mem
+
+            def eager(fn, reps=3):
+                fn()
+                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                torch.cuda.synchronize()
+                e0.record()
+                for _ in range(reps):
+                    fn()
+                e1.record()
+                torch.cuda.synchronize()
+                return e0.elapsed_time(e1) / reps
+
+            def run_pair(op, backward):
+                def fn():
+                    a, b = f0.detach().requires_grad_(backward), f1.detach().requires_grad_(backward)
+                    out = op(a, b, D, tau)
+                    if backward:
+                        out.backward(gd)
+                return fn
+            for name, backward in (("fwd", False), ("fwd_bwd", True)):
+                r = res["ops"]["corr_softargmax_%s_C%d" % (name, C)]
+                r["peak_bytes_op"] = peak(run_pair(tx.corr_softargmax, backward))
+                ms = eager(run_pair(tx.corr_softargmax_pytorch, backward))
+                r["peak_bytes_pytorch"] = peak(run_pair(tx.corr_softargmax_pytorch, backward))
+                add("corr_softargmax_pytorch_%s_C%d" % (name, C), ms, ms, floors[name][0],
+                    extra={"note": "corr_softargmax_pytorch with autograd on the GPU, timed eagerly",
+                           "peak_bytes": r["peak_bytes_pytorch"]})
+                r["speedup_vs_torch"] = ms / r["ms_median"]
+            with torch.no_grad():
+                ref = tx.corr_softargmax_pytorch(f0, f1, D, tau)
+            res["ops"]["corr_softargmax_fwd_C%d" % C]["max_abs_err_vs_torch_fp32"] = float((disp - ref).abs().max())
+            del f0, f1, g0, g1, gd, disp, lse, ref
+        res["sm_clock"] = clk
     if "proj_nn" in only:
         T = 4
         xyz, K, poses = synth.make_clouds(T, H, W)
